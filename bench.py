@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — front-end frames/s at 640x480 (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over the C5 sequence of BASELINE.json: 8192 synthetic TUM-fr3-shaped 640x480 RGB-D frames,
@@ -72,6 +72,12 @@ ALG_BYTES_FRAME = 6403474 + 2150400 + 2 * 3024000 + 3452928 + 2359296 + 909312 +
 # dram__bytes_read.sum + dram__bytes_write.sum per frame of the same kernels, from this round's committed ncu capture
 # (profiles/r2b_ncu_full_orb_kernels_b296.csv for the ORB kernels; profiles/r1d_* for the others, unchanged kernels)
 NCU_DRAM_BYTES = {'k_resize x7': 1555000, 'k_fast_strips': 968000, 'k_describe': 1102000, 'k_lsd_prep': 3592000, 'k_plane_blocks': 857000}
+DUMP_BYTES = 64 * 10 ** 6                                                      # --dump-outputs writes at most this much
+DUMP_SEED = 0                                                                  # which frames of the last call --dump-outputs writes
+# rows past the frame's count in these outputs are scratch, not results: --dump-outputs writes the valid rows of the sampled frames one
+# after the other (the count outputs say how many belong to each frame)
+DUMP_ROWS = dict(kps='kp_counts', desc='kp_counts', kp_depth='kp_counts', kp_uright='kp_counts', keylines='line_counts',
+                 line_desc='line_counts', linevec3='line_counts', planes7='n_planes')
 
 
 def _gen(args):
@@ -267,6 +273,47 @@ def shard(n, world, rank):
     return lo, hi - lo
 
 
+def _float_dtype(dt):
+    """the float type that holds every value of dt exactly: floats stay, 8- / 16-bit integers -> float32, wider -> float64"""
+    return dt if dt.kind == 'f' else np.dtype(np.float32 if dt.itemsize <= 2 else np.float64)
+
+
+def _float_bytes(dt):
+    """bytes --dump-outputs may write per element of dt: the float copy, and a float32 finite mask for float outputs"""
+    if dt.names:
+        return sum(_float_bytes(dt.fields[f][0]) for f in dt.names)
+    return _float_dtype(dt).itemsize + (4 if dt.kind == 'f' else 0)
+
+
+def dump_outputs(out_dir, shapes, d_out, n, frames):
+    """--dump-outputs: the outputs of the first n frames held in d_out (output_shapes layout), sampled to at most DUMP_BYTES, as
+    out_dir/<name>.npy in float32 / float64, every value finite.  A structured output gives one file per field (kps_x,
+    keylines_class_id, ...); the outputs of DUMP_ROWS keep only the valid rows.  Where an output holds NaN or inf (surface normals
+    that have none), those entries are written as 0 and <name>_finite.npy is 1 where the value is finite, 0 where it is not.
+    frames: the sequence index of each of the n frames (frame.npy)."""
+    import torch
+    per_frame = sum(int(np.prod(sh[1:])) * _float_bytes(np.dtype(dt)) for sh, dt in shapes.values()) + 8
+    k = max(1, min(n, (DUMP_BYTES - (1 << 16)) // per_frame))              # 64 KB for the .npy headers
+    pick = np.sort(np.random.RandomState(DUMP_SEED).choice(n, k, replace=False))
+    sel = torch.from_numpy(pick).to(next(iter(d_out.values())).device)
+    host = {}
+    for name, (sh, dt) in shapes.items():
+        rows = d_out[name].view(sh[0], -1).index_select(0, sel).cpu().numpy()
+        host[name] = rows.view(dt).reshape((k,) + tuple(sh[1:]))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'frame.npy'), np.asarray(frames, np.float64)[pick])
+    for name, a in host.items():
+        for key, v in ({f'{name}_{f}': a[f] for f in a.dtype.names} if a.dtype.names else {name: a}).items():
+            v = v.astype(_float_dtype(v.dtype))
+            if name in DUMP_ROWS:
+                v = v[np.arange(v.shape[1])[None, :] < host[DUMP_ROWS[name]][:, None]]
+            finite = np.isfinite(v)
+            if not finite.all():
+                np.save(os.path.join(out_dir, key + '_finite.npy'), finite.astype(np.float32))
+                v = np.where(finite, v, 0).astype(v.dtype)
+            np.save(os.path.join(out_dir, key + '.npy'), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -282,7 +329,14 @@ def main():
     ap.add_argument('--device-only', action='store_true', help='profiling aid: only the device-resident loop')
     ap.add_argument('--as-shard', default='', help='profiling aid: R/W = process the range rank R of W would get (single process)')
     ap.add_argument('--e2e-only', action='store_true', help='profiling aid: skip the per-stage passes, the latency probe and the CPU baseline')
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='after the timed steps, write the outputs of the last call of the last step (rank 0; a fixed, seeded sample of '
+                         f'its frames, at most {DUMP_BYTES // 10 ** 6} MB) as DIR/<name>.npy in float32 / float64, to compare two builds')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
 
     rank = int(os.environ.get('RANK', 0))
@@ -403,6 +457,9 @@ def main():
     launches_per_step = fe.last_launches() * calls_per_step
     value = args.frames * args.steps / (ms * 1e-3)
     means = dict(keypoints=d_counts('kp_counts'), lines=d_counts('line_counts'), planes=d_counts('n_planes'))
+    if args.dump_outputs and rank == 0:
+        last = (count - 1) // call * call                     # d_out holds what the last call of the step wrote: frames last .. count - 1
+        dump_outputs(args.dump_outputs, shapes, d_out, count - last, np.arange(first + last, first + count))
 
     if args.device_only:
         emit({'metric': METRIC, 'value': value, 'unit': 'frames/s', 'ms_per_step': ms / args.steps, 'rank': rank, 'ms_per_step_this_rank': ms_rank / args.steps, 'host_enqueue_ms_per_step': host_enqueue_ms, 'device_only': True, 'frames_per_step': args.frames,

@@ -2,6 +2,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 
@@ -35,18 +37,30 @@ def test_version_and_error_strings(hvo):
     assert isinstance(l.hvo_last_error(), bytes)
 
 
-def test_create_fails_loudly_without_a_device(hvo):
-    """No CPU fallback: on a box without CUDA every create call reports HVO_ERR_CUDA."""
-    try:
-        n = hvo.device_count()
-    except hvo.HvoError as e:
-        assert e.status == hvo.HVO_ERR_CUDA
-        n = 0
-    if n > 0:
-        pytest.skip('a CUDA device is present')
-    with pytest.raises(hvo.HvoError) as ei:
-        hvo.ORBextractor(1000, 1.2, 8, 20, 7, width=640, height=480)
-    assert ei.value.status == hvo.HVO_ERR_CUDA
+_NO_DEVICE = '''
+import hvo_b200 as hvo
+try:
+    n = hvo.device_count()
+except hvo.HvoError as e:
+    assert e.status == hvo.HVO_ERR_CUDA, e
+    n = 0
+assert n == 0, n
+try:
+    hvo.ORBextractor(1000, 1.2, 8, 20, 7, width=640, height=480)
+except hvo.HvoError as e:
+    assert e.status == hvo.HVO_ERR_CUDA, e
+else:
+    raise AssertionError('created without a device')
+print('ok')
+'''
+
+
+def test_create_fails_loudly_without_a_device():
+    """No CPU fallback: on a box without CUDA every create call reports HVO_ERR_CUDA.  Checked in a child process that sees no
+    device (CUDA_VISIBLE_DEVICES empty), so that it runs on a box with GPUs as well."""
+    r = subprocess.run([sys.executable, '-c', _NO_DEVICE], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=''),
+                       capture_output=True, text=True)
+    assert r.returncode == 0 and r.stdout.strip() == 'ok', r.stdout + r.stderr
 
 
 def test_argument_validation_needs_no_device(hvo):
