@@ -39,6 +39,24 @@ class _RgbdParams(C.Structure):
     _fields_ = [('depth_factor', C.c_float), ('bf', C.c_float), ('distorted', C.c_int)]
 
 
+class _Camera(C.Structure):
+    _fields_ = [(n, C.c_float) for n in ('fx', 'fy', 'cx', 'cy', 'k1', 'k2', 'p1', 'p2', 'k3')]
+
+
+def _dist5(dist):
+    """mDistCoef (4 entries, or 5 when Camera.k3 != 0) -> k1, k2, p1, p2, k3 as float32."""
+    d = np.asarray(dist, np.float32).ravel()
+    if len(d) not in (4, 5):
+        raise HvoError(HVO_ERR_ARG, f'dist must hold k1, k2, p1, p2 [, k3] (got {len(d)} values)')
+    return np.concatenate([d, np.zeros(5 - len(d), np.float32)])
+
+
+def _camera(K, dist):
+    """hvo_camera of mK (3x3) and mDistCoef, both narrowed to float32 as the reference stores them."""
+    K = np.asarray(K, np.float32).reshape(3, 3)
+    return _Camera(K[0, 0], K[1, 1], K[0, 2], K[1, 2], *_dist5(dist))
+
+
 _lib = None
 _vp = C.c_void_p
 
@@ -61,6 +79,9 @@ ABI = {
     'hvo_orb_stage_times': (C.c_int, [_vp, C.POINTER(C.c_float)]),
     'hvo_orb_last_launches': (C.c_int, [_vp]),
     'hvo_stereo_uright_from_depth': (C.c_int, [_vp, _vp, C.c_int, C.c_float, _vp]),
+    'hvo_undistort_points': (C.c_int, [C.POINTER(_Camera), _vp, C.c_int, _vp]),
+    'hvo_image_bounds': (C.c_int, [C.POINTER(_Camera), C.c_int, C.c_int] + [C.POINTER(C.c_float)] * 4),
+    'hvo_orb_undistort_batch_device': (C.c_int, [_vp, C.POINTER(_Camera), _vp, _vp, C.c_int, _vp, C.c_float, _vp, _vp]),
     'hvo_membership4_expand': (C.c_int, [_vp, C.c_int, _vp]),
     'hvo_seq_create': (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int, C.c_int, _vp]),
     'hvo_seq_destroy': (None, [_vp]),
@@ -268,6 +289,22 @@ def frustum_cam(Rcw, tcw, fx, fy, cx, cy, bf, bounds, scale_factor=1.2, n_levels
     return c
 
 
+def undistort_points(pts, K, dist):
+    """cv2.undistortPoints(pts, K, dist, None, K) bit for bit (hvo_undistort_points, host): pts [n,2] -> float32 [n,2]; K 3x3,
+    dist = k1, k2, p1, p2 [, k3], narrowed to float32 as the reference's mK / mDistCoef.  No k1 == 0 shortcut."""
+    p = np.ascontiguousarray(np.asarray(pts, np.float32).reshape(-1, 2))
+    out = np.empty_like(p)
+    _check(lib().hvo_undistort_points(C.byref(_camera(K, dist)), _np_ptr(p), len(p), _np_ptr(out)))
+    return out
+
+
+def image_bounds(K, dist, width, height):
+    """Frame::ComputeImageBounds (reference src/Frame.cc:1733-1760) -> (mnMinX, mnMaxX, mnMinY, mnMaxY) as float32."""
+    v = [C.c_float(0) for _ in range(4)]
+    _check(lib().hvo_image_bounds(C.byref(_camera(K, dist)), int(width), int(height), *[C.byref(a) for a in v]))
+    return tuple(np.float32(a.value) for a in v)
+
+
 def predict_scale_thresholds(log_scale_factor, lo, n):
     thr = np.empty(max(n, 1), np.float32)
     _check(lib().hvo_predict_scale_thresholds(float(log_scale_factor), int(lo), int(n), _np_ptr(thr)))
@@ -365,13 +402,19 @@ class ORBextractor:
         return kps[:n.value].copy(), desc[:n.value].copy()
 
     # -- batched host path ----------------------------------------------------------------------------
-    def extract_batch(self, frames, depth16=None, depth_factor=None, bf=None, out=None, distorted=False):
+    def extract_batch(self, frames, depth16=None, depth_factor=None, bf=None, out=None, distorted=False, camera=None):
         """frames [n,h,w] uint8 (host; pinned memory makes the copies asynchronous).  Returns
         dict(counts, kps [n,cap], desc [n,cap,32], depth, uright).  distorted: the camera has k1 != 0, so mvuRight needs the
-        undistorted keypoints (Frame.cc:1944): uright comes back as -1, form it with stereo_uright_from_depth()."""
+        undistorted keypoints (Frame.cc:1944): uright comes back as -1, form it with stereo_uright_from_depth().
+        camera = (K, dist): Frame::UndistortKeyPoints on the device as well (hvo_orb_undistort_batch_device): the result gains
+        kps_un [n,cap] (mvKeysUn) and uright is formed from it."""
         assert frames.dtype == np.uint8 and frames.ndim == 3 and frames.flags.c_contiguous
         n, h, w = frames.shape
         self._ensure(w, h)
+        if camera is not None:
+            if out is not None:
+                raise HvoError(HVO_ERR_ARG, 'out= is not supported together with camera=')
+            return self._extract_batch_undistorted(frames, depth16, depth_factor, bf, camera)
         cap = self.capacity
         if out is None:
             out = dict(counts=np.empty(n, np.int32), kps=np.empty((n, cap), KP_DTYPE), desc=np.empty((n, cap, 32), np.uint8))
@@ -387,6 +430,40 @@ class ORBextractor:
                                            _np_ptr(out['depth']) if depth16 is not None else None,
                                            _np_ptr(out['uright']) if depth16 is not None else None))
         return out
+
+    def _extract_batch_undistorted(self, frames, depth16, depth_factor, bf, camera):
+        import torch
+        n, cap = len(frames), self.capacity
+        dev = torch.device('cuda', self.device)
+        g = torch.from_numpy(frames).to(dev)
+        kps = torch.empty((n, cap, KP_DTYPE.itemsize), dtype=torch.uint8, device=dev)
+        kps_un = torch.empty_like(kps)
+        desc = torch.empty((n, cap, 32), dtype=torch.uint8, device=dev)
+        counts = torch.empty(n, dtype=torch.int32, device=dev)
+        rgbd = depth16 is not None
+        if rgbd:
+            assert depth16.dtype == np.uint16 and depth16.shape == frames.shape
+            d16 = torch.from_numpy(np.ascontiguousarray(depth16)).to(dev)
+            kd, ku = torch.empty((n, cap), dtype=torch.float32, device=dev), torch.empty((n, cap), dtype=torch.float32, device=dev)
+        torch.cuda.synchronize(dev)   # the uploads ran on torch's stream; the handle's stream starts after them
+        self.extract_batch_device(g.data_ptr(), n, kps.data_ptr(), desc.data_ptr(), counts.data_ptr(), d16.data_ptr() if rgbd else None,
+                                  float(depth_factor or 0.0), float(bf or 0.0), kd.data_ptr() if rgbd else None,
+                                  ku.data_ptr() if rgbd else None, distorted=True)
+        self.undistort_batch_device(camera, kps.data_ptr(), counts.data_ptr(), n, kd.data_ptr() if rgbd else None, float(bf or 0.0),
+                                    kps_un.data_ptr(), ku.data_ptr() if rgbd else None)
+        self.sync()
+        out = dict(counts=counts.cpu().numpy(), kps=kps.cpu().numpy().view(KP_DTYPE).reshape(n, cap),
+                   desc=desc.cpu().numpy(), kps_un=kps_un.cpu().numpy().view(KP_DTYPE).reshape(n, cap))
+        if rgbd:
+            out['depth'], out['uright'] = kd.cpu().numpy(), ku.cpu().numpy()
+        return out
+
+    def undistort_batch_device(self, camera, d_kps, d_counts, nframes, d_kp_depth=None, bf=0.0, d_kps_un=None, d_kp_uright=None):
+        """hvo_orb_undistort_batch_device on the handle's stream: camera = (K, dist); raw device pointers (int) or None."""
+        K, dist = camera
+        _check(lib().hvo_orb_undistort_batch_device(self._h, C.byref(_camera(K, dist)), _vp(d_kps), _vp(d_counts), int(nframes),
+                                                    _vp(d_kp_depth) if d_kp_depth else None, float(bf),
+                                                    _vp(d_kps_un) if d_kps_un else None, _vp(d_kp_uright) if d_kp_uright else None))
 
     @staticmethod
     def stereo_uright_from_depth(keys_un, kp_depth, bf):
@@ -1836,12 +1913,12 @@ class ORBmatcher:
 class _FrameParams(C.Structure):
     _fields_ = [('orb', _OrbParams), ('line', _LineParams), ('fx', C.c_float), ('fy', C.c_float), ('cx', C.c_float), ('cy', C.c_float),
                 ('depth_factor', C.c_float), ('bf', C.c_float), ('distorted', C.c_int), ('stages', C.c_int), ('max_planes', C.c_int), ('line_cull', C.c_int),
-                ('lanes', C.c_int)]
+                ('lanes', C.c_int), ('k1', C.c_float), ('k2', C.c_float), ('p1', C.c_float), ('p2', C.c_float), ('k3', C.c_float)]
 
 
 class _FrameOutputs(C.Structure):
     _fields_ = [(n, _vp) for n in ('kps', 'desc', 'kp_counts', 'kp_depth', 'kp_uright', 'keylines', 'line_desc', 'linevec3',
-                                   'line_counts', 'n_planes', 'planes7', 'membership', 'normals8', 'membership8', 'membership4', 'normals3')]
+                                   'line_counts', 'n_planes', 'planes7', 'membership', 'normals8', 'membership8', 'membership4', 'normals3', 'kps_un')]
 
 
 class FrameFrontEnd:
@@ -1851,17 +1928,19 @@ class FrameFrontEnd:
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, bf=40.0, nfeatures=1000, scale_factor=1.2, nlevels=8, ini_th=20,
                  min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=16, max_batch=1, device=0, line_cull=False, lanes=0, membership='i32',
-                 distorted=False, normals='n8'):
+                 distorted=False, normals='n8', dist=None):
         """membership: 'i32' (int32 labels, -1 = none), 'u8' (one byte per pixel, 255 = none: what a host caller needs to
         rebuild plane_vertices_), 'both', or 'u4' (host calls only: two pixels per byte, 15 = none, max_planes <= 15; expand with
         membership4_expand).  The int32 image is always the device-side working image.
         normals: 'n8' (SurfaceNormal rows: normal, position, pixel) or 'n3' (host calls only: the normal alone; normals3_expand
-        rebuilds the rows from the depth image)."""
+        rebuilds the rows from the depth image).
+        dist: mDistCoef (k1, k2, p1, p2 [, k3]).  With a non-zero coefficient the handle runs Frame::UndistortKeyPoints on the device:
+        kp_uright is formed from the undistorted keypoints and the outputs gain kps_un (mvKeysUn)."""
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
-        prm = _FrameParams(_OrbParams(nfeatures, scale_factor, nlevels, ini_th, min_th), _LineParams(1, 1.2, n_lines, 0.125),
-                           fx, fy, cx, cy, float(np.float32(depth_factor)), bf, int(bool(distorted)), stages, max_planes, int(bool(line_cull)), int(lanes))
+        prm = self._params(fx, fy, cx, cy, depth_factor, bf, nfeatures, scale_factor, nlevels, ini_th, min_th, n_lines, stages, max_planes,
+                           line_cull, lanes, distorted, dist)
         out = _vp()
         _check(lib().hvo_frame_create(C.byref(prm), int(width), int(height), int(max_batch), int(device), C.byref(out)))
         self._h = out
@@ -1871,6 +1950,14 @@ class FrameFrontEnd:
         self.orb_capacity, self.max_lines, self.normals_count = a.value, b.value, c.value
         _check(lib().hvo_frame_lanes(out, C.byref(a), C.byref(b)))
         self.lanes, self.chunk = a.value, b.value
+
+    def _params(self, fx, fy, cx, cy, depth_factor, bf, nfeatures, scale_factor, nlevels, ini_th, min_th, n_lines, stages, max_planes,
+                line_cull, lanes, distorted, dist):
+        d5 = _dist5(dist) if dist is not None else np.zeros(5, np.float32)
+        self.undistorts = bool(d5.any())
+        return _FrameParams(_OrbParams(nfeatures, scale_factor, nlevels, ini_th, min_th), _LineParams(1, 1.2, n_lines, 0.125),
+                            fx, fy, cx, cy, float(np.float32(depth_factor)), bf, int(bool(distorted) or self.undistorts), stages, max_planes,
+                            int(bool(line_cull)), int(lanes), *[float(v) for v in d5])
 
     def close(self):
         if getattr(self, '_h', None):
@@ -1891,6 +1978,8 @@ class FrameFrontEnd:
             c = self.orb_capacity
             sh.update(kps=((n, c), KP_DTYPE), desc=((n, c, 32), np.uint8), kp_counts=((n,), np.int32), kp_depth=((n, c), np.float32),
                       kp_uright=((n, c), np.float32))
+            if self.undistorts:
+                sh.update(kps_un=((n, c), KP_DTYPE))
         if self.stages & STAGE_LINES:
             c = self.max_lines
             sh.update(keylines=((n, c), KL_DTYPE), line_desc=((n, c, 32), np.uint8), linevec3=((n, c, 3), np.float64),
@@ -1949,14 +2038,18 @@ class FrameFrontEnd:
         if out is None:
             out = self.alloc_host(n)
         else:   # the C side writes through raw pointers: every caller-supplied array must have the exact layout
-            for k, (shape, dt) in self.output_shapes(n, device=False).items():
-                a = out.get(k)
-                if a is None or a.shape != tuple(shape) or a.dtype != np.dtype(dt) or not a.flags.c_contiguous:
-                    raise HvoError(HVO_ERR_ARG, f'out[{k!r}] must be a C-contiguous {np.dtype(dt)} array of shape {tuple(shape)}')
+            self._check_out(out, self.output_shapes(n, device=False))
         o = self._outputs({k: v.ctypes.data for k, v in out.items()})
         f = lib().hvo_frame_extract_batch if wait else lib().hvo_frame_extract_batch_async
         _check(f(self._h, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o)))
         return out
+
+    @staticmethod
+    def _check_out(out, shapes):
+        for k, (shape, dt) in shapes.items():
+            a = out.get(k)
+            if a is None or a.shape != tuple(shape) or a.dtype != np.dtype(dt) or not a.flags.c_contiguous:
+                raise HvoError(HVO_ERR_ARG, f'out[{k!r}] must be a C-contiguous {np.dtype(dt)} array of shape {tuple(shape)}')
 
     def extract_batch_device(self, d_gray, d_depth16, n, d_ptrs):
         """d_ptrs: name -> device pointer (int) for every output of output_shapes(n).  Asynchronous."""
@@ -1985,12 +2078,12 @@ class FrameSequence(FrameFrontEnd):
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, devices, frames_per_call=2368, bf=40.0, nfeatures=1000, scale_factor=1.2,
                  nlevels=8, ini_th=20, min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=15, line_cull=True, lanes=0, membership='u4',
-                 normals='n3', distorted=False):
+                 normals='n3', distorted=False, dist=None):
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
-        prm = _FrameParams(_OrbParams(nfeatures, scale_factor, nlevels, ini_th, min_th), _LineParams(1, 1.2, n_lines, 0.125),
-                           fx, fy, cx, cy, float(np.float32(depth_factor)), bf, int(bool(distorted)), stages, max_planes, int(bool(line_cull)), int(lanes))
+        prm = self._params(fx, fy, cx, cy, depth_factor, bf, nfeatures, scale_factor, nlevels, ini_th, min_th, n_lines, stages, max_planes,
+                           line_cull, lanes, distorted, dist)
         dev = (C.c_int * len(devices))(*[int(d) for d in devices])
         out = _vp()
         _check(lib().hvo_seq_create(C.byref(prm), int(width), int(height), dev, len(devices), int(frames_per_call), C.byref(out)))
@@ -2022,6 +2115,8 @@ class FrameSequence(FrameFrontEnd):
             raise HvoError(HVO_ERR_ARG, f'gray / depth16 must be [n, {self.h}, {self.w}]')
         if out is None:
             out = self.alloc_host(n)
+        else:   # kps_un at least: the other arrays' check is a separate change
+            self._check_out(out, {k: v for k, v in self.output_shapes(n, device=False).items() if k == 'kps_un'})
         o = self._outputs({k: v.ctypes.data for k, v in out.items()})
         _check(lib().hvo_seq_extract(self._seq, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o)))
         return out

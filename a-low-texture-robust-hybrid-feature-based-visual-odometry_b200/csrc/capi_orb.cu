@@ -1,4 +1,6 @@
 // C ABI for the ORB extractor (include/hvo_capi.h).  No torch types, no exceptions across the boundary.
+#include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstring>
@@ -7,6 +9,7 @@
 #include <vector>
 
 #include "orb.cuh"
+#include "undistort.cuh"
 
 namespace hvo {
 static thread_local char g_err[512] = "";
@@ -277,6 +280,43 @@ int hvo_stereo_uright_from_depth(const hvo_keypoint* keys_un, const float* kp_de
         uright[i] = d > 0.f ? keys_un[i].x - bf / d : -1.f;   // host code is built with -ffp-contract=off
     }
     return HVO_OK;
+}
+
+static bool camera_ok(const hvo_camera* c) {
+    return c && c->fx != 0.f && c->fy != 0.f && std::isfinite(c->fx) && std::isfinite(c->fy) && std::isfinite(c->cx) && std::isfinite(c->cy);
+}
+
+int hvo_undistort_points(const hvo_camera* cam, const float* xy, int n, float* xy_un) {
+    HVO_CHECK_ARG(camera_ok(cam), "camera missing or fx / fy zero or not finite");
+    HVO_CHECK_ARG(n >= 0 && (n == 0 || (xy && xy_un)), "null argument");
+    for (int i = 0; i < n; ++i) undistort_point(*cam, xy[2 * i], xy[2 * i + 1], &xy_un[2 * i], &xy_un[2 * i + 1]);
+    return HVO_OK;
+}
+
+int hvo_image_bounds(const hvo_camera* cam, int width, int height, float* min_x, float* max_x, float* min_y, float* max_y) {
+    HVO_CHECK_ARG(camera_ok(cam), "camera missing or fx / fy zero or not finite");
+    HVO_CHECK_ARG(min_x && max_x && min_y && max_y && width > 0 && height > 0, "bad argument");
+    if (cam->k1 == 0.f) {   // the reference tests mDistCoef.at<float>(0) only
+        *min_x = 0.f; *max_x = (float)width; *min_y = 0.f; *max_y = (float)height;
+        return HVO_OK;
+    }
+    const float c[8] = {0.f, 0.f, (float)width, 0.f, 0.f, (float)height, (float)width, (float)height};
+    float u[8];
+    for (int i = 0; i < 4; ++i) undistort_point(*cam, c[2 * i], c[2 * i + 1], &u[2 * i], &u[2 * i + 1]);
+    *min_x = std::min(u[0], u[4]); *max_x = std::max(u[2], u[6]);
+    *min_y = std::min(u[1], u[3]); *max_y = std::max(u[5], u[7]);
+    return HVO_OK;
+}
+
+int hvo_orb_undistort_batch_device(hvo_orb* h, const hvo_camera* cam, const hvo_keypoint* d_kps, const int32_t* d_counts, int nframes,
+                                   const float* d_kp_depth, float bf, hvo_keypoint* d_kps_un, float* d_kp_uright) {
+    HVO_CHECK_ARG(h, "null handle");
+    HVO_CHECK_ARG(camera_ok(cam), "camera missing or fx / fy zero or not finite");
+    HVO_CHECK_ARG(d_kps && d_counts, "null device buffer");
+    HVO_CHECK_ARG(!d_kp_uright || d_kp_depth, "kp_uright needs kp_depth");
+    HVO_CHECK_ARG(nframes >= 1 && nframes <= 65535, "nframes out of range (1..65535)");
+    HVO_CUDA(cudaSetDevice(h->device));
+    return h->undistort(*cam, d_kps, d_counts, nframes, d_kp_depth, bf, d_kps_un, d_kp_uright);
 }
 
 int hvo_orb_last_launches(const hvo_orb* h) { return h ? h->last_launches : 0; }

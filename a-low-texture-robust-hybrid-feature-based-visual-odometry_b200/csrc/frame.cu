@@ -98,6 +98,8 @@ struct hvo_frame {
     int next_lane = 0;   // host API: lane of the next chunk (round-robin across calls)
     int* d_fault = nullptr;   // {first faulty frame, pipeline codes}, sticky until read
     int* h_fault = nullptr;   // pinned copy
+    bool undistort = false;   // distorted camera with coefficients: mvKeysUn / mvuRight are formed on the device
+    hvo_camera cam{};
 };
 
 static const int kNoFault = 0x7fffffff;
@@ -122,6 +124,7 @@ static hvo_frame_outputs outputs_at(const hvo_frame* h, const hvo_frame_outputs&
     if (o.membership4) r.membership4 = o.membership4 + off * (px / 2);
     if (o.normals8) r.normals8 = o.normals8 + off * (size_t)h->normals_count * 8;
     if (o.normals3) r.normals3 = o.normals3 + off * (size_t)h->normals_count * 3;
+    if (o.kps_un) r.kps_un = o.kps_un + off * c;
     return r;
 }
 
@@ -193,6 +196,11 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
         int st = hvo_orb_extract_batch_device(L.orb, d_gray, n, o.kps, o.desc, o.kp_counts, d_depth, &rg, o.kp_depth, o.kp_uright);
         if (st != HVO_OK) return st;
         *launches += hvo_orb_last_launches(L.orb) + 1;
+        if (h->undistort) {
+            st = hvo_orb_undistort_batch_device(L.orb, &h->cam, o.kps, o.kp_counts, n, o.kp_depth, h->p.bf, o.kps_un, o.kp_uright);
+            if (st != HVO_OK) return st;
+            ++*launches;
+        }
         k_frame_fold_status<<<1, 32, 0, s>>>(orb_error_flag(L.orb), 1, 1, 0, base, FAULT_ORB, h->d_fault);   // one flag per chunk
         HVO_CUDA(cudaMemsetAsync(orb_error_flag(L.orb), 0, sizeof(int), s));
         HVO_CUDA(cudaEventRecord(L.cdone[0], s));
@@ -255,6 +263,7 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
             HVO_CUDA(cudaMemcpyAsync(host->desc, o.desc, N * c * 32, cudaMemcpyDeviceToHost, s));
             if (host->kp_depth) HVO_CUDA(cudaMemcpyAsync(host->kp_depth, o.kp_depth, N * c * 4, cudaMemcpyDeviceToHost, s));
             if (host->kp_uright) HVO_CUDA(cudaMemcpyAsync(host->kp_uright, o.kp_uright, N * c * 4, cudaMemcpyDeviceToHost, s));
+            if (host->kps_un) HVO_CUDA(cudaMemcpyAsync(host->kps_un, o.kps_un, N * c * sizeof(hvo_keypoint), cudaMemcpyDeviceToHost, s));
         }
         timeline_mark(s, "end_orb");
         HVO_CUDA(cudaEventRecord(L.join[0], s));
@@ -335,6 +344,8 @@ int hvo_frame_create(const hvo_frame_params* p, int width, int height, int max_b
     hvo_frame* h = new (std::nothrow) hvo_frame();
     if (!h) { set_error("out of host memory"); return HVO_ERR_ARG; }
     h->p = *p; h->device = device; h->width = width; h->height = height; h->max_batch = max_batch;
+    h->undistort = p->distorted != 0 && (p->k1 != 0.f || p->k2 != 0.f || p->p1 != 0.f || p->p2 != 0.f || p->k3 != 0.f);
+    h->cam = hvo_camera{p->fx, p->fy, p->cx, p->cy, p->k1, p->k2, p->p1, p->p2, p->k3};
     // default: two lanes once a chunk still holds >= 1024 frames (measured on B200: the ordered kernels, one warp / CTA per
     // frame, need about that many frames per launch; 4 x 256 is 25 % slower than 1 x 1024)
     int nl = p->lanes > 0 ? p->lanes : (max_batch >= 2048 ? 2 : 1);
@@ -412,6 +423,7 @@ int hvo_frame_create(const hvo_frame_params* p, int width, int height, int max_b
                 HVO_TRY(cudaMalloc(&o.kp_counts, B * 4));
                 HVO_TRY(cudaMalloc(&o.kp_depth, B * c * 4));
                 HVO_TRY(cudaMalloc(&o.kp_uright, B * c * 4));
+                if (h->undistort) HVO_TRY(cudaMalloc(&o.kps_un, B * c * sizeof(hvo_keypoint)));
             }
             if (L.line) {
                 const size_t c = (size_t)h->max_lines;
@@ -455,7 +467,7 @@ void hvo_frame_destroy(hvo_frame* h) {
         if (L.fork_depth) cudaEventDestroy(L.fork_depth);
         hvo_frame_outputs& o = L.d_out;
         void* bufs[] = {L.d_gray, L.d_depth, o.kps, o.desc, o.kp_counts, o.kp_depth, o.kp_uright, o.keylines, o.line_desc, o.linevec3,
-                        o.line_counts, o.n_planes, o.planes7, o.membership, o.membership8, o.normals8, o.membership4, o.normals3};
+                        o.line_counts, o.n_planes, o.planes7, o.membership, o.membership8, o.normals8, o.membership4, o.normals3, o.kps_un};
         for (void* b : bufs) if (b) cudaFree(b);
         if (L.fork) cudaEventDestroy(L.fork);
         for (auto& e : L.join) if (e) cudaEventDestroy(e);
@@ -491,6 +503,7 @@ static int frame_check_outputs(const hvo_frame* h, const hvo_frame_outputs* o, b
     if (h->p.stages & ST_LINE) HVO_CHECK_ARG(o->keylines && o->line_desc && o->line_counts, "line outputs missing");
     if (h->p.stages & ST_PLANE) HVO_CHECK_ARG(o->n_planes && o->planes7 && (o->membership || (!device && (o->membership8 || o->membership4))), "plane outputs missing");
     if (h->p.stages & ST_NORMALS) HVO_CHECK_ARG(o->normals8 || (!device && o->normals3), "normals output missing");
+    if (o->kps_un) HVO_CHECK_ARG(h->undistort && (h->p.stages & ST_ORB), "kps_un needs the ORB stage and a distorted camera with coefficients");
     if (o->membership4) {
         HVO_CHECK_ARG(h->p.max_planes <= 15, "membership4 needs max_planes <= 15");
         HVO_CHECK_ARG(((size_t)h->width * h->height) % 16 == 0, "membership4 needs width * height divisible by 16");
@@ -563,6 +576,7 @@ int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint1
         if (!out->membership8 && !out->membership4) d.membership8 = nullptr;
         if (!out->membership4) d.membership4 = nullptr;
         if (!out->normals3) d.normals3 = nullptr;
+        if (!out->kps_un) d.kps_un = nullptr;
         const hvo_frame_outputs hostk = outputs_at(h, *out, (size_t)off);
         st = lane_launch(h, L, L.fork, L.fork_depth, L.d_gray, L.d_depth, n, off, d, &hostk, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
         if (st != HVO_OK) return st;

@@ -11,10 +11,15 @@
 //                               patch in shared memory (.cc:1083-1084), steered rBRIEF-256 (.cc:106-144),
 //                               KeyPoint assembly (.cc:835-846,1093-1099), RGB-D depth lookup
 //                               (Frame.cc:1940-1961) - no blurred pyramid in HBM
+//   k_undistort_kps x1          distorted cameras only: one thread per keypoint, Frame::UndistortKeyPoints
+//                               (Frame.cc:1701-1731, cv::undistortPoints in FP64, undistort.cuh) and mvuRight from the
+//                               undistorted x.  A kernel of its own: five dependent FP64 iterations on lane 0 of
+//                               k_describe would lengthen every describe warp
 //
 // Float semantics are pinned with explicit round-to-nearest intrinsics (no FMA contraction) so that
 // angles, sample coordinates and scaled keypoint positions are bit-identical to the CPU oracle.
 #include "orb.cuh"
+#include "undistort.cuh"
 
 #include <algorithm>
 #include <cfloat>
@@ -916,6 +921,23 @@ __global__ void __launch_bounds__(kDescWarps * 32) k_describe(const __grid_const
     }
 }
 
+// Frame::UndistortKeyPoints (Frame.cc:1701-1731) and the mvuRight of ComputeStereoFromRGBD (:1953-1958) on the keypoints k_describe
+// wrote: row i of frame blockIdx.y, rows at or past counts[f] untouched.  kp_depth > 0 exactly where k_describe found 0 < d < 7.
+__global__ void __launch_bounds__(128) k_undistort_kps(const hvo_camera cam, int cap, const hvo_keypoint* __restrict__ kps,
+                                                       const int32_t* __restrict__ counts, const float* __restrict__ kp_depth, float bf,
+                                                       hvo_keypoint* __restrict__ kps_un, float* __restrict__ kp_uright) {
+    const int f = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= min(counts[f], cap)) return;
+    const long long o = (long long)f * cap + i;
+    hvo_keypoint k = kps[o];
+    if (cam.k1 != 0.f) undistort_point(cam, k.x, k.y, &k.x, &k.y);   // the reference tests k1 only (Frame.cc:1703)
+    if (kps_un) kps_un[o] = k;
+    if (kp_uright) {
+        const float d = kp_depth[o];
+        kp_uright[o] = d > 0.f ? __fsub_rn(k.x, __fdiv_rn(bf, d)) : -1.f;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------
@@ -1188,5 +1210,14 @@ int hvo_orb::run(const uint8_t* d_gray, int nframes, hvo_keypoint* d_kps_out, ui
     if (profiling) { HVO_CUDA(cudaEventRecord(ev[5], stream)); have_stage_times = true; }
     HVO_CUDA(cudaGetLastError());
     last_launches = launches;
+    return HVO_OK;
+}
+
+int hvo_orb::undistort(const hvo_camera& cam, const hvo_keypoint* d_kps, const int32_t* d_counts, int nframes, const float* d_kp_depth,
+                       float bf, hvo_keypoint* d_kps_un, float* d_kp_uright) {
+    timeline_mark(stream, "k_undistort_kps");
+    k_undistort_kps<<<dim3(div_up(g.out_cap, 128), nframes), 128, 0, stream>>>(cam, g.out_cap, d_kps, d_counts, d_kp_depth, bf, d_kps_un,
+                                                                              d_kp_uright);
+    HVO_CUDA(cudaGetLastError());
     return HVO_OK;
 }

@@ -84,4 +84,6 @@ struct hvo_orb {
     void release();
     int run(const uint8_t* d_gray, int nframes, hvo_keypoint* d_kps_out, uint8_t* d_desc_out, int32_t* d_counts_out,
             const uint16_t* d_depth16, const hvo_rgbd_params* rgbd, float* d_kp_depth, float* d_kp_uright);
+    int undistort(const hvo_camera& cam, const hvo_keypoint* d_kps, const int32_t* d_counts, int nframes, const float* d_kp_depth, float bf,
+                  hvo_keypoint* d_kps_un, float* d_kp_uright);
 };

@@ -41,6 +41,7 @@ static hvo_frame_outputs seq_outputs_at(const hvo_seq* s, const hvo_frame_output
     if (o.membership4) r.membership4 = o.membership4 + off * (px / 2);
     if (o.normals8) r.normals8 = o.normals8 + off * nc * 8;
     if (o.normals3) r.normals3 = o.normals3 + off * nc * 3;
+    if (o.kps_un) r.kps_un = o.kps_un + off * c;
     return r;
 }
 

@@ -63,20 +63,40 @@ typedef struct hvo_keypoint {
 /* Optional RGB-D epilogue = Frame::ComputeStereoFromRGBD (src/Frame.cc:1940-1961) fused after extraction.
  * depth is raw 16-bit (TUM: metres*5000); depth_factor = 1/DepthMapFactor (src/Tracking.cc:156-160).
  * kp_depth (mvDepth) is sampled at the DISTORTED keypoint, as the reference does (Frame.cc:1948-1951), and is always valid.
- * kp_uright (mvuRight) is kpU.pt.x - bf / d with kpU the UNDISTORTED keypoint (Frame.cc:1944, 1957).  Undistortion
- * (Frame::UndistortKeyPoints, Frame.cc:1701-1731, cv::undistortPoints) stays on the host, so the device can form mvuRight only
- * for a camera without distortion (mvKeysUn == mvKeys, Frame.cc:1703-1707): set `distorted` for any other camera (TUM1.yaml,
- * TUM2.yaml, ICSL_LPVO.yaml have k1 != 0); kp_uright is then filled with -1 and the caller forms it after UndistortKeyPoints with
- * hvo_stereo_uright_from_depth(). */
+ * kp_uright (mvuRight) is kpU.pt.x - bf / d with kpU the UNDISTORTED keypoint (Frame.cc:1944, 1957).  The extract calls form it
+ * only for a camera without distortion (mvKeysUn == mvKeys, Frame.cc:1703-1707).  For any other camera (TUM1.yaml, TUM2.yaml,
+ * ICSL_LPVO.yaml have k1 != 0) set `distorted`: kp_uright is then filled with -1, and hvo_orb_undistort_batch_device() forms
+ * mvKeysUn and mvuRight on the device right after the extraction (the frame handle does this itself when hvo_frame_params
+ * carries the coefficients).  hvo_stereo_uright_from_depth() is the host form for keypoints undistorted elsewhere. */
 typedef struct hvo_rgbd_params {
     float depth_factor; /* metres per raw unit, e.g. 1/5000 */
     float bf;           /* stereo baseline * fx (Camera.bf) */
-    int distorted;      /* != 0: Camera.k1 != 0, kp_uright is not formed on the device */
+    int distorted;      /* != 0: Camera.k1 != 0, kp_uright is not formed by the extract call */
 } hvo_rgbd_params;
 
 /* mvuRight of a distorted camera, host side: uright[i] = keys_un[i].x - bf / kp_depth[i] where kp_depth[i] > 0, else -1
  * (the second half of Frame::ComputeStereoFromRGBD, Frame.cc:1953-1958, on the undistorted keypoints). */
 int hvo_stereo_uright_from_depth(const hvo_keypoint* keys_un, const float* kp_depth, int n, float bf, float* uright);
+
+/* mK and mDistCoef as the reference holds them (CV_32F): DistCoef = k1, k2, p1, p2, and k3 when Camera.k3 != 0 (k3 = 0 otherwise). */
+typedef struct hvo_camera {
+    float fx, fy, cx, cy;
+    float k1, k2, p1, p2, k3;
+} hvo_camera;
+
+/* cv::undistortPoints(xy, xy_un, mK, mDistCoef, noArray(), mK) of OpenCV 4.13, bit for bit: xy / xy_un are n (x, y) float pairs
+ * (may alias).  Plain cv::undistortPoints, without the k1 == 0 shortcut of Frame::UndistortKeyPoints.  Host function, no CUDA. */
+int hvo_undistort_points(const hvo_camera* cam, const float* xy, int n, float* xy_un);
+/* Frame::ComputeImageBounds (src/Frame.cc:1733-1760): mnMinX = min of the undistorted corners (0,0), (0,rows); mnMaxX = max of
+ * (cols,0), (cols,rows); likewise in y.  k1 == 0 gives 0, width, 0, height, as the reference tests only k1.  Host function. */
+int hvo_image_bounds(const hvo_camera* cam, int width, int height, float* min_x, float* max_x, float* min_y, float* max_y);
+/* Frame::UndistortKeyPoints + the mvuRight half of ComputeStereoFromRGBD on device-resident extraction results, asynchronous on the
+ * handle's stream (so it follows a hvo_orb_extract_batch_device call in order).  Rows [f][i] with i < d_counts[f] of the
+ * [nframes][hvo_orb_capacity] arrays are read; d_kps_un (may be NULL) receives the keypoint with x, y undistorted; d_kp_uright (may
+ * be NULL, needs d_kp_depth) receives x_un - bf / d where d_kp_depth > 0, else -1.  k1 == 0: kps_un = kps, as the reference.  Rows past
+ * the count are not written. */
+int hvo_orb_undistort_batch_device(hvo_orb* h, const hvo_camera* cam, const hvo_keypoint* d_kps, const int32_t* d_counts, int nframes,
+                                   const float* d_kp_depth, float bf, hvo_keypoint* d_kps_un, float* d_kp_uright);
 
 /* Create an extractor for frames of width x height, up to max_batch frames per call, on CUDA `device`. */
 int hvo_orb_create(const hvo_orb_params* params, int width, int height, int max_batch, int device, hvo_orb** out);
@@ -562,7 +582,8 @@ typedef struct hvo_frame_params {
     float fx, fy, cx, cy; /* Camera.* */
     float depth_factor;   /* 1 / DepthMapFactor */
     float bf;             /* Camera.bf */
-    int distorted;        /* != 0: Camera.k1 != 0 (see hvo_rgbd_params): kp_uright is filled with -1 */
+    int distorted;        /* != 0: Camera.k1 != 0 (see hvo_rgbd_params): with all coefficients below 0, kp_uright is filled with -1;
+                             with a non-zero coefficient the handle undistorts on the device (kps_un, kp_uright) */
     int stages;           /* HVO_STAGE_* bits */
     int max_planes;       /* rows of planes7 per frame */
     int line_cull;        /* != 0: Frame::cullingLine after the line extractor, as Frame::ExtractLSD does (src/Frame.cc:939) */
@@ -572,6 +593,7 @@ typedef struct hvo_frame_params {
                              own scratch exists once (chunk-sized): the kernels of consecutive chunks run one after the other.
                              A chunk of >= 2048 frames runs its pipelines one after the other (planes, lines, ORB, normals), each
                              alone at its saturating batch; smaller chunks run them side by side (lowest latency). */
+    float k1, k2, p1, p2, k3; /* Camera.k1 .. k3 (mDistCoef, see hvo_camera); all 0 = no undistortion on the device */
 } hvo_frame_params;
 
 /* Output arrays of a batch of n frames.  Host pointers for hvo_frame_extract_batch, device pointers for
@@ -597,6 +619,8 @@ typedef struct hvo_frame_outputs {
                                                      max_planes <= 15 and an even H*W.  hvo_membership4_expand() restores labels */
     float* normals3;       /* [n][normals_count][3]  the normal only (NaN = none); position and pixel of a SurfaceNormal are
                                                      functions of (m, n) and the depth: hvo_normals3_expand() restores normals8 */
+    hvo_keypoint* kps_un;  /* [n][orb_capacity]      mvKeysUn (Frame::UndistortKeyPoints)   optional; only for a handle created
+                                                     with distorted != 0 and a non-zero coefficient                  */
 } hvo_frame_outputs;
 
 /* Host-side expanders of the compact outputs (plain C loops, no CUDA). */
