@@ -89,6 +89,8 @@ ABI = {
     'hvo_seq_capacities': (C.c_int, [_vp, _vp, _vp, _vp]),
     'hvo_seq_shard': (None, [C.c_int, C.c_int, C.c_int, _vp, _vp]),
     'hvo_seq_extract': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp]),
+    'hvo_seq_set_vocabulary': (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int]),
+    'hvo_seq_extract_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
     'hvo_seq_last_ms': (C.c_float, [_vp]),
     'hvo_normals3_expand': (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp]),
     'hvo_orb_level_size': (C.c_int, [_vp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
@@ -209,6 +211,10 @@ ABI = {
     'hvo_frame_extract_batch': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp]),
     'hvo_frame_extract_batch_async': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp]),
     'hvo_frame_extract_batch_device': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp]),
+    'hvo_frame_set_vocabulary': (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int]),
+    'hvo_frame_extract_batch_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
+    'hvo_frame_extract_batch_async_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
+    'hvo_frame_extract_batch_device_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
     'hvo_frame_last_launches': (C.c_int, [_vp]),
     'hvo_frame_sync': (C.c_int, [_vp]),
     'hvo_frame_timer_start': (C.c_int, [_vp]),
@@ -1314,6 +1320,16 @@ assert PROJ_QUERY_DTYPE.itemsize == 32
 GRID_COLS, GRID_ROWS = 64, 48
 
 
+def _vocabulary_args(voc):
+    """The vocabulary dict as the leading arguments of hvo_bow_set_vocabulary (n_nodes, child_start, child_ids, node_desc, node_weight,
+    node_word, depth_levels); the arrays are returned as well, to be kept alive over the call."""
+    cs = np.ascontiguousarray(voc['child_start'], np.int32); ci = np.ascontiguousarray(voc['child_ids'], np.int32)
+    nd = np.ascontiguousarray(voc['node_desc'], np.uint8); nw = np.ascontiguousarray(voc['node_weight'], np.float64)
+    wd = np.ascontiguousarray(voc['node_word'], np.int32)
+    args = (len(nw), _np_ptr(cs), _np_ptr(ci) if len(ci) else None, _np_ptr(nd), _np_ptr(nw), _np_ptr(wd), int(voc['L']))
+    return args, (cs, ci, nd, nw, wd)
+
+
 class ORBVocabulary:
     """Mirror of ORB_SLAM2::ORBVocabulary (= DBoW2::TemplatedVocabulary<FORB::TDescriptor, FORB>, reference include/ORBVocabulary.h) for the
     one call on the path, transform(features, BowVector, FeatureVector, levelsup) as used by Frame::ComputeBoW (src/Frame.cc:1692-1699).
@@ -1323,11 +1339,8 @@ class ORBVocabulary:
         out = _vp()
         _check(lib().hvo_bow_create(int(device), C.byref(out)))
         self._h = out
-        cs = np.ascontiguousarray(voc['child_start'], np.int32); ci = np.ascontiguousarray(voc['child_ids'], np.int32)
-        nd = np.ascontiguousarray(voc['node_desc'], np.uint8); nw = np.ascontiguousarray(voc['node_weight'], np.float64)
-        wd = np.ascontiguousarray(voc['node_word'], np.int32)
-        _check(lib().hvo_bow_set_vocabulary(self._h, len(nw), _np_ptr(cs), _np_ptr(ci) if len(ci) else None, _np_ptr(nd), _np_ptr(nw), _np_ptr(wd),
-                                            int(voc['L'])))
+        args, _keep = _vocabulary_args(voc)
+        _check(lib().hvo_bow_set_vocabulary(self._h, *args))
 
     def close(self):
         if getattr(self, '_h', None):
@@ -1921,21 +1934,29 @@ class _FrameOutputs(C.Structure):
                                    'line_counts', 'n_planes', 'planes7', 'membership', 'normals8', 'membership8', 'membership4', 'normals3', 'kps_un')]
 
 
+class _FrameBowOutputs(C.Structure):
+    _fields_ = [(n, _vp) for n in ('bow_counts', 'bow_words', 'bow_values', 'fv_order', 'fv_counts', 'node_of', 'word_of')]
+
+
 class FrameFrontEnd:
     """The extraction part of ORB_SLAM2::Frame::Frame(imGray, imDepth, ...) (reference src/Frame.cc:188-233): ORB + RGB-D
     depth lookup, LSD/LBD lines, PEAC planes and surface normals of a batch of frames, three concurrent CUDA streams."""
     FIELDS = [f[0] for f in _FrameOutputs._fields_]
+    BOW_FIELDS = [f[0] for f in _FrameBowOutputs._fields_]
+    vocabulary = None
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, bf=40.0, nfeatures=1000, scale_factor=1.2, nlevels=8, ini_th=20,
                  min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=16, max_batch=1, device=0, line_cull=False, lanes=0, membership='i32',
-                 distorted=False, normals='n8', dist=None):
+                 distorted=False, normals='n8', dist=None, vocabulary=None, levelsup=4):
         """membership: 'i32' (int32 labels, -1 = none), 'u8' (one byte per pixel, 255 = none: what a host caller needs to
         rebuild plane_vertices_), 'both', or 'u4' (host calls only: two pixels per byte, 15 = none, max_planes <= 15; expand with
         membership4_expand).  The int32 image is always the device-side working image.
         normals: 'n8' (SurfaceNormal rows: normal, position, pixel) or 'n3' (host calls only: the normal alone; normals3_expand
         rebuilds the rows from the depth image).
         dist: mDistCoef (k1, k2, p1, p2 [, k3]).  With a non-zero coefficient the handle runs Frame::UndistortKeyPoints on the device:
-        kp_uright is formed from the undistorted keypoints and the outputs gain kps_un (mvKeysUn)."""
+        kp_uright is formed from the undistorted keypoints and the outputs gain kps_un (mvKeysUn).
+        vocabulary: the dict ORBVocabulary takes.  Every frame then also gets what Frame::ComputeBoW computes, transform(mDescriptors,
+        mBowVec, mFeatVec, levelsup), on the device right after its descriptors: the outputs gain the BoW arrays (see bow())."""
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
@@ -1950,6 +1971,19 @@ class FrameFrontEnd:
         self.orb_capacity, self.max_lines, self.normals_count = a.value, b.value, c.value
         _check(lib().hvo_frame_lanes(out, C.byref(a), C.byref(b)))
         self.lanes, self.chunk = a.value, b.value
+        if vocabulary is not None:
+            self.set_vocabulary(vocabulary, levelsup)
+
+    def set_vocabulary(self, vocabulary, levelsup=4):
+        """Attach a vocabulary (the dict ORBVocabulary takes) or, with None, detach it (hvo_frame_set_vocabulary / hvo_seq_set_vocabulary)."""
+        f, h = (lib().hvo_seq_set_vocabulary, self._seq) if getattr(self, '_seq', None) else (lib().hvo_frame_set_vocabulary, self._h)
+        self.vocabulary = None
+        if vocabulary is None:
+            _check(f(h, 0, None, None, None, None, None, 0, 0))
+            return
+        args, _keep = _vocabulary_args(vocabulary)
+        _check(f(h, *args, int(levelsup)))
+        self.vocabulary, self.levelsup = vocabulary, int(levelsup)
 
     def _params(self, fx, fy, cx, cy, depth_factor, bf, nfeatures, scale_factor, nlevels, ini_th, min_th, n_lines, stages, max_planes,
                 line_cull, lanes, distorted, dist):
@@ -1980,6 +2014,9 @@ class FrameFrontEnd:
                       kp_uright=((n, c), np.float32))
             if self.undistorts:
                 sh.update(kps_un=((n, c), KP_DTYPE))
+            if self.vocabulary is not None:
+                sh.update(bow_counts=((n,), np.int32), bow_words=((n, c), np.int32), bow_values=((n, c), np.float64), fv_order=((n, c), np.int32),
+                          fv_counts=((n,), np.int32), node_of=((n, c), np.int32), word_of=((n, c), np.int32))
         if self.stages & STAGE_LINES:
             c = self.max_lines
             sh.update(keylines=((n, c), KL_DTYPE), line_desc=((n, c, 32), np.uint8), linevec3=((n, c, 3), np.float64),
@@ -2027,6 +2064,25 @@ class FrameFrontEnd:
             setattr(o, k, ptrs.get(k))
         return o
 
+    def _bow_outputs(self, ptrs):
+        """hvo_frame_bow_outputs by reference, or None without a vocabulary (the call then computes no BoW)."""
+        if self.vocabulary is None:
+            return None
+        o = _FrameBowOutputs()
+        for k in self.BOW_FIELDS:
+            setattr(o, k, ptrs.get(k))
+        return C.byref(o)
+
+    @staticmethod
+    def bow(out, f):
+        """Frame f's mBowVec / mFeatVec from the outputs of a handle with a vocabulary: ((words, values), {node: [feature, ...]}), the
+        form of ORBVocabulary.transform()[:2]."""
+        nw, nf = int(out['bow_counts'][f]), int(out['fv_counts'][f])
+        fv = {}
+        for i in out['fv_order'][f, :nf]:
+            fv.setdefault(int(out['node_of'][f, i]), []).append(int(i))
+        return (out['bow_words'][f, :nw].copy(), out['bow_values'][f, :nw].copy()), fv
+
     def extract_batch(self, gray, depth16, out=None, wait=True):
         """gray [n,h,w] uint8, depth16 [n,h,w] uint16 (host) -> dict of host arrays (see output_shapes).  wait=False queues the
         call and returns (pinned buffers, untouched until sync()): the next call's uploads overlap this call's tail."""
@@ -2039,9 +2095,10 @@ class FrameFrontEnd:
             out = self.alloc_host(n)
         else:   # the C side writes through raw pointers: every caller-supplied array must have the exact layout
             self._check_out(out, self.output_shapes(n, device=False))
-        o = self._outputs({k: v.ctypes.data for k, v in out.items()})
-        f = lib().hvo_frame_extract_batch if wait else lib().hvo_frame_extract_batch_async
-        _check(f(self._h, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o)))
+        ptrs = {k: v.ctypes.data for k, v in out.items()}
+        o = self._outputs(ptrs)
+        f = lib().hvo_frame_extract_batch_bow if wait else lib().hvo_frame_extract_batch_async_bow
+        _check(f(self._h, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs)))
         return out
 
     @staticmethod
@@ -2054,7 +2111,7 @@ class FrameFrontEnd:
     def extract_batch_device(self, d_gray, d_depth16, n, d_ptrs):
         """d_ptrs: name -> device pointer (int) for every output of output_shapes(n).  Asynchronous."""
         o = self._outputs(d_ptrs)
-        _check(lib().hvo_frame_extract_batch_device(self._h, _vp(d_gray), _vp(d_depth16), n, C.byref(o)))
+        _check(lib().hvo_frame_extract_batch_device_bow(self._h, _vp(d_gray), _vp(d_depth16), n, C.byref(o), self._bow_outputs(d_ptrs)))
 
     def last_launches(self):
         return lib().hvo_frame_last_launches(self._h)
@@ -2078,7 +2135,7 @@ class FrameSequence(FrameFrontEnd):
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, devices, frames_per_call=2368, bf=40.0, nfeatures=1000, scale_factor=1.2,
                  nlevels=8, ini_th=20, min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=15, line_cull=True, lanes=0, membership='u4',
-                 normals='n3', distorted=False, dist=None):
+                 normals='n3', distorted=False, dist=None, vocabulary=None, levelsup=4):
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
@@ -2094,6 +2151,8 @@ class FrameSequence(FrameFrontEnd):
         a, b, c = C.c_int(0), C.c_int(0), C.c_int(0)
         _check(lib().hvo_seq_capacities(out, C.byref(a), C.byref(b), C.byref(c)))
         self.orb_capacity, self.max_lines, self.normals_count = a.value, b.value, c.value
+        if vocabulary is not None:
+            self.set_vocabulary(vocabulary, levelsup)
 
     def close(self):
         if getattr(self, '_seq', None):
@@ -2115,10 +2174,11 @@ class FrameSequence(FrameFrontEnd):
             raise HvoError(HVO_ERR_ARG, f'gray / depth16 must be [n, {self.h}, {self.w}]')
         if out is None:
             out = self.alloc_host(n)
-        else:   # kps_un at least: the other arrays' check is a separate change
-            self._check_out(out, {k: v for k, v in self.output_shapes(n, device=False).items() if k == 'kps_un'})
-        o = self._outputs({k: v.ctypes.data for k, v in out.items()})
-        _check(lib().hvo_seq_extract(self._seq, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o)))
+        else:   # kps_un and the BoW arrays at least: the other arrays' check is a separate change
+            self._check_out(out, {k: v for k, v in self.output_shapes(n, device=False).items() if k == 'kps_un' or k in self.BOW_FIELDS})
+        ptrs = {k: v.ctypes.data for k, v in out.items()}
+        o = self._outputs(ptrs)
+        _check(lib().hvo_seq_extract_bow(self._seq, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs)))
         return out
 
     def last_ms(self):

@@ -4,14 +4,19 @@
 // BowVector::addWeight / normalize BowVector.cpp:33-83, FeatureVector::addFeature FeatureVector.cpp) for the vocabulary ORB-SLAM2 uses:
 // TF-IDF weights, L1 scoring (so the vector is L1-normalised at the end).
 //
-//   k_bow_descend   one warp per descriptor: at every level the children of the current node are scored 32 at a time (8 x __popc per
-//                   lane), the first child of minimum distance wins (strict '<' in child order, as in the reference), until a leaf;
-//                   the node passed at level L - levelsup is kept for the FeatureVector
+//   k_bow_descend   one tile of T = 8, 16 or 32 lanes per descriptor (the smallest that holds the vocabulary's largest branching
+//                   factor; wider nodes are scored T children at a time): at every level the children of the current node are scored
+//                   (8 x __popc per lane), the first child of minimum distance wins (strict '<' in child order, as in the reference),
+//                   until a leaf; the node passed at level L - levelsup is kept for the FeatureVector
 //   k_bow_frame     one CTA per frame: (word, feature) keys sorted in shared memory; one thread per distinct word accumulates its
 //                   weights in feature order (value = w; value += w ...: the additions BowVector::addWeight performs), words are
 //                   compacted in ascending order (std::map order), one thread sums |value| in that order (BowVector::normalize L1)
 //                   and every value is divided by the norm; a second sort by (node, feature) gives the FeatureVector order
 // All floating point is double, one rounding per operation, in the reference's order: the vectors are bit-identical.
+//
+// Both kernels serve two layouts of the descriptor rows (BowRows): the compact one of hvo_bow_transform (frame f = rows offsets[f] ..
+// offsets[f+1]) and the frame handle's (frame f = rows f * orb_capacity .., kp_counts[f] of them, the counts read on the device).  Rows
+// at or past a frame's count are neither read nor written.
 #include <algorithm>
 #include <climits>
 #include <new>
@@ -22,20 +27,33 @@ namespace hvo {
 
 static const int kBowMaxFeatures = 4096;   // per frame (shared-memory sort)
 
-__global__ void __launch_bounds__(128) k_bow_descend(const uint4* __restrict__ desc, int total, const int* __restrict__ child_start,
+// frame f = rows base(f) .. base(f) + count(f) of the per-row arrays
+struct BowRows {
+    const int* offsets;   // compact layout: base = offsets[f], count = offsets[f+1] - offsets[f]
+    const int* counts;    // otherwise: base = f * stride, count = counts[f]
+    int stride;
+    __device__ __forceinline__ int base(int f) const { return offsets ? offsets[f] : f * stride; }
+    __device__ __forceinline__ int count(int f) const { return offsets ? offsets[f + 1] - offsets[f] : counts[f]; }
+    __device__ __forceinline__ bool valid(int i) const { return offsets || i % stride < counts[i / stride]; }   // i < total
+};
+
+template <int T>
+__global__ void __launch_bounds__(128) k_bow_descend(const uint4* __restrict__ desc, BowRows rows, int total, const int* __restrict__ child_start,
                                                      const int* __restrict__ child_ids, const uint4* __restrict__ node_desc,
                                                      const double* __restrict__ node_weight, const int* __restrict__ node_word, int nid_level,
                                                      int* __restrict__ word_of, int* __restrict__ node_of, double* __restrict__ weight_of) {
-    const int i = (blockIdx.x * 128 + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (i >= total) return;
-    const uint4 qa = desc[2 * i], qb = desc[2 * i + 1];
+    const int i = (int)(((long long)blockIdx.x * 128 + threadIdx.x) / T), lane = threadIdx.x & (T - 1);
+    if (i >= total || !rows.valid(i)) return;   // the whole tile leaves together
+    const unsigned tile = T == 32 ? 0xffffffffu : ((1u << T) - 1u) << (threadIdx.x & 31 & ~(T - 1));
+    const uint4 qa = desc[2 * (size_t)i], qb = desc[2 * (size_t)i + 1];
     int cur = 0, level = 0, nid = 0;   // nid stays the root when nid_level <= 0 (TemplatedVocabulary.h:1240)
     while (true) {
         const int b = child_start[cur], e = child_start[cur + 1];
         if (b == e) break;             // leaf
         ++level;
-        unsigned best = 0xffffffffu;   // (distance << 16 | position among the children): the minimum is the first child of least distance
-        for (int base = b; base < e; base += 32) {
+        unsigned best = 0xffffffffu;   // (distance << 16 | position among the children): the minimum is the first child of least distance,
+                                       // whatever the tile width
+        for (int base = b; base < e; base += T) {
             const int c = base + lane;
             unsigned key = 0xffffffffu;
             if (c < e) {
@@ -45,7 +63,7 @@ __global__ void __launch_bounds__(128) k_bow_descend(const uint4* __restrict__ d
                               __popc(qb.y ^ db.y) + __popc(qb.z ^ db.z) + __popc(qb.w ^ db.w);
                 key = ((unsigned)d << 16) | (unsigned)(c - b);
             }
-            best = min(best, __reduce_min_sync(0xffffffffu, key));
+            best = min(best, __reduce_min_sync(tile, key));
         }
         cur = child_ids[b + (int)(best & 0xffffu)];
         if (level == nid_level) nid = cur;
@@ -73,7 +91,7 @@ __device__ __forceinline__ void bow_bitonic_sort(unsigned long long* key, int N)
         }
 }
 
-__global__ void __launch_bounds__(256) k_bow_frame(const int* __restrict__ offsets, const int* __restrict__ word_of, const int* __restrict__ node_of,
+__global__ void __launch_bounds__(256) k_bow_frame(BowRows rows, const int* __restrict__ word_of, const int* __restrict__ node_of,
                                                    const double* __restrict__ weight_of, int* __restrict__ bow_counts, int* __restrict__ bow_words,
                                                    double* __restrict__ bow_values, int* __restrict__ fv_order, int* __restrict__ fv_counts) {
     extern __shared__ unsigned long long key[];   // [N]
@@ -81,7 +99,7 @@ __global__ void __launch_bounds__(256) k_bow_frame(const int* __restrict__ offse
     __shared__ int s_total;
     __shared__ double s_norm;
     const int f = blockIdx.x, tid = threadIdx.x;
-    const int base = offsets[f], n = offsets[f + 1] - base;
+    const int base = rows.base(f), n = rows.count(f);
     int N = 1;
     while (N < n) N <<= 1;
     // ---- BowVector: sort by (word, feature); stopped features go to the end ----
@@ -163,6 +181,7 @@ struct hvo_bow {
     int device = 0;
     cudaStream_t stream = nullptr;
     int n_nodes = 0, levels = 0;
+    int tile = 32;   // lanes per descriptor in k_bow_descend: 8, 16 or 32 (the largest branching factor, capped at 32)
     int *d_child_start = nullptr, *d_child_ids = nullptr, *d_node_word = nullptr;
     uint8_t* d_node_desc = nullptr;
     double* d_node_weight = nullptr;
@@ -219,9 +238,11 @@ int hvo_bow_set_vocabulary(hvo_bow* h, int n_nodes, const int32_t* child_start, 
     HVO_CHECK_ARG(n_nodes >= 1 && depth_levels >= 1, "empty vocabulary");
     HVO_CHECK_ARG(child_start[0] == 0, "child_start[0] must be 0");
     const int nchild = child_start[n_nodes];
+    int max_children = 0;
     for (int i = 0; i < n_nodes; ++i) {
         HVO_CHECK_ARG(child_start[i + 1] >= child_start[i], "child_start must be non-decreasing");
         HVO_CHECK_ARG(child_start[i + 1] - child_start[i] < 65536, "too many children in one node");
+        max_children = std::max(max_children, child_start[i + 1] - child_start[i]);
     }
     for (int i = 0; i < nchild; ++i) HVO_CHECK_ARG(child_ids[i] > 0 && child_ids[i] < n_nodes, "child id out of range");
     HVO_CUDA(cudaSetDevice(h->device));
@@ -237,6 +258,7 @@ int hvo_bow_set_vocabulary(hvo_bow* h, int n_nodes, const int32_t* child_start, 
     HVO_CUDA(cudaMemcpyAsync(h->d_node_weight, node_weight, (size_t)n_nodes * 8, cudaMemcpyHostToDevice, s));
     HVO_CUDA(cudaStreamSynchronize(s));
     h->n_nodes = n_nodes; h->levels = depth_levels;
+    h->tile = max_children <= 8 ? 8 : max_children <= 16 ? 16 : 32;
     return HVO_OK;
 }
 
@@ -257,22 +279,36 @@ static int bow_reserve(hvo_bow* h, int total, int nframes) {
     return HVO_OK;
 }
 
+// The two kernels on `nframes` frames laid out as `rows` (`total` rows, at most `max_rows` per frame), asynchronous on `s`.
+static int bow_launch(const hvo_bow* h, cudaStream_t s, const uint8_t* d_desc, BowRows rows, int total, int nframes, int max_rows, int levelsup,
+                      int* word_of, int* node_of, double* weight_of, int* bow_counts, int* bow_words, double* bow_values, int* fv_order, int* fv_counts) {
+    const uint4* q = reinterpret_cast<const uint4*>(d_desc);
+    const uint4* nd = reinterpret_cast<const uint4*>(h->d_node_desc);
+    const int nid_level = h->levels - levelsup;
+    const unsigned blocks = (unsigned)(((long long)total * h->tile + 127) / 128);
+#define HVO_BOW_DESCEND(T) k_bow_descend<T><<<blocks, 128, 0, s>>>(q, rows, total, h->d_child_start, h->d_child_ids, nd, h->d_node_weight, \
+                                                                   h->d_node_word, nid_level, word_of, node_of, weight_of)
+    if (h->tile == 8) HVO_BOW_DESCEND(8);
+    else if (h->tile == 16) HVO_BOW_DESCEND(16);
+    else HVO_BOW_DESCEND(32);
+#undef HVO_BOW_DESCEND
+    int N = 1;
+    while (N < max_rows) N <<= 1;
+    k_bow_frame<<<nframes, 256, (size_t)N * 8, s>>>(rows, word_of, node_of, weight_of, bow_counts, bow_words, bow_values, fv_order, fv_counts);
+    HVO_CUDA(cudaGetLastError());
+    return HVO_OK;
+}
+
 static int bow_run(hvo_bow* h, const uint8_t* d_desc, int total, int nframes, const int32_t* offsets, int levelsup) {
     cudaStream_t s = h->stream;
     int maxn = 0;
     for (int f = 0; f < nframes; ++f) maxn = std::max(maxn, offsets[f + 1] - offsets[f]);
     HVO_CHECK_ARG(maxn <= kBowMaxFeatures, "more than 4096 features in one frame");
     HVO_CUDA(cudaMemcpyAsync(h->d_offsets, offsets, ((size_t)nframes + 1) * 4, cudaMemcpyHostToDevice, s));
-    k_bow_descend<<<div_up(total * 32, 128), 128, 0, s>>>(reinterpret_cast<const uint4*>(d_desc), total, h->d_child_start, h->d_child_ids,
-                                                          reinterpret_cast<const uint4*>(h->d_node_desc), h->d_node_weight, h->d_node_word,
-                                                          h->levels - levelsup, h->d_word, h->d_node, h->d_weight);
-    int N = 1;
-    while (N < maxn) N <<= 1;
-    k_bow_frame<<<nframes, 256, (size_t)N * 8, s>>>(h->d_offsets, h->d_word, h->d_node, h->d_weight, h->d_bow_counts, h->d_bow_words, h->d_bow_values,
-                                                     h->d_fv, h->d_fv_counts);
-    HVO_CUDA(cudaGetLastError());
+    const int st = bow_launch(h, s, d_desc, BowRows{h->d_offsets, nullptr, 0}, total, nframes, maxn, levelsup, h->d_word, h->d_node, h->d_weight,
+                              h->d_bow_counts, h->d_bow_words, h->d_bow_values, h->d_fv, h->d_fv_counts);
     h->last_launches = 2;
-    return HVO_OK;
+    return st;
 }
 
 int hvo_bow_transform(hvo_bow* h, const uint8_t* desc, const int32_t* offsets, int nframes, int levelsup, int32_t* word_of, int32_t* node_of,
@@ -307,3 +343,16 @@ int hvo_bow_transform(hvo_bow* h, const uint8_t* desc, const int32_t* offsets, i
 int hvo_bow_last_launches(const hvo_bow* h) { return h ? h->last_launches : 0; }
 
 }  // extern "C"
+
+namespace hvo {
+
+// The frame handle's layout: frame f = rows f * stride .., d_counts[f] of them (device), every output [nframes][stride] or [nframes].
+int bow_frame_launch(hvo_bow* h, cudaStream_t s, const uint8_t* d_desc, const int32_t* d_counts, int nframes, int stride, int levelsup,
+                     double* d_weight, const hvo_frame_bow_outputs* o) {
+    HVO_CHECK_ARG(stride <= kBowMaxFeatures, "more than 4096 features in one frame");
+    return bow_launch(h, s, d_desc, BowRows{nullptr, d_counts, stride}, nframes * stride, nframes, stride, levelsup, o->word_of, o->node_of, d_weight,
+                      o->bow_counts, o->bow_words, o->bow_values, o->fv_order, o->fv_counts);
+}
+int bow_max_features() { return kBowMaxFeatures; }
+
+}  // namespace hvo

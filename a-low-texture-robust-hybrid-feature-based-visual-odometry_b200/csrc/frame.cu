@@ -22,6 +22,9 @@ int* orb_error_flag(hvo_orb* h);
 const int* line_segment_counts(hvo_line* h);
 int line_segment_cap(hvo_line* h);
 const int32_t* plane_status(hvo_plane* h);
+int bow_frame_launch(hvo_bow* h, cudaStream_t s, const uint8_t* d_desc, const int32_t* d_counts, int nframes, int stride, int levelsup,
+                     double* d_weight, const hvo_frame_bow_outputs* o);
+int bow_max_features();
 }  // namespace hvo
 using namespace hvo;
 
@@ -85,6 +88,7 @@ struct FrameLane {
     uint8_t* d_gray = nullptr;
     uint16_t* d_depth = nullptr;
     hvo_frame_outputs d_out;  // device staging of every output (host API)
+    hvo_frame_bow_outputs d_bow{};  // device staging of the BoW outputs (host API; allocated while a vocabulary is attached)
 };
 
 struct hvo_frame {
@@ -100,6 +104,9 @@ struct hvo_frame {
     int* h_fault = nullptr;   // pinned copy
     bool undistort = false;   // distorted camera with coefficients: mvKeysUn / mvuRight are formed on the device
     hvo_camera cam{};
+    hvo_bow* bow = nullptr;   // attached vocabulary (hvo_frame_set_vocabulary)
+    int levelsup = 4;
+    double* d_bow_weight = nullptr;   // per-row leaf weights of one chunk: shared by the lanes, whose ORB kernels run in order on one stream
 };
 
 static const int kNoFault = 0x7fffffff;
@@ -127,6 +134,18 @@ static hvo_frame_outputs outputs_at(const hvo_frame* h, const hvo_frame_outputs&
     if (o.kps_un) r.kps_un = o.kps_un + off * c;
     return r;
 }
+static hvo_frame_bow_outputs outputs_at(const hvo_frame* h, const hvo_frame_bow_outputs& o, size_t off) {
+    const size_t c = (size_t)h->orb_cap;
+    hvo_frame_bow_outputs r = o;
+    if (o.bow_counts) r.bow_counts = o.bow_counts + off;
+    if (o.bow_words) r.bow_words = o.bow_words + off * c;
+    if (o.bow_values) r.bow_values = o.bow_values + off * c;
+    if (o.fv_order) r.fv_order = o.fv_order + off * c;
+    if (o.fv_counts) r.fv_counts = o.fv_counts + off;
+    if (o.node_of) r.node_of = o.node_of + off * c;
+    if (o.word_of) r.word_of = o.word_of + off * c;
+    return r;
+}
 
 // The pipelines of one lane on n frames: wait for `start`, run, optionally copy each stage's results back on its own
 // stream, record the lane's join events.  Launch order = placement order: the ordered (latency-bound) pipelines first.
@@ -139,11 +158,14 @@ static hvo_frame_outputs outputs_at(const hvo_frame* h, const hvo_frame_outputs&
 // them slower (4736 frames: 16.2 K frames/s side by side, 18.2 K one after the other; ORB / normals beside the ordered kernels:
 // 16.5-17.3 K).  So a chunk of >= kSerialFrames frames runs its pipelines ONE AFTER THE OTHER (planes, lines, ORB, normals), each at
 // its saturating batch, and the download of a pipeline's results runs beside the kernels of the next one.
+// bo (device, NULL = no BoW) / host_bo (host, NULL = nothing to download): the BoW kernels follow the ORB kernels on the ORB stream; their
+// downloads are the first of phase 2.
 // HVO_FRAME_SERIAL=0 / 1 forces one schedule (tuning aid).  Also measured for 1024-frame chunks and rejected: planes || lines first and
 // ORB || normals afterwards (87 instead of 65-79 ms), a third priority level that puts planes above lines (no change).
 static const int kSerialFrames = 2048;
 static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_t start_depth, const uint8_t* d_gray, const uint16_t* d_depth, int n,
-                       int base, const hvo_frame_outputs& o, const hvo_frame_outputs* host, int* launches, FrameLane* after = nullptr) {
+                       int base, const hvo_frame_outputs& o, const hvo_frame_outputs* host, const hvo_frame_bow_outputs* bo,
+                       const hvo_frame_bow_outputs* host_bo, int* launches, FrameLane* after = nullptr) {
     const size_t N = (size_t)n, px = (size_t)h->width * h->height;
     static const int serial_env = [] { const char* e = getenv("HVO_FRAME_SERIAL"); return e ? atoi(e) : -1; }();
     const bool serial = serial_env >= 0 ? serial_env == 1 : n >= kSerialFrames;
@@ -201,6 +223,11 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
             if (st != HVO_OK) return st;
             ++*launches;
         }
+        if (bo) {
+            st = bow_frame_launch(h->bow, s, o.desc, o.kp_counts, n, h->orb_cap, h->levelsup, h->d_bow_weight, bo);
+            if (st != HVO_OK) return st;
+            *launches += 2;
+        }
         k_frame_fold_status<<<1, 32, 0, s>>>(orb_error_flag(L.orb), 1, 1, 0, base, FAULT_ORB, h->d_fault);   // one flag per chunk
         HVO_CUDA(cudaMemsetAsync(orb_error_flag(L.orb), 0, sizeof(int), s));
         HVO_CUDA(cudaEventRecord(L.cdone[0], s));
@@ -227,6 +254,20 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
         if (host) { HVO_CUDA(cudaStreamWaitEvent(L.down[i], L.cdone[i], 0)); *out = L.down[i]; }
         return HVO_OK;
     };
+    // the BoW rows first, on the ORB download stream: side by side they are ready long before the planes, so a download into pageable
+    // memory (which holds the calling thread until it is done) runs while the ordered pipelines still compute instead of after them
+    if (host && host_bo) {
+        cudaStream_t s;
+        if (int ds = down_stream(0, orb_stream(L.orb), &s)) return ds;
+        const size_t c = (size_t)h->orb_cap;
+        HVO_CUDA(cudaMemcpyAsync(host_bo->bow_counts, bo->bow_counts, N * 4, cudaMemcpyDeviceToHost, s));
+        HVO_CUDA(cudaMemcpyAsync(host_bo->bow_words, bo->bow_words, N * c * 4, cudaMemcpyDeviceToHost, s));
+        HVO_CUDA(cudaMemcpyAsync(host_bo->bow_values, bo->bow_values, N * c * 8, cudaMemcpyDeviceToHost, s));
+        if (host_bo->fv_order) HVO_CUDA(cudaMemcpyAsync(host_bo->fv_order, bo->fv_order, N * c * 4, cudaMemcpyDeviceToHost, s));
+        if (host_bo->fv_counts) HVO_CUDA(cudaMemcpyAsync(host_bo->fv_counts, bo->fv_counts, N * 4, cudaMemcpyDeviceToHost, s));
+        if (host_bo->node_of) HVO_CUDA(cudaMemcpyAsync(host_bo->node_of, bo->node_of, N * c * 4, cudaMemcpyDeviceToHost, s));
+        if (host_bo->word_of) HVO_CUDA(cudaMemcpyAsync(host_bo->word_of, bo->word_of, N * c * 4, cudaMemcpyDeviceToHost, s));
+    }
     if (h->p.stages & ST_PLANE) {
         cudaStream_t s;
         if (int ds = down_stream(2, plane_stream(L.plane), &s)) return ds;
@@ -451,10 +492,24 @@ int hvo_frame_create(const hvo_frame_params* p, int width, int height, int max_b
     return HVO_OK;
 }
 
+static void frame_detach_vocabulary(hvo_frame* h) {
+    for (FrameLane& L : h->lane) {
+        hvo_frame_bow_outputs& o = L.d_bow;
+        void* bufs[] = {o.bow_counts, o.bow_words, o.bow_values, o.fv_order, o.fv_counts, o.node_of, o.word_of};
+        for (void* b : bufs) if (b) cudaFree(b);
+        o = hvo_frame_bow_outputs{};
+    }
+    if (h->d_bow_weight) cudaFree(h->d_bow_weight);
+    h->d_bow_weight = nullptr;
+    hvo_bow_destroy(h->bow);
+    h->bow = nullptr;
+}
+
 void hvo_frame_destroy(hvo_frame* h) {
     if (!h) return;
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
+    frame_detach_vocabulary(h);
     for (int li = 0; li < kMaxLanes; ++li) {
         FrameLane& L = h->lane[li];
         if (L.owns) {
@@ -512,10 +567,56 @@ static int frame_check_outputs(const hvo_frame* h, const hvo_frame_outputs* o, b
     return HVO_OK;
 }
 
-int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out) {
+static int frame_check_bow_outputs(const hvo_frame* h, const hvo_frame_bow_outputs* b, bool device) {
+    if (!b) return HVO_OK;
+    HVO_CHECK_ARG(h->bow, "BoW outputs need a vocabulary (hvo_frame_set_vocabulary)");
+    HVO_CHECK_ARG(b->bow_counts && b->bow_words && b->bow_values, "bow_counts / bow_words / bow_values missing");
+    HVO_CHECK_ARG(!b->fv_order || b->node_of, "fv_order needs node_of");
+    if (device) HVO_CHECK_ARG(b->fv_order && b->fv_counts && b->node_of && b->word_of, "device BoW outputs: every array is required");
+    return HVO_OK;
+}
+
+int hvo_frame_set_vocabulary(hvo_frame* h, int n_nodes, const int32_t* child_start, const int32_t* child_ids, const uint8_t* node_desc,
+                             const double* node_weight, const int32_t* node_word, int depth_levels, int levelsup) {
+    HVO_CHECK_ARG(h, "null handle");
+    HVO_CHECK_ARG(n_nodes >= 0, "n_nodes < 0");
+    HVO_CUDA(cudaSetDevice(h->device));
+    HVO_CUDA(cudaStreamSynchronize(h->stream));   // queued calls may still use the BoW buffers
+    frame_detach_vocabulary(h);
+    if (n_nodes == 0) return HVO_OK;
+    HVO_CHECK_ARG(h->p.stages & ST_ORB, "a vocabulary needs the ORB stage");
+    HVO_CHECK_ARG(h->orb_cap <= bow_max_features(), "orb_capacity > 4096: too many features per frame for the BoW sort");
+    int st = hvo_bow_create(h->device, &h->bow);   // (also makes h->device current)
+    if (st == HVO_OK) st = hvo_bow_set_vocabulary(h->bow, n_nodes, child_start, child_ids, node_desc, node_weight, node_word, depth_levels);
+    const size_t c = (size_t)h->orb_cap;
+    do {
+#define HVO_TRY(call) if ((call) != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(cudaGetLastError())); st = HVO_ERR_CUDA; break; }
+        if (st != HVO_OK) break;
+        HVO_TRY(cudaMalloc(&h->d_bow_weight, (size_t)h->lane[0].cap * c * 8));
+        for (int li = 0; li < h->nlanes && st == HVO_OK; ++li) {
+            const size_t B = (size_t)h->lane[li].cap;
+            hvo_frame_bow_outputs& o = h->lane[li].d_bow;
+            HVO_TRY(cudaMalloc(&o.bow_counts, B * 4));
+            HVO_TRY(cudaMalloc(&o.bow_words, B * c * 4));
+            HVO_TRY(cudaMalloc(&o.bow_values, B * c * 8));
+            HVO_TRY(cudaMalloc(&o.fv_order, B * c * 4));
+            HVO_TRY(cudaMalloc(&o.fv_counts, B * 4));
+            HVO_TRY(cudaMalloc(&o.node_of, B * c * 4));
+            HVO_TRY(cudaMalloc(&o.word_of, B * c * 4));
+        }
+#undef HVO_TRY
+    } while (0);
+    if (st != HVO_OK) { frame_detach_vocabulary(h); return st; }
+    h->levelsup = levelsup;
+    return HVO_OK;
+}
+
+int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                       const hvo_frame_bow_outputs* d_bow) {
     HVO_CHECK_ARG(h && d_gray && d_depth16, "null argument");
     HVO_CHECK_ARG(nframes >= 1 && nframes <= h->max_batch, "nframes out of range for this handle");
     int st = frame_check_outputs(h, d_out, true);
+    if (st == HVO_OK) st = frame_check_bow_outputs(h, d_bow, true);
     if (st != HVO_OK) return st;
     if (h->p.stages & ST_ORB) HVO_CHECK_ARG(d_out->kp_depth && d_out->kp_uright, "kp_depth / kp_uright missing");
     if (h->p.stages & ST_LINE) HVO_CHECK_ARG(d_out->linevec3, "linevec3 missing");
@@ -532,8 +633,9 @@ int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const ui
     for (int off = 0; off < nframes; off += per, ++used) {
         FrameLane& L = h->lane[used];
         const int n = std::min(per, nframes - off);
-        st = lane_launch(h, L, h->fork, nullptr, d_gray + (size_t)off * px, d_depth16 + (size_t)off * px, n, off, outputs_at(h, *d_out, (size_t)off), nullptr, &launches,
-                         h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
+        const hvo_frame_bow_outputs bo = d_bow ? outputs_at(h, *d_bow, (size_t)off) : hvo_frame_bow_outputs{};
+        st = lane_launch(h, L, h->fork, nullptr, d_gray + (size_t)off * px, d_depth16 + (size_t)off * px, n, off, outputs_at(h, *d_out, (size_t)off), nullptr,
+                         d_bow ? &bo : nullptr, nullptr, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
         if (st != HVO_OK) return st;
         h->last_lane = used;
     }
@@ -545,10 +647,16 @@ int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const ui
     return HVO_OK;
 }
 
-int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out) {
+    return hvo_frame_extract_batch_device_bow(h, d_gray, d_depth16, nframes, d_out, nullptr);
+}
+
+int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                      const hvo_frame_bow_outputs* bow) {
     HVO_CHECK_ARG(h && gray && depth16, "null argument");
     HVO_CHECK_ARG(nframes >= 1, "nframes < 1");
     int st = frame_check_outputs(h, out, false);
+    if (st == HVO_OK) st = frame_check_bow_outputs(h, bow, false);
     if (st != HVO_OK) return st;
     HVO_CUDA(cudaSetDevice(h->device));
     const size_t px = (size_t)h->width * h->height;
@@ -578,7 +686,9 @@ int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint1
         if (!out->normals3) d.normals3 = nullptr;
         if (!out->kps_un) d.kps_un = nullptr;
         const hvo_frame_outputs hostk = outputs_at(h, *out, (size_t)off);
-        st = lane_launch(h, L, L.fork, L.fork_depth, L.d_gray, L.d_depth, n, off, d, &hostk, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
+        const hvo_frame_bow_outputs hostb = bow ? outputs_at(h, *bow, (size_t)off) : hvo_frame_bow_outputs{};
+        st = lane_launch(h, L, L.fork, L.fork_depth, L.d_gray, L.d_depth, n, off, d, &hostk, bow ? &L.d_bow : nullptr, bow ? &hostb : nullptr, &launches,
+                         h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
         if (st != HVO_OK) return st;
         h->last_lane = li;
     }
@@ -591,11 +701,20 @@ int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint1
     return HVO_OK;
 }
 
-int hvo_frame_extract_batch(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
-    const int st = hvo_frame_extract_batch_async(h, gray, depth16, nframes, out);
+int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+    return hvo_frame_extract_batch_async_bow(h, gray, depth16, nframes, out, nullptr);
+}
+
+int hvo_frame_extract_batch_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                const hvo_frame_bow_outputs* bow) {
+    const int st = hvo_frame_extract_batch_async_bow(h, gray, depth16, nframes, out, bow);
     if (st != HVO_OK) return st;
     HVO_CUDA(cudaStreamSynchronize(h->stream));
     return frame_check_fault(h);
+}
+
+int hvo_frame_extract_batch(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+    return hvo_frame_extract_batch_bow(h, gray, depth16, nframes, out, nullptr);
 }
 
 int hvo_frame_last_launches(const hvo_frame* h) { return h ? h->last_launches : 0; }

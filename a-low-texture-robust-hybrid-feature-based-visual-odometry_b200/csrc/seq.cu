@@ -44,6 +44,18 @@ static hvo_frame_outputs seq_outputs_at(const hvo_seq* s, const hvo_frame_output
     if (o.kps_un) r.kps_un = o.kps_un + off * c;
     return r;
 }
+static hvo_frame_bow_outputs seq_outputs_at(const hvo_seq* s, const hvo_frame_bow_outputs& o, size_t off) {
+    const size_t c = (size_t)s->orb_cap;
+    hvo_frame_bow_outputs r = o;
+    if (o.bow_counts) r.bow_counts = o.bow_counts + off;
+    if (o.bow_words) r.bow_words = o.bow_words + off * c;
+    if (o.bow_values) r.bow_values = o.bow_values + off * c;
+    if (o.fv_order) r.fv_order = o.fv_order + off * c;
+    if (o.fv_counts) r.fv_counts = o.fv_counts + off;
+    if (o.node_of) r.node_of = o.node_of + off * c;
+    if (o.word_of) r.word_of = o.word_of + off * c;
+    return r;
+}
 
 extern "C" {
 
@@ -89,7 +101,18 @@ void hvo_seq_shard(int nframes, int ndevices, int d, int* first, int* count) {
     *count = base + (d < rem ? 1 : 0);
 }
 
-int hvo_seq_extract(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+int hvo_seq_set_vocabulary(hvo_seq* s, int n_nodes, const int32_t* child_start, const int32_t* child_ids, const uint8_t* node_desc,
+                           const double* node_weight, const int32_t* node_word, int depth_levels, int levelsup) {
+    HVO_CHECK_ARG(s, "null handle");
+    for (size_t d = 0; d < s->handles.size(); ++d) {
+        const int st = hvo_frame_set_vocabulary(s->handles[d], n_nodes, child_start, child_ids, node_desc, node_weight, node_word, depth_levels, levelsup);
+        if (st != HVO_OK) return st;
+    }
+    return HVO_OK;
+}
+
+int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                        const hvo_frame_bow_outputs* bow) {
     HVO_CHECK_ARG(s && gray && depth16 && out && nframes >= 1, "bad argument");
     const int nd = (int)s->devices.size();
     const size_t px = (size_t)s->width * s->height;
@@ -107,7 +130,8 @@ int hvo_seq_extract(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, in
             for (int off = 0; st == HVO_OK && off < count; off += s->call_frames) {
                 const int n = std::min(s->call_frames, count - off);
                 const hvo_frame_outputs o = seq_outputs_at(s, *out, (size_t)(first + off));
-                st = hvo_frame_extract_batch_async(h, gray + (size_t)(first + off) * px, depth16 + (size_t)(first + off) * px, n, &o);
+                const hvo_frame_bow_outputs b = bow ? seq_outputs_at(s, *bow, (size_t)(first + off)) : hvo_frame_bow_outputs{};
+                st = hvo_frame_extract_batch_async_bow(h, gray + (size_t)(first + off) * px, depth16 + (size_t)(first + off) * px, n, &o, bow ? &b : nullptr);
             }
             float ms = 0.f;
             const int st2 = hvo_frame_timer_stop(h, &ms);   // waits for every download of this device; reports device-side faults
@@ -121,6 +145,10 @@ int hvo_seq_extract(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, in
     for (int d = 0; d < nd; ++d)
         if (status[d] != HVO_OK) { set_error("device %d: %s", s->devices[d], errors[d].c_str()); return status[d]; }
     return HVO_OK;
+}
+
+int hvo_seq_extract(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+    return hvo_seq_extract_bow(s, gray, depth16, nframes, out, nullptr);
 }
 
 float hvo_seq_last_ms(const hvo_seq* s) { return s ? s->last_ms : 0.f; }

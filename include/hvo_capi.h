@@ -623,6 +623,21 @@ typedef struct hvo_frame_outputs {
                                                      with distorted != 0 and a non-zero coefficient                  */
 } hvo_frame_outputs;
 
+/* Bag-of-words vectors of a batch of n frames (Frame::ComputeBoW, src/Frame.cc:1692-1699: transform(mDescriptors rows, mBowVec, mFeatVec,
+ * levelsup)), for a handle with a vocabulary (hvo_frame_set_vocabulary).  Frame f's rows are those of hvo_bow_transform on the frame's
+ * descriptor rows [0, kp_counts[f]), bit for bit; rows at or past a frame's count are not written.  Host pointers for the host calls,
+ * device pointers for hvo_frame_extract_batch_device_bow.                                                                          */
+typedef struct hvo_frame_bow_outputs {
+    int32_t* bow_counts;  /* [n]                    words in mBowVec                                                               */
+    int32_t* bow_words;   /* [n][orb_capacity]      ascending word ids (first bow_counts[f] rows)                                  */
+    double* bow_values;   /* [n][orb_capacity]      their L1-normalised values, bit-identical to DBoW2                              */
+    int32_t* fv_order;    /* [n][orb_capacity]      feature indices sorted by (node_of, feature), first fv_counts[f] rows; runs of
+                                                    equal node_of are mFeatVec's vectors             optional on the host (needs node_of) */
+    int32_t* fv_counts;   /* [n]                    features not stopped                             optional on the host            */
+    int32_t* node_of;     /* [n][orb_capacity]      node at level m_L - levelsup (mFeatVec keys; 0 = root)  optional on the host         */
+    int32_t* word_of;     /* [n][orb_capacity]      word id, or -1 where the word is stopped          optional on the host            */
+} hvo_frame_bow_outputs;
+
 /* Host-side expanders of the compact outputs (plain C loops, no CUDA). */
 /* labels4 [H*W/2] -> labels [H*W] int32 (-1 = none) */
 int hvo_membership4_expand(const uint8_t* labels4, int npixels, int32_t* labels);
@@ -646,6 +661,23 @@ int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint1
 /* Everything device-resident (n <= max_batch); asynchronous.  hvo_frame_sync / hvo_frame_timer_stop wait for all pipelines. */
 int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes,
                                    const hvo_frame_outputs* d_out);
+/* Attach a vocabulary: the arrays of hvo_bow_set_vocabulary (validated and uploaded by it, to a vocabulary object the handle owns on its
+ * device), plus levelsup (Frame::ComputeBoW passes 4).  Waits for the handle's queued work first.  Every later *_bow call given BoW
+ * outputs then computes the frames' BowVector / FeatureVector on the device right after the ORB descriptors, on the ORB stream, and
+ * returns them with the frame's other outputs; calls without BoW outputs compute none.  Refused (HVO_ERR_ARG) for a handle without
+ * the ORB stage or with hvo_frame_capacities' orb_capacity > 4096.  n_nodes == 0 detaches the vocabulary (the other arrays may be NULL).
+ * Attaching replaces the previous vocabulary; a refused or failed attach leaves the handle without one. */
+int hvo_frame_set_vocabulary(hvo_frame* h, int n_nodes, const int32_t* child_start, const int32_t* child_ids, const uint8_t* node_desc,
+                             const double* node_weight, const int32_t* node_word, int depth_levels, int levelsup);
+/* hvo_frame_extract_batch / _async / _device with BoW outputs as well.  bow == NULL: exactly the call without _bow.  With bow != NULL
+ * the handle needs a vocabulary; on the host bow_counts, bow_words and bow_values are required and fv_order needs node_of; on the
+ * device every array of hvo_frame_bow_outputs is required.  Otherwise HVO_ERR_ARG. */
+int hvo_frame_extract_batch_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                const hvo_frame_bow_outputs* bow);
+int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                      const hvo_frame_bow_outputs* bow);
+int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                       const hvo_frame_bow_outputs* d_bow);
 int hvo_frame_last_launches(const hvo_frame* h);
 int hvo_frame_sync(hvo_frame* h);
 int hvo_frame_timer_start(hvo_frame* h);
@@ -668,6 +700,12 @@ int hvo_seq_capacities(const hvo_seq* s, int* orb_capacity, int* max_lines, int*
 void hvo_seq_shard(int nframes, int ndevices, int d, int* first, int* count);
 /* blocks until every output row has been written; a device-side fault or CUDA error of any device is returned with its device id */
 int hvo_seq_extract(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out);
+/* hvo_frame_set_vocabulary on every device's handle (same arguments and rules). */
+int hvo_seq_set_vocabulary(hvo_seq* s, int n_nodes, const int32_t* child_start, const int32_t* child_ids, const uint8_t* node_desc,
+                           const double* node_weight, const int32_t* node_word, int depth_levels, int levelsup);
+/* hvo_seq_extract with the BoW outputs of hvo_frame_extract_batch_bow (host arrays of n frames); bow == NULL: hvo_seq_extract. */
+int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                        const hvo_frame_bow_outputs* bow);
 /* device time of the last hvo_seq_extract: CUDA events around each device's share (uploads, kernels, downloads), max over devices */
 float hvo_seq_last_ms(const hvo_seq* s);
 
