@@ -91,6 +91,9 @@ ABI = {
     'hvo_seq_extract': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp]),
     'hvo_seq_set_vocabulary': (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int]),
     'hvo_seq_extract_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
+    'hvo_seq_extract_grid': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp]),
+    'hvo_seq_image_bounds': (C.c_int, [_vp] + [C.POINTER(C.c_float)] * 4),
+    'hvo_seq_line_grid_capacity': (C.c_int, [_vp]),
     'hvo_seq_last_ms': (C.c_float, [_vp]),
     'hvo_normals3_expand': (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp]),
     'hvo_orb_level_size': (C.c_int, [_vp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
@@ -215,6 +218,11 @@ ABI = {
     'hvo_frame_extract_batch_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
     'hvo_frame_extract_batch_async_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
     'hvo_frame_extract_batch_device_bow': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp]),
+    'hvo_frame_extract_batch_grid': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp]),
+    'hvo_frame_extract_batch_async_grid': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp]),
+    'hvo_frame_extract_batch_device_grid': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp]),
+    'hvo_frame_image_bounds': (C.c_int, [_vp] + [C.POINTER(C.c_float)] * 4),
+    'hvo_frame_line_grid_capacity': (C.c_int, [_vp]),
     'hvo_frame_last_launches': (C.c_int, [_vp]),
     'hvo_frame_sync': (C.c_int, [_vp]),
     'hvo_frame_timer_start': (C.c_int, [_vp]),
@@ -1938,16 +1946,22 @@ class _FrameBowOutputs(C.Structure):
     _fields_ = [(n, _vp) for n in ('bow_counts', 'bow_words', 'bow_values', 'fv_order', 'fv_counts', 'node_of', 'word_of')]
 
 
+class _FrameGridOutputs(C.Structure):
+    _fields_ = [(n, _vp) for n in ('grid_counts', 'grid_items', 'lgrid_counts', 'lgrid_items')]
+
+
 class FrameFrontEnd:
     """The extraction part of ORB_SLAM2::Frame::Frame(imGray, imDepth, ...) (reference src/Frame.cc:188-233): ORB + RGB-D
     depth lookup, LSD/LBD lines, PEAC planes and surface normals of a batch of frames, three concurrent CUDA streams."""
     FIELDS = [f[0] for f in _FrameOutputs._fields_]
     BOW_FIELDS = [f[0] for f in _FrameBowOutputs._fields_]
+    GRID_FIELDS = [f[0] for f in _FrameGridOutputs._fields_]
     vocabulary = None
+    grids = False
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, bf=40.0, nfeatures=1000, scale_factor=1.2, nlevels=8, ini_th=20,
                  min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=16, max_batch=1, device=0, line_cull=False, lanes=0, membership='i32',
-                 distorted=False, normals='n8', dist=None, vocabulary=None, levelsup=4):
+                 distorted=False, normals='n8', dist=None, vocabulary=None, levelsup=4, grids=False):
         """membership: 'i32' (int32 labels, -1 = none), 'u8' (one byte per pixel, 255 = none: what a host caller needs to
         rebuild plane_vertices_), 'both', or 'u4' (host calls only: two pixels per byte, 15 = none, max_planes <= 15; expand with
         membership4_expand).  The int32 image is always the device-side working image.
@@ -1956,7 +1970,9 @@ class FrameFrontEnd:
         dist: mDistCoef (k1, k2, p1, p2 [, k3]).  With a non-zero coefficient the handle runs Frame::UndistortKeyPoints on the device:
         kp_uright is formed from the undistorted keypoints and the outputs gain kps_un (mvKeysUn).
         vocabulary: the dict ORBVocabulary takes.  Every frame then also gets what Frame::ComputeBoW computes, transform(mDescriptors,
-        mBowVec, mFeatVec, levelsup), on the device right after its descriptors: the outputs gain the BoW arrays (see bow())."""
+        mBowVec, mFeatVec, levelsup), on the device right after its descriptors: the outputs gain the BoW arrays (see bow()).
+        grids: every frame also gets Frame::AssignFeaturesToGrid / AssignFeaturesToGridForLine (mGrid, mGridForLine) with the handle's
+        image_bounds(): the outputs gain grid_counts / grid_items (ORB stage) and lgrid_counts / lgrid_items (line stage), see grid()."""
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
@@ -1971,6 +1987,7 @@ class FrameFrontEnd:
         self.orb_capacity, self.max_lines, self.normals_count = a.value, b.value, c.value
         _check(lib().hvo_frame_lanes(out, C.byref(a), C.byref(b)))
         self.lanes, self.chunk = a.value, b.value
+        self.grids, self.line_grid_capacity = bool(grids), lib().hvo_frame_line_grid_capacity(out)
         if vocabulary is not None:
             self.set_vocabulary(vocabulary, levelsup)
 
@@ -1984,6 +2001,13 @@ class FrameFrontEnd:
         args, _keep = _vocabulary_args(vocabulary)
         _check(f(h, *args, int(levelsup)))
         self.vocabulary, self.levelsup = vocabulary, int(levelsup)
+
+    def image_bounds(self):
+        """(mnMinX, mnMaxX, mnMinY, mnMaxY) the grids are built with (hvo_frame_image_bounds), float32 as module-level image_bounds()."""
+        f, h = (lib().hvo_seq_image_bounds, self._seq) if getattr(self, '_seq', None) else (lib().hvo_frame_image_bounds, self._h)
+        v = [C.c_float(0) for _ in range(4)]
+        _check(f(h, *[C.byref(a) for a in v]))
+        return tuple(np.float32(a.value) for a in v)
 
     def _params(self, fx, fy, cx, cy, depth_factor, bf, nfeatures, scale_factor, nlevels, ini_th, min_th, n_lines, stages, max_planes,
                 line_cull, lanes, distorted, dist):
@@ -2017,10 +2041,14 @@ class FrameFrontEnd:
             if self.vocabulary is not None:
                 sh.update(bow_counts=((n,), np.int32), bow_words=((n, c), np.int32), bow_values=((n, c), np.float64), fv_order=((n, c), np.int32),
                           fv_counts=((n,), np.int32), node_of=((n, c), np.int32), word_of=((n, c), np.int32))
+            if self.grids:
+                sh.update(grid_counts=((n, 64 * 48), np.uint16), grid_items=((n, c), np.uint16))
         if self.stages & STAGE_LINES:
             c = self.max_lines
             sh.update(keylines=((n, c), KL_DTYPE), line_desc=((n, c, 32), np.uint8), linevec3=((n, c, 3), np.float64),
                       line_counts=((n,), np.int32))
+            if self.grids:
+                sh.update(lgrid_counts=((n, 64 * 48), np.uint16), lgrid_items=((n, self.line_grid_capacity), np.uint16))
         if self.stages & STAGE_PLANES:
             sh.update(n_planes=((n,), np.int32), planes7=((n, self.max_planes, 7), np.float64))
             if device or self.membership_mode in ('i32', 'both'):
@@ -2073,6 +2101,30 @@ class FrameFrontEnd:
             setattr(o, k, ptrs.get(k))
         return C.byref(o)
 
+    def _grid_outputs(self, ptrs):
+        """hvo_frame_grid_outputs by reference, or None for a handle created without grids."""
+        if not self.grids:
+            return None
+        o = _FrameGridOutputs()
+        for k in self.GRID_FIELDS:
+            setattr(o, k, ptrs.get(k))
+        return C.byref(o)
+
+    @staticmethod
+    def _cells(counts, items, f):
+        c = np.asarray(counts[f], np.int32)
+        return c, np.asarray(items[f, :int(c.sum())], np.int32)
+
+    @staticmethod
+    def grid(out, f):
+        """Frame f's mGrid: (counts int32 [3072], items int32), cell = ix * 48 + iy, the form of oracle.grid_build."""
+        return FrameFrontEnd._cells(out['grid_counts'], out['grid_items'], f)
+
+    @staticmethod
+    def line_grid(out, f):
+        """Frame f's mGridForLine: (counts int32 [3072], items int32), the form of oracle.line_grid_build."""
+        return FrameFrontEnd._cells(out['lgrid_counts'], out['lgrid_items'], f)
+
     @staticmethod
     def bow(out, f):
         """Frame f's mBowVec / mFeatVec from the outputs of a handle with a vocabulary: ((words, values), {node: [feature, ...]}), the
@@ -2097,8 +2149,8 @@ class FrameFrontEnd:
             self._check_out(out, self.output_shapes(n, device=False))
         ptrs = {k: v.ctypes.data for k, v in out.items()}
         o = self._outputs(ptrs)
-        f = lib().hvo_frame_extract_batch_bow if wait else lib().hvo_frame_extract_batch_async_bow
-        _check(f(self._h, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs)))
+        f = lib().hvo_frame_extract_batch_grid if wait else lib().hvo_frame_extract_batch_async_grid
+        _check(f(self._h, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs), self._grid_outputs(ptrs)))
         return out
 
     @staticmethod
@@ -2111,7 +2163,8 @@ class FrameFrontEnd:
     def extract_batch_device(self, d_gray, d_depth16, n, d_ptrs):
         """d_ptrs: name -> device pointer (int) for every output of output_shapes(n).  Asynchronous."""
         o = self._outputs(d_ptrs)
-        _check(lib().hvo_frame_extract_batch_device_bow(self._h, _vp(d_gray), _vp(d_depth16), n, C.byref(o), self._bow_outputs(d_ptrs)))
+        _check(lib().hvo_frame_extract_batch_device_grid(self._h, _vp(d_gray), _vp(d_depth16), n, C.byref(o), self._bow_outputs(d_ptrs),
+                                                         self._grid_outputs(d_ptrs)))
 
     def last_launches(self):
         return lib().hvo_frame_last_launches(self._h)
@@ -2135,7 +2188,7 @@ class FrameSequence(FrameFrontEnd):
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, devices, frames_per_call=2368, bf=40.0, nfeatures=1000, scale_factor=1.2,
                  nlevels=8, ini_th=20, min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=15, line_cull=True, lanes=0, membership='u4',
-                 normals='n3', distorted=False, dist=None, vocabulary=None, levelsup=4):
+                 normals='n3', distorted=False, dist=None, vocabulary=None, levelsup=4, grids=False):
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
@@ -2151,6 +2204,7 @@ class FrameSequence(FrameFrontEnd):
         a, b, c = C.c_int(0), C.c_int(0), C.c_int(0)
         _check(lib().hvo_seq_capacities(out, C.byref(a), C.byref(b), C.byref(c)))
         self.orb_capacity, self.max_lines, self.normals_count = a.value, b.value, c.value
+        self.grids, self.line_grid_capacity = bool(grids), lib().hvo_seq_line_grid_capacity(out)
         if vocabulary is not None:
             self.set_vocabulary(vocabulary, levelsup)
 
@@ -2174,11 +2228,13 @@ class FrameSequence(FrameFrontEnd):
             raise HvoError(HVO_ERR_ARG, f'gray / depth16 must be [n, {self.h}, {self.w}]')
         if out is None:
             out = self.alloc_host(n)
-        else:   # kps_un and the BoW arrays at least: the other arrays' check is a separate change
-            self._check_out(out, {k: v for k, v in self.output_shapes(n, device=False).items() if k == 'kps_un' or k in self.BOW_FIELDS})
+        else:   # kps_un, the BoW and the grid arrays at least: the other arrays' check is a separate change
+            self._check_out(out, {k: v for k, v in self.output_shapes(n, device=False).items()
+                                  if k == 'kps_un' or k in self.BOW_FIELDS or k in self.GRID_FIELDS})
         ptrs = {k: v.ctypes.data for k, v in out.items()}
         o = self._outputs(ptrs)
-        _check(lib().hvo_seq_extract_bow(self._seq, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs)))
+        _check(lib().hvo_seq_extract_grid(self._seq, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs),
+                                          self._grid_outputs(ptrs)))
         return out
 
     def last_ms(self):

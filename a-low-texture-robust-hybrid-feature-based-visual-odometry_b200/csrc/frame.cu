@@ -25,11 +25,16 @@ const int32_t* plane_status(hvo_plane* h);
 int bow_frame_launch(hvo_bow* h, cudaStream_t s, const uint8_t* d_desc, const int32_t* d_counts, int nframes, int stride, int levelsup,
                      double* d_weight, const hvo_frame_bow_outputs* o);
 int bow_max_features();
+int proj_grid_frames_launch(cudaStream_t s, const hvo_keypoint* d_kps, const int32_t* d_counts, int nframes, int stride, float min_x, float min_y,
+                            float max_x, float max_y, uint16_t* d_cell_count, uint16_t* d_cell_items);
+int lproj_grid_frames_launch(cudaStream_t s, const hvo_keyline* d_kl, const int32_t* d_counts, int nframes, int stride, float min_x, float min_y,
+                             float max_x, float max_y, uint32_t* d_bits, uint16_t* d_cell_count, uint16_t* d_cell_items);
 }  // namespace hvo
 using namespace hvo;
 
 enum { ST_ORB = 1, ST_LINE = 2, ST_PLANE = 4, ST_NORMALS = 8 };
 static const int kMaxLanes = 8;
+static const int kGridCells = 64 * 48;   // FRAME_GRID_COLS x FRAME_GRID_ROWS
 
 // Device-side capacity faults of the pipelines (ORB quadtree arena, LSD segment buffer, plane refinement queue) are folded,
 // on the pipeline's own stream right after its kernels, into one sticky record per frame handle: fault[0] = lowest frame index
@@ -89,6 +94,7 @@ struct FrameLane {
     uint16_t* d_depth = nullptr;
     hvo_frame_outputs d_out;  // device staging of every output (host API)
     hvo_frame_bow_outputs d_bow{};  // device staging of the BoW outputs (host API; allocated while a vocabulary is attached)
+    hvo_frame_grid_outputs d_grid{};  // device staging of the grid outputs (host API; allocated by the first call that asks for grids)
 };
 
 struct hvo_frame {
@@ -107,6 +113,8 @@ struct hvo_frame {
     hvo_bow* bow = nullptr;   // attached vocabulary (hvo_frame_set_vocabulary)
     int levelsup = 4;
     double* d_bow_weight = nullptr;   // per-row leaf weights of one chunk: shared by the lanes, whose ORB kernels run in order on one stream
+    float min_x = 0.f, max_x = 0.f, min_y = 0.f, max_y = 0.f;   // mnMinX .. mnMaxY (Frame::ComputeImageBounds), the grids' bounds
+    uint32_t* d_lgrid_bits = nullptr;   // line grid bit rows of one chunk: shared by the lanes, whose line kernels run in order on one stream
 };
 
 static const int kNoFault = 0x7fffffff;
@@ -146,6 +154,14 @@ static hvo_frame_bow_outputs outputs_at(const hvo_frame* h, const hvo_frame_bow_
     if (o.word_of) r.word_of = o.word_of + off * c;
     return r;
 }
+static hvo_frame_grid_outputs outputs_at(const hvo_frame* h, const hvo_frame_grid_outputs& o, size_t off) {
+    hvo_frame_grid_outputs r = o;
+    if (o.grid_counts) r.grid_counts = o.grid_counts + off * kGridCells;
+    if (o.grid_items) r.grid_items = o.grid_items + off * (size_t)h->orb_cap;
+    if (o.lgrid_counts) r.lgrid_counts = o.lgrid_counts + off * kGridCells;
+    if (o.lgrid_items) r.lgrid_items = o.lgrid_items + off * 64 * (size_t)h->max_lines;
+    return r;
+}
 
 // The pipelines of one lane on n frames: wait for `start`, run, optionally copy each stage's results back on its own
 // stream, record the lane's join events.  Launch order = placement order: the ordered (latency-bound) pipelines first.
@@ -159,13 +175,15 @@ static hvo_frame_bow_outputs outputs_at(const hvo_frame* h, const hvo_frame_bow_
 // 16.5-17.3 K).  So a chunk of >= kSerialFrames frames runs its pipelines ONE AFTER THE OTHER (planes, lines, ORB, normals), each at
 // its saturating batch, and the download of a pipeline's results runs beside the kernels of the next one.
 // bo (device, NULL = no BoW) / host_bo (host, NULL = nothing to download): the BoW kernels follow the ORB kernels on the ORB stream; their
-// downloads are the first of phase 2.
+// downloads are the first of phase 2.  go / host_go likewise for the grids (a NULL pair = no such grid): the point grid follows the
+// undistortion on the ORB stream, the line grid the line kernels on the line stream; each is downloaded with its pipeline's results.
 // HVO_FRAME_SERIAL=0 / 1 forces one schedule (tuning aid).  Also measured for 1024-frame chunks and rejected: planes || lines first and
 // ORB || normals afterwards (87 instead of 65-79 ms), a third priority level that puts planes above lines (no change).
 static const int kSerialFrames = 2048;
 static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_t start_depth, const uint8_t* d_gray, const uint16_t* d_depth, int n,
                        int base, const hvo_frame_outputs& o, const hvo_frame_outputs* host, const hvo_frame_bow_outputs* bo,
-                       const hvo_frame_bow_outputs* host_bo, int* launches, FrameLane* after = nullptr) {
+                       const hvo_frame_bow_outputs* host_bo, const hvo_frame_grid_outputs* go, const hvo_frame_grid_outputs* host_go, int* launches,
+                       FrameLane* after = nullptr) {
     const size_t N = (size_t)n, px = (size_t)h->width * h->height;
     static const int serial_env = [] { const char* e = getenv("HVO_FRAME_SERIAL"); return e ? atoi(e) : -1; }();
     const bool serial = serial_env >= 0 ? serial_env == 1 : n >= kSerialFrames;
@@ -207,6 +225,12 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
         int st = hvo_line_extract_batch_device(L.line, d_gray, n, o.keylines, o.line_desc, o.linevec3, o.line_counts);
         if (st != HVO_OK) return st;
         *launches += hvo_line_last_launches(L.line) + 1;
+        if (go && go->lgrid_counts) {   // on the keylines returned (after cullingLine when line_cull is set), as Frame::Frame
+            st = lproj_grid_frames_launch(s, o.keylines, o.line_counts, n, h->max_lines, h->min_x, h->min_y, h->max_x, h->max_y, h->d_lgrid_bits,
+                                          go->lgrid_counts, go->lgrid_items);
+            if (st != HVO_OK) return st;
+            *launches += 2;
+        }
         k_frame_fold_status<<<(n + 255) / 256, 256, 0, s>>>(line_segment_counts(L.line), n, 0, line_segment_cap(L.line), base, FAULT_LINE, h->d_fault);
         HVO_CUDA(cudaEventRecord(L.cdone[1], s));
         prev_done = L.cdone[1];
@@ -220,6 +244,12 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
         *launches += hvo_orb_last_launches(L.orb) + 1;
         if (h->undistort) {
             st = hvo_orb_undistort_batch_device(L.orb, &h->cam, o.kps, o.kp_counts, n, o.kp_depth, h->p.bf, o.kps_un, o.kp_uright);
+            if (st != HVO_OK) return st;
+            ++*launches;
+        }
+        if (go && go->grid_counts) {    // on mvKeysUn
+            st = proj_grid_frames_launch(s, h->undistort ? o.kps_un : o.kps, o.kp_counts, n, h->orb_cap, h->min_x, h->min_y, h->max_x, h->max_y,
+                                         go->grid_counts, go->grid_items);
             if (st != HVO_OK) return st;
             ++*launches;
         }
@@ -290,6 +320,10 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
             HVO_CUDA(cudaMemcpyAsync(host->keylines, o.keylines, N * c * sizeof(hvo_keyline), cudaMemcpyDeviceToHost, s));
             HVO_CUDA(cudaMemcpyAsync(host->line_desc, o.line_desc, N * c * 32, cudaMemcpyDeviceToHost, s));
             if (host->linevec3) HVO_CUDA(cudaMemcpyAsync(host->linevec3, o.linevec3, N * c * 24, cudaMemcpyDeviceToHost, s));
+            if (host_go && host_go->lgrid_counts) {
+                HVO_CUDA(cudaMemcpyAsync(host_go->lgrid_counts, go->lgrid_counts, N * kGridCells * 2, cudaMemcpyDeviceToHost, s));
+                HVO_CUDA(cudaMemcpyAsync(host_go->lgrid_items, go->lgrid_items, N * 64 * c * 2, cudaMemcpyDeviceToHost, s));
+            }
         }
         timeline_mark(s, "end_lines");
         HVO_CUDA(cudaEventRecord(L.join[1], s));
@@ -305,6 +339,10 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
             if (host->kp_depth) HVO_CUDA(cudaMemcpyAsync(host->kp_depth, o.kp_depth, N * c * 4, cudaMemcpyDeviceToHost, s));
             if (host->kp_uright) HVO_CUDA(cudaMemcpyAsync(host->kp_uright, o.kp_uright, N * c * 4, cudaMemcpyDeviceToHost, s));
             if (host->kps_un) HVO_CUDA(cudaMemcpyAsync(host->kps_un, o.kps_un, N * c * sizeof(hvo_keypoint), cudaMemcpyDeviceToHost, s));
+            if (host_go && host_go->grid_counts) {
+                HVO_CUDA(cudaMemcpyAsync(host_go->grid_counts, go->grid_counts, N * kGridCells * 2, cudaMemcpyDeviceToHost, s));
+                HVO_CUDA(cudaMemcpyAsync(host_go->grid_items, go->grid_items, N * c * 2, cudaMemcpyDeviceToHost, s));
+            }
         }
         timeline_mark(s, "end_orb");
         HVO_CUDA(cudaEventRecord(L.join[0], s));
@@ -432,6 +470,10 @@ int hvo_frame_create(const hvo_frame_params* p, int width, int height, int max_b
     h->orb_cap = L0.orb ? hvo_orb_capacity(L0.orb) : 0;
     h->max_lines = L0.line ? hvo_line_max_lines(L0.line) : 0;
     h->normals_count = L0.normals ? hvo_normals_count(L0.normals) : 0;
+    // Frame::ComputeImageBounds; a handle that does not undistort has the reference's k1 == 0 bounds
+    h->max_x = (float)width; h->max_y = (float)height;
+    if (h->undistort) st = hvo_image_bounds(&h->cam, width, height, &h->min_x, &h->max_x, &h->min_y, &h->max_y);
+    if (st != HVO_OK) { hvo_frame_destroy(h); return st; }
     do {
 #define HVO_TRY(call) if ((call) != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(cudaGetLastError())); st = HVO_ERR_CUDA; break; }
         HVO_TRY(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
@@ -524,12 +566,15 @@ void hvo_frame_destroy(hvo_frame* h) {
         void* bufs[] = {L.d_gray, L.d_depth, o.kps, o.desc, o.kp_counts, o.kp_depth, o.kp_uright, o.keylines, o.line_desc, o.linevec3,
                         o.line_counts, o.n_planes, o.planes7, o.membership, o.membership8, o.normals8, o.membership4, o.normals3, o.kps_un};
         for (void* b : bufs) if (b) cudaFree(b);
+        void* gbufs[] = {L.d_grid.grid_counts, L.d_grid.grid_items, L.d_grid.lgrid_counts, L.d_grid.lgrid_items};
+        for (void* b : gbufs) if (b) cudaFree(b);
         if (L.fork) cudaEventDestroy(L.fork);
         for (auto& e : L.join) if (e) cudaEventDestroy(e);
         for (auto& e : L.cdone) if (e) cudaEventDestroy(e);
         if (L.up) cudaStreamDestroy(L.up);
     }
     if (h->d_fault) cudaFree(h->d_fault);
+    if (h->d_lgrid_bits) cudaFree(h->d_lgrid_bits);
     if (h->h_fault) cudaFreeHost(h->h_fault);
     if (h->fork) cudaEventDestroy(h->fork);
     for (auto& e : h->tev) if (e) cudaEventDestroy(e);
@@ -576,6 +621,40 @@ static int frame_check_bow_outputs(const hvo_frame* h, const hvo_frame_bow_outpu
     return HVO_OK;
 }
 
+static int frame_check_grid_outputs(const hvo_frame* h, const hvo_frame_grid_outputs* g, const hvo_frame_outputs* o, bool device) {
+    if (!g) return HVO_OK;
+    HVO_CHECK_ARG(!g->grid_counts == !g->grid_items && !g->lgrid_counts == !g->lgrid_items, "grid_counts / grid_items and lgrid_counts / lgrid_items go in pairs");
+    if (g->grid_counts) {
+        HVO_CHECK_ARG(h->p.stages & ST_ORB, "point grid outputs need the ORB stage");
+        HVO_CHECK_ARG(h->orb_cap <= 65535, "point grid outputs need orb_capacity <= 65535 (uint16 items)");
+        if (device && h->undistort) HVO_CHECK_ARG(o->kps_un, "point grids of an undistorting handle are built on kps_un: the device call needs it");
+    }
+    if (g->lgrid_counts) {
+        HVO_CHECK_ARG(h->p.stages & ST_LINE, "line grid outputs need the line stage");
+        HVO_CHECK_ARG(h->max_lines <= 65535, "line grid outputs need max_lines <= 65535 (uint16 items)");
+    }
+    return HVO_OK;
+}
+
+// Allocated by the first call that asks for a grid, kept until destroy: the line grid's bit rows (one chunk, shared by the lanes) and, for
+// the host calls, every lane's device staging of the requested grids.
+static int frame_reserve_grids(hvo_frame* h, const hvo_frame_grid_outputs* g, bool host) {
+    const size_t B = (size_t)h->lane[0].cap;
+    if (g->lgrid_counts && !h->d_lgrid_bits) HVO_CUDA(cudaMalloc(&h->d_lgrid_bits, B * kGridCells * div_up(h->max_lines, 32) * sizeof(uint32_t)));
+    for (int li = 0; host && li < h->nlanes; ++li) {
+        hvo_frame_grid_outputs& o = h->lane[li].d_grid;
+        if (g->grid_counts) {
+            if (!o.grid_counts) HVO_CUDA(cudaMalloc(&o.grid_counts, B * kGridCells * 2));
+            if (!o.grid_items) HVO_CUDA(cudaMalloc(&o.grid_items, B * h->orb_cap * 2));
+        }
+        if (g->lgrid_counts) {
+            if (!o.lgrid_counts) HVO_CUDA(cudaMalloc(&o.lgrid_counts, B * kGridCells * 2));
+            if (!o.lgrid_items) HVO_CUDA(cudaMalloc(&o.lgrid_items, B * 64 * h->max_lines * 2));
+        }
+    }
+    return HVO_OK;
+}
+
 int hvo_frame_set_vocabulary(hvo_frame* h, int n_nodes, const int32_t* child_start, const int32_t* child_ids, const uint8_t* node_desc,
                              const double* node_weight, const int32_t* node_word, int depth_levels, int levelsup) {
     HVO_CHECK_ARG(h, "null handle");
@@ -611,16 +690,18 @@ int hvo_frame_set_vocabulary(hvo_frame* h, int n_nodes, const int32_t* child_sta
     return HVO_OK;
 }
 
-int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
-                                       const hvo_frame_bow_outputs* d_bow) {
+int hvo_frame_extract_batch_device_grid(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                        const hvo_frame_bow_outputs* d_bow, const hvo_frame_grid_outputs* d_grid) {
     HVO_CHECK_ARG(h && d_gray && d_depth16, "null argument");
     HVO_CHECK_ARG(nframes >= 1 && nframes <= h->max_batch, "nframes out of range for this handle");
     int st = frame_check_outputs(h, d_out, true);
     if (st == HVO_OK) st = frame_check_bow_outputs(h, d_bow, true);
+    if (st == HVO_OK) st = frame_check_grid_outputs(h, d_grid, d_out, true);
     if (st != HVO_OK) return st;
     if (h->p.stages & ST_ORB) HVO_CHECK_ARG(d_out->kp_depth && d_out->kp_uright, "kp_depth / kp_uright missing");
     if (h->p.stages & ST_LINE) HVO_CHECK_ARG(d_out->linevec3, "linevec3 missing");
     HVO_CUDA(cudaSetDevice(h->device));
+    if (d_grid && (st = frame_reserve_grids(h, d_grid, false)) != HVO_OK) return st;
     const size_t px = (size_t)h->width * h->height;
     HVO_CUDA(cudaEventRecord(h->fork, h->stream));
     int launches = 0, used = 0;
@@ -634,8 +715,9 @@ int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, cons
         FrameLane& L = h->lane[used];
         const int n = std::min(per, nframes - off);
         const hvo_frame_bow_outputs bo = d_bow ? outputs_at(h, *d_bow, (size_t)off) : hvo_frame_bow_outputs{};
+        const hvo_frame_grid_outputs go = d_grid ? outputs_at(h, *d_grid, (size_t)off) : hvo_frame_grid_outputs{};
         st = lane_launch(h, L, h->fork, nullptr, d_gray + (size_t)off * px, d_depth16 + (size_t)off * px, n, off, outputs_at(h, *d_out, (size_t)off), nullptr,
-                         d_bow ? &bo : nullptr, nullptr, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
+                         d_bow ? &bo : nullptr, nullptr, d_grid ? &go : nullptr, nullptr, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
         if (st != HVO_OK) return st;
         h->last_lane = used;
     }
@@ -647,18 +729,25 @@ int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, cons
     return HVO_OK;
 }
 
-int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out) {
-    return hvo_frame_extract_batch_device_bow(h, d_gray, d_depth16, nframes, d_out, nullptr);
+int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                       const hvo_frame_bow_outputs* d_bow) {
+    return hvo_frame_extract_batch_device_grid(h, d_gray, d_depth16, nframes, d_out, d_bow, nullptr);
 }
 
-int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
-                                      const hvo_frame_bow_outputs* bow) {
+int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out) {
+    return hvo_frame_extract_batch_device_grid(h, d_gray, d_depth16, nframes, d_out, nullptr, nullptr);
+}
+
+int hvo_frame_extract_batch_async_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                       const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
     HVO_CHECK_ARG(h && gray && depth16, "null argument");
     HVO_CHECK_ARG(nframes >= 1, "nframes < 1");
     int st = frame_check_outputs(h, out, false);
     if (st == HVO_OK) st = frame_check_bow_outputs(h, bow, false);
+    if (st == HVO_OK) st = frame_check_grid_outputs(h, grid, out, false);
     if (st != HVO_OK) return st;
     HVO_CUDA(cudaSetDevice(h->device));
+    if (grid && (st = frame_reserve_grids(h, grid, true)) != HVO_OK) return st;
     const size_t px = (size_t)h->width * h->height;
     // chunks: as few as the lane capacity allows, of equal size.  Chunks go round-robin through the lanes ACROSS calls
     // (next_lane), so that the upload of a one-chunk call overlaps the kernels of the previous call on the other lane.
@@ -684,11 +773,15 @@ int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const u
         if (!out->membership8 && !out->membership4) d.membership8 = nullptr;
         if (!out->membership4) d.membership4 = nullptr;
         if (!out->normals3) d.normals3 = nullptr;
-        if (!out->kps_un) d.kps_un = nullptr;
+        if (!out->kps_un && !(grid && grid->grid_counts)) d.kps_un = nullptr;   // (the point grid is built on kps_un)
+        hvo_frame_grid_outputs dg{};   // the requested pairs of the lane's grid staging
+        if (grid && grid->grid_counts) { dg.grid_counts = L.d_grid.grid_counts; dg.grid_items = L.d_grid.grid_items; }
+        if (grid && grid->lgrid_counts) { dg.lgrid_counts = L.d_grid.lgrid_counts; dg.lgrid_items = L.d_grid.lgrid_items; }
         const hvo_frame_outputs hostk = outputs_at(h, *out, (size_t)off);
         const hvo_frame_bow_outputs hostb = bow ? outputs_at(h, *bow, (size_t)off) : hvo_frame_bow_outputs{};
-        st = lane_launch(h, L, L.fork, L.fork_depth, L.d_gray, L.d_depth, n, off, d, &hostk, bow ? &L.d_bow : nullptr, bow ? &hostb : nullptr, &launches,
-                         h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
+        const hvo_frame_grid_outputs hostg = grid ? outputs_at(h, *grid, (size_t)off) : hvo_frame_grid_outputs{};
+        st = lane_launch(h, L, L.fork, L.fork_depth, L.d_gray, L.d_depth, n, off, d, &hostk, bow ? &L.d_bow : nullptr, bow ? &hostb : nullptr,
+                         grid ? &dg : nullptr, grid ? &hostg : nullptr, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
         if (st != HVO_OK) return st;
         h->last_lane = li;
     }
@@ -701,21 +794,39 @@ int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const u
     return HVO_OK;
 }
 
-int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
-    return hvo_frame_extract_batch_async_bow(h, gray, depth16, nframes, out, nullptr);
+int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                      const hvo_frame_bow_outputs* bow) {
+    return hvo_frame_extract_batch_async_grid(h, gray, depth16, nframes, out, bow, nullptr);
 }
 
-int hvo_frame_extract_batch_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
-                                const hvo_frame_bow_outputs* bow) {
-    const int st = hvo_frame_extract_batch_async_bow(h, gray, depth16, nframes, out, bow);
+int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+    return hvo_frame_extract_batch_async_grid(h, gray, depth16, nframes, out, nullptr, nullptr);
+}
+
+int hvo_frame_extract_batch_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                 const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
+    const int st = hvo_frame_extract_batch_async_grid(h, gray, depth16, nframes, out, bow, grid);
     if (st != HVO_OK) return st;
     HVO_CUDA(cudaStreamSynchronize(h->stream));
     return frame_check_fault(h);
 }
 
-int hvo_frame_extract_batch(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
-    return hvo_frame_extract_batch_bow(h, gray, depth16, nframes, out, nullptr);
+int hvo_frame_extract_batch_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                const hvo_frame_bow_outputs* bow) {
+    return hvo_frame_extract_batch_grid(h, gray, depth16, nframes, out, bow, nullptr);
 }
+
+int hvo_frame_extract_batch(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+    return hvo_frame_extract_batch_grid(h, gray, depth16, nframes, out, nullptr, nullptr);
+}
+
+int hvo_frame_image_bounds(const hvo_frame* h, float* min_x, float* max_x, float* min_y, float* max_y) {
+    HVO_CHECK_ARG(h && min_x && max_x && min_y && max_y, "null argument");
+    *min_x = h->min_x; *max_x = h->max_x; *min_y = h->min_y; *max_y = h->max_y;
+    return HVO_OK;
+}
+
+int hvo_frame_line_grid_capacity(const hvo_frame* h) { return h ? 64 * h->max_lines : 0; }
 
 int hvo_frame_last_launches(const hvo_frame* h) { return h ? h->last_launches : 0; }
 int hvo_frame_sync(hvo_frame* h) {

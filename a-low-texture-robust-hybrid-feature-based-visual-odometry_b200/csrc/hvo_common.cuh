@@ -54,6 +54,27 @@ void timeline_mark(cudaStream_t s, const char* name);
 static inline int div_up(int a, int b) { return (a + b - 1) / b; }
 static inline size_t align_up(size_t a, size_t b) { return (a + b - 1) / b * b; }
 
+// Exclusive scan over a 1024-thread CTA of 3 consecutive values per thread (the 64 x 48 = 3072 cells of a frame grid): returns the
+// prefix of thread tid's first value.  s_part: 32 ints of shared memory; ends with a __syncthreads, so s_part may be reused.
+__device__ __forceinline__ int block_exclusive_scan3(int sum, int* s_part) {
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    int pre = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, pre, o); if (lane >= o) pre += t; }
+    if (lane == 31) s_part[wid] = pre;
+    __syncthreads();
+    if (wid == 0) {
+        int w = s_part[lane];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, w, o); if (lane >= o) w += t; }
+        s_part[lane] = w;
+    }
+    __syncthreads();
+    const int base = pre - sum + (wid > 0 ? s_part[wid - 1] : 0);
+    __syncthreads();
+    return base;
+}
+
 __device__ __forceinline__ int reflect101(int p, int n) {
     // single reflection is enough for |overshoot| < n (halo radii here are <= 21 px)
     if (p < 0) p = -p;

@@ -11,7 +11,8 @@
 // cell row; the 32 lines of a word are tested in parallel and folded into best / second in ascending order, which is the
 // order the reference visits them in.  Lines accepted into the candidate list are remembered in a per-warp bit row (the
 // reference's unordered_set).  The greedy "skip lines that already hold a map line" rule is resolved like the point
-// matcher's (project.cu): rounds over all queries until no choice changes.
+// matcher's (project.cu): rounds over all queries until no choice changes.  The frame pipeline builds the bit rows of every frame of a call
+// (k_lproj_grid, one thread per (frame, line)) and compacts them into mGridForLine's counts and items (k_lproj_grid_compact).
 #include <algorithm>
 #include <climits>
 #include <new>
@@ -43,19 +44,27 @@ struct LQuery {  // hvo_lproj_query
 };
 static_assert(sizeof(LQuery) == sizeof(hvo_lproj_query), "query layout");
 
-// one thread per line: ORB_SLAM2::LineIterator over the grid (doubles), one atomicOr per visited cell
-__global__ void k_lproj_grid(const hvo_keyline* __restrict__ kl, int n, LGridGeom g, int W, uint32_t* __restrict__ cells, LKey* __restrict__ keys) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+// One thread per (frame, line): ORB_SLAM2::LineIterator over the grid (doubles), one atomicOr per visited cell.  Frame f = blockIdx.x:
+// keyline rows [f * stride, + n_f), n_f = counts ? counts[f] : n, bit rows at cells + f * 3072 * W; keys (NULL in the frame pipeline)
+// receives the LKey rows.
+__global__ void k_lproj_grid(const hvo_keyline* __restrict__ kl, int n, const int32_t* __restrict__ counts, int stride, LGridGeom g, int W,
+                             uint32_t* __restrict__ cells, LKey* __restrict__ keys) {
+    const int i = blockIdx.y * blockDim.x + threadIdx.x, f = blockIdx.x;
+    if (counts) n = min(counts[f], stride);
     if (i >= n) return;
-    const hvo_keyline k = kl[i];
-    LKey o;
-    o.sx = k.startPointX; o.sy = k.startPointY;
-    float dx = __fsub_rn(k.startPointX, k.endPointX), dy = __fsub_rn(k.startPointY, k.endPointY);
-    const float nrm = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
-    o.d2x = __fdiv_rn(dx, nrm); o.d2y = __fdiv_rn(dy, nrm);
-    o.ocx = __fsub_rn(k.ePointInOctaveX, k.sPointInOctaveX); o.ocy = __fsub_rn(k.ePointInOctaveY, k.sPointInOctaveY);
-    o.length = k.lineLength; o.octave = k.octave;
-    keys[i] = o;
+    const hvo_keyline k = kl[(size_t)f * stride + i];
+    cells += (size_t)f * kLGridCells * W;
+    if (keys) {
+        LKey o;
+        o.sx = k.startPointX; o.sy = k.startPointY;
+        float dx = __fsub_rn(k.startPointX, k.endPointX), dy = __fsub_rn(k.startPointY, k.endPointY);
+        const float nrm = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
+        o.d2x = __fdiv_rn(dx, nrm); o.d2y = __fdiv_rn(dy, nrm);
+        o.ocx = __fsub_rn(k.ePointInOctaveX, k.sPointInOctaveX); o.ocy = __fsub_rn(k.ePointInOctaveY, k.sPointInOctaveY);
+        o.length = k.lineLength; o.octave = k.octave;
+        keys[i] = o;
+    }
+    // the reference walks endpoint * inv without the min_x / min_y offset (Frame.cc:849-872)
     double x1 = (double)__fmul_rn(k.startPointX, g.inv_w), y1 = (double)__fmul_rn(k.startPointY, g.inv_h);
     double x2 = (double)__fmul_rn(k.endPointX, g.inv_w), y2 = (double)__fmul_rn(k.endPointY, g.inv_h);
     const bool steep = fabs(y2 - y1) > fabs(x2 - x1);
@@ -72,6 +81,53 @@ __global__ void k_lproj_grid(const hvo_keyline* __restrict__ kl, int n, LGridGeo
         error -= ddy;
         if (error < 0) { y += ystep; error += ddx; }
     }
+}
+
+// One CTA per frame: bit rows -> mGridForLine as counts [f][3072] + items [f][items_stride], a cell's lines ascending (the reference's
+// push_back order).  Only the first sum(counts) items are written.
+__global__ void __launch_bounds__(1024) k_lproj_grid_compact(const uint32_t* __restrict__ cells, int W, uint16_t* __restrict__ cell_count,
+                                                             uint16_t* __restrict__ cell_items, int items_stride) {
+    __shared__ int s_part[32];
+    const int tid = threadIdx.x, f = blockIdx.x;
+    cells += (size_t)f * kLGridCells * W;
+    cell_items += (size_t)f * items_stride;
+    int v[3], sum = 0;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const uint32_t* row = cells + (size_t)(tid * 3 + k) * W;
+        int c = 0;
+        for (int w = 0; w < W; ++w) c += __popc(row[w]);
+        v[k] = c; sum += c;
+    }
+    int o = block_exclusive_scan3(sum, s_part);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        cell_count[(size_t)f * kLGridCells + tid * 3 + k] = (uint16_t)v[k];
+        const uint32_t* row = cells + (size_t)(tid * 3 + k) * W;
+        for (int w = 0; w < W; ++w)
+            for (uint32_t b = row[w]; b; b &= b - 1) cell_items[o++] = (uint16_t)(32 * w + __ffs(b) - 1);
+    }
+}
+
+static LGridGeom lgrid_geom(float min_x, float min_y, float max_x, float max_y) {
+    LGridGeom g;
+    g.min_x = min_x; g.min_y = min_y;
+    g.inv_w = (float)kLGridCols / (max_x - min_x);   // Frame.cc:419-420
+    g.inv_h = (float)kLGridRows / (max_y - min_y);
+    return g;
+}
+
+// The frame pipeline's line grids (hvo_frame_grid_outputs): nframes frames of `stride` keyline rows, counts on the device; d_bits =
+// scratch of nframes * 3072 * ceil(stride / 32) words.  A line visits at most 64 in-grid cells (LineIterator advances the major axis
+// by one cell per step), so 64 * stride items per frame always suffice.
+int lproj_grid_frames_launch(cudaStream_t s, const hvo_keyline* d_kl, const int32_t* d_counts, int nframes, int stride, float min_x, float min_y,
+                             float max_x, float max_y, uint32_t* d_bits, uint16_t* d_cell_count, uint16_t* d_cell_items) {
+    const int W = div_up(stride, 32);
+    HVO_CUDA(cudaMemsetAsync(d_bits, 0, (size_t)nframes * kLGridCells * W * sizeof(uint32_t), s));
+    k_lproj_grid<<<dim3(nframes, div_up(stride, 128)), 128, 0, s>>>(d_kl, 0, d_counts, stride, lgrid_geom(min_x, min_y, max_x, max_y), W, d_bits, nullptr);
+    k_lproj_grid_compact<<<nframes, 1024, 0, s>>>(d_bits, W, d_cell_count, d_cell_items, kLGridCols * stride);
+    HVO_CUDA(cudaGetLastError());
+    return HVO_OK;
 }
 
 // Walks GetFeaturesInAreaForLine for one query (whole warp).  visit(id, pass, sample) is called once per word of candidate
@@ -372,9 +428,7 @@ int hvo_lproj_set_frame(hvo_lproj* h, const hvo_keyline* keylines_un, const doub
     h->n = n;
     h->W = std::max(1, div_up(n, 32));
     h->has3d = lines3d != nullptr;
-    h->g.min_x = min_x; h->g.min_y = min_y;
-    h->g.inv_w = (float)kLGridCols / (max_x - min_x);   // Frame.cc:419-420
-    h->g.inv_h = (float)kLGridRows / (max_y - min_y);
+    h->g = lgrid_geom(min_x, min_y, max_x, max_y);
     cudaStream_t s = h->stream;
     HVO_CUDA(cudaMemsetAsync(h->d_cells, 0, (size_t)kLGridCells * h->W * sizeof(uint32_t), s));
     if (n > 0) {
@@ -382,7 +436,7 @@ int hvo_lproj_set_frame(hvo_lproj* h, const hvo_keyline* keylines_un, const doub
         HVO_CUDA(cudaMemcpyAsync(h->d_func, line_functions, (size_t)n * 24, cudaMemcpyHostToDevice, s));
         HVO_CUDA(cudaMemcpyAsync(h->d_desc, desc, (size_t)n * 32, cudaMemcpyHostToDevice, s));
         if (lines3d) HVO_CUDA(cudaMemcpyAsync(h->d_l3d, lines3d, (size_t)n * 48, cudaMemcpyHostToDevice, s));
-        k_lproj_grid<<<div_up(n, 128), 128, 0, s>>>(h->d_kl, n, h->g, h->W, h->d_cells, h->d_keys);
+        k_lproj_grid<<<dim3(1, div_up(n, 128)), 128, 0, s>>>(h->d_kl, n, nullptr, 0, h->g, h->W, h->d_cells, h->d_keys);
         HVO_CUDA(cudaGetLastError());
     }
     HVO_CUDA(cudaStreamSynchronize(s));  // the host arrays may be released on return

@@ -6,8 +6,9 @@
 //   ORBmatcher::SearchByProjection(F, MapPoints)    src/ORBmatcher.cc:45-132          (mode 0)
 //   ORBmatcher::SearchByProjection(Cur, Last / KF)  src/ORBmatcher.cc:1353-1497, 1499-1628   (mode 1, matching part)
 //
-//   k_proj_grid    one CTA: cell of every keypoint (round), histogram, exclusive scan, scatter, per-cell index sort, so a
-//                  cell lists its keypoints in index order exactly like the reference's push_back loop
+//   k_proj_grid    one CTA per frame: cell of every keypoint (round), histogram, exclusive scan, scatter, per-cell index sort, so a
+//                  cell lists its keypoints in index order exactly like the reference's push_back loop (hvo_proj_set_frame: one
+//                  frame; the frame pipeline: every frame of a call, hvo_frame_grid_outputs)
 //   k_proj_round   one warp per query: the cells of the window in the reference's order (ix outer, iy inner; the iy run of
 //                  one ix is contiguous in memory), 32 candidates at a time: level / window / right-coordinate filters and
 //                  8 x __popc per lane, then the reference's sequential best / second update over the surviving lanes
@@ -33,61 +34,87 @@ struct ProjKey { float x, y; int octave; float uright; };  // 16 bytes per keypo
 struct ProjQuery { float u, v, r; int min_level, max_level; float ur; int claims; int pad; };  // hvo_proj_query
 struct GridGeom { float min_x, min_y, inv_w, inv_h; };
 
+// Frame::PosInGrid (Frame.cc:1680-1690): the cell (ix * 48 + iy) of an undistorted keypoint, -1 outside the grid
+__device__ __forceinline__ int pos_in_grid(const GridGeom& g, float x, float y) {
+    const int px = (int)roundf(__fmul_rn(__fsub_rn(x, g.min_x), g.inv_w)), py = (int)roundf(__fmul_rn(__fsub_rn(y, g.min_y), g.inv_h));
+    return (px >= 0 && px < kGridCols && py >= 0 && py < kGridRows) ? px * kGridRows + py : -1;
+}
+
+// One CTA per frame: frame f = keypoint rows [f * stride, + n_f), n_f = counts ? counts[f] : n.  Outputs of frame f: cell_start
+// [3073] (exclusive scan; NULL in the frame pipeline) or cell_count [f][3072]; cell_items [f][stride] (the first sum(counts) entries
+// written); pk [n] ProjKey rows (NULL in the frame pipeline).
+template <class Item>
 __global__ void __launch_bounds__(1024) k_proj_grid(const hvo_keypoint* __restrict__ keys, const float* __restrict__ uright, int n,
-                                                    GridGeom g, ProjKey* __restrict__ pk, int* __restrict__ cell_start,
-                                                    int* __restrict__ cell_items, int* __restrict__ cell_of) {
+                                                    const int32_t* __restrict__ counts, int stride, GridGeom g, ProjKey* __restrict__ pk,
+                                                    int* __restrict__ cell_start, uint16_t* __restrict__ cell_count, Item* __restrict__ cell_items) {
     __shared__ int s_cnt[kGridCells];
     __shared__ int s_part[32];
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int tid = threadIdx.x, f = blockIdx.x;
+    if (counts) n = min(counts[f], stride);
+    keys += (size_t)f * stride;
+    cell_items += (size_t)f * stride;
     for (int c = tid; c < kGridCells; c += 1024) s_cnt[c] = 0;
     __syncthreads();
     for (int i = tid; i < n; i += 1024) {
         const hvo_keypoint k = keys[i];
-        ProjKey p;
-        p.x = k.x; p.y = k.y; p.octave = k.octave; p.uright = uright ? uright[i] : -1.f;
-        pk[i] = p;
-        const int px = (int)roundf(__fmul_rn(__fsub_rn(k.x, g.min_x), g.inv_w)), py = (int)roundf(__fmul_rn(__fsub_rn(k.y, g.min_y), g.inv_h));
-        int c = -1;
-        if (px >= 0 && px < kGridCols && py >= 0 && py < kGridRows) { c = px * kGridRows + py; atomicAdd(&s_cnt[c], 1); }
-        cell_of[i] = c;
+        if (pk) {
+            ProjKey p;
+            p.x = k.x; p.y = k.y; p.octave = k.octave; p.uright = uright ? uright[i] : -1.f;
+            pk[i] = p;
+        }
+        const int c = pos_in_grid(g, k.x, k.y);
+        if (c >= 0) atomicAdd(&s_cnt[c], 1);
     }
     __syncthreads();
     // exclusive scan of the 3072 counts: 3 per thread
-    int v[3], sum = 0;
+    int v[3], start[3], sum = 0;
 #pragma unroll
     for (int k = 0; k < 3; ++k) { v[k] = s_cnt[tid * 3 + k]; sum += v[k]; }
-    int pre = sum;
+    int base = block_exclusive_scan3(sum, s_part);
 #pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, pre, o); if (lane >= o) pre += t; }
-    if (lane == 31) s_part[wid] = pre;
-    __syncthreads();
-    if (wid == 0) {
-        int w = s_part[lane];
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, w, o); if (lane >= o) w += t; }
-        s_part[lane] = w;
+    for (int k = 0; k < 3; ++k) {
+        const int c = tid * 3 + k;
+        if (cell_start) cell_start[c] = base;
+        if (cell_count) cell_count[(size_t)f * kGridCells + c] = (uint16_t)v[k];
+        start[k] = s_cnt[c] = base;
+        base += v[k];
     }
-    __syncthreads();
-    int base = pre - sum + (wid > 0 ? s_part[wid - 1] : 0);
-#pragma unroll
-    for (int k = 0; k < 3; ++k) { cell_start[tid * 3 + k] = base; s_cnt[tid * 3 + k] = base; base += v[k]; }
-    if (tid == 1023) cell_start[kGridCells] = base;
+    if (cell_start && tid == 1023) cell_start[kGridCells] = base;
     __syncthreads();
     for (int i = tid; i < n; i += 1024) {
-        const int c = cell_of[i];
-        if (c >= 0) cell_items[atomicAdd(&s_cnt[c], 1)] = i;
+        const hvo_keypoint k = keys[i];
+        const int c = pos_in_grid(g, k.x, k.y);
+        if (c >= 0) cell_items[atomicAdd(&s_cnt[c], 1)] = (Item)i;
     }
     __syncthreads();
     // a cell lists its keypoints in index order (reference: push_back in the i loop)
-    for (int c = tid; c < kGridCells; c += 1024) {
-        const int b = cell_start[c], e = s_cnt[c];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const int b = start[k], e = b + v[k];
         for (int i = b + 1; i < e; ++i) {
-            const int x = cell_items[i];
+            const Item x = cell_items[i];
             int j = i - 1;
             while (j >= b && cell_items[j] > x) { cell_items[j + 1] = cell_items[j]; --j; }
             cell_items[j + 1] = x;
         }
     }
+}
+
+static GridGeom grid_geom(float min_x, float min_y, float max_x, float max_y) {
+    GridGeom g;
+    g.min_x = min_x; g.min_y = min_y;
+    g.inv_w = (float)kGridCols / (max_x - min_x);   // Frame.cc:419-420
+    g.inv_h = (float)kGridRows / (max_y - min_y);
+    return g;
+}
+
+// The frame pipeline's point grids (hvo_frame_grid_outputs): nframes frames of `stride` keypoint rows, counts on the device.
+int proj_grid_frames_launch(cudaStream_t s, const hvo_keypoint* d_kps, const int32_t* d_counts, int nframes, int stride, float min_x, float min_y,
+                            float max_x, float max_y, uint16_t* d_cell_count, uint16_t* d_cell_items) {
+    k_proj_grid<uint16_t><<<nframes, 1024, 0, s>>>(d_kps, nullptr, 0, d_counts, stride, grid_geom(min_x, min_y, max_x, max_y), nullptr, nullptr,
+                                                   d_cell_count, d_cell_items);
+    HVO_CUDA(cudaGetLastError());
+    return HVO_OK;
 }
 
 struct ProjWindow { int x0, x1, y0, y1; bool empty; };
@@ -487,7 +514,7 @@ struct hvo_proj {
     float* d_uright = nullptr;
     uint8_t* d_desc = nullptr;
     ProjKey* d_pk = nullptr;
-    int *d_cell_start = nullptr, *d_cell_items = nullptr, *d_cell_of = nullptr;
+    int *d_cell_start = nullptr, *d_cell_items = nullptr;
     uint8_t* d_claimed = nullptr;
     int *d_claim0 = nullptr, *d_claim_a = nullptr, *d_claim_b = nullptr;
     ProjQuery* d_q = nullptr;
@@ -522,7 +549,7 @@ static int proj_reserve_keys(hvo_proj* h, int n) {
     const int cap = std::max(n, 2048);
     int st;
     if ((st = grow(h->d_keys, cap)) || (st = grow(h->d_uright, cap)) || (st = grow(h->d_desc, (size_t)cap * 32)) || (st = grow(h->d_pk, cap)) ||
-        (st = grow(h->d_cell_items, cap)) || (st = grow(h->d_cell_of, cap)) || (st = grow(h->d_claimed, cap)) || (st = grow(h->d_claim0, cap)) ||
+        (st = grow(h->d_cell_items, cap)) || (st = grow(h->d_claimed, cap)) || (st = grow(h->d_claim0, cap)) ||
         (st = grow(h->d_claim_a, cap)) || (st = grow(h->d_claim_b, cap)) || (st = grow(h->d_area, cap)))
         return st;
     h->kcap = cap;
@@ -574,7 +601,7 @@ void hvo_proj_destroy(hvo_proj* h) {
     if (!h) return;
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    void* bufs[] = {h->d_keys, h->d_uright, h->d_desc, h->d_pk, h->d_cell_start, h->d_cell_items, h->d_cell_of, h->d_claimed, h->d_claim0,
+    void* bufs[] = {h->d_keys, h->d_uright, h->d_desc, h->d_pk, h->d_cell_start, h->d_cell_items, h->d_claimed, h->d_claim0,
                     h->d_claim_a, h->d_claim_b, h->d_q, h->d_qdesc, h->d_choice, h->d_cdist, h->d_flag, h->d_area, h->d_off, h->d_cand, h->d_best4,
                     h->d_inv_sigma2, h->d_thr, h->d_pts, h->d_track, h->d_skip, h->d_claims, h->d_m21, h->d_mdist};
     for (void* b : bufs) if (b) cudaFree(b);
@@ -593,16 +620,15 @@ int hvo_proj_set_frame(hvo_proj* h, const hvo_keypoint* keys_un, const float* ur
     int st = proj_reserve_keys(h, n);
     if (st != HVO_OK) return st;
     h->n = n;
-    h->g.min_x = min_x; h->g.min_y = min_y;
-    h->g.inv_w = (float)kGridCols / (max_x - min_x);   // Frame.cc:419-420
-    h->g.inv_h = (float)kGridRows / (max_y - min_y);
+    h->g = grid_geom(min_x, min_y, max_x, max_y);
     h->gw = h->g;
     if (n > 0) {
         HVO_CUDA(cudaMemcpyAsync(h->d_keys, keys_un, (size_t)n * sizeof(hvo_keypoint), cudaMemcpyHostToDevice, h->stream));
         if (uright) HVO_CUDA(cudaMemcpyAsync(h->d_uright, uright, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
         HVO_CUDA(cudaMemcpyAsync(h->d_desc, desc, (size_t)n * 32, cudaMemcpyHostToDevice, h->stream));
     }
-    k_proj_grid<<<1, 1024, 0, h->stream>>>(h->d_keys, uright ? h->d_uright : nullptr, n, h->g, h->d_pk, h->d_cell_start, h->d_cell_items, h->d_cell_of);
+    k_proj_grid<int><<<1, 1024, 0, h->stream>>>(h->d_keys, uright ? h->d_uright : nullptr, n, nullptr, 0, h->g, h->d_pk, h->d_cell_start, nullptr,
+                                                 h->d_cell_items);
     HVO_CUDA(cudaGetLastError());
     h->last_launches = 1;
     return HVO_OK;

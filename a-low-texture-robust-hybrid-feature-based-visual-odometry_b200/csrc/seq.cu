@@ -57,6 +57,15 @@ static hvo_frame_bow_outputs seq_outputs_at(const hvo_seq* s, const hvo_frame_bo
     return r;
 }
 
+static hvo_frame_grid_outputs seq_outputs_at(const hvo_seq* s, const hvo_frame_grid_outputs& o, size_t off) {
+    hvo_frame_grid_outputs r = o;
+    if (o.grid_counts) r.grid_counts = o.grid_counts + off * 3072;
+    if (o.grid_items) r.grid_items = o.grid_items + off * (size_t)s->orb_cap;
+    if (o.lgrid_counts) r.lgrid_counts = o.lgrid_counts + off * 3072;
+    if (o.lgrid_items) r.lgrid_items = o.lgrid_items + off * 64 * (size_t)s->max_lines;
+    return r;
+}
+
 extern "C" {
 
 int hvo_seq_create(const hvo_frame_params* p, int width, int height, const int* devices, int ndevices, int frames_per_call, hvo_seq** out) {
@@ -111,8 +120,8 @@ int hvo_seq_set_vocabulary(hvo_seq* s, int n_nodes, const int32_t* child_start, 
     return HVO_OK;
 }
 
-int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
-                        const hvo_frame_bow_outputs* bow) {
+int hvo_seq_extract_grid(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                         const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
     HVO_CHECK_ARG(s && gray && depth16 && out && nframes >= 1, "bad argument");
     const int nd = (int)s->devices.size();
     const size_t px = (size_t)s->width * s->height;
@@ -131,7 +140,9 @@ int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16
                 const int n = std::min(s->call_frames, count - off);
                 const hvo_frame_outputs o = seq_outputs_at(s, *out, (size_t)(first + off));
                 const hvo_frame_bow_outputs b = bow ? seq_outputs_at(s, *bow, (size_t)(first + off)) : hvo_frame_bow_outputs{};
-                st = hvo_frame_extract_batch_async_bow(h, gray + (size_t)(first + off) * px, depth16 + (size_t)(first + off) * px, n, &o, bow ? &b : nullptr);
+                const hvo_frame_grid_outputs g = grid ? seq_outputs_at(s, *grid, (size_t)(first + off)) : hvo_frame_grid_outputs{};
+                st = hvo_frame_extract_batch_async_grid(h, gray + (size_t)(first + off) * px, depth16 + (size_t)(first + off) * px, n, &o, bow ? &b : nullptr,
+                                                        grid ? &g : nullptr);
             }
             float ms = 0.f;
             const int st2 = hvo_frame_timer_stop(h, &ms);   // waits for every download of this device; reports device-side faults
@@ -147,9 +158,21 @@ int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16
     return HVO_OK;
 }
 
-int hvo_seq_extract(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
-    return hvo_seq_extract_bow(s, gray, depth16, nframes, out, nullptr);
+int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                        const hvo_frame_bow_outputs* bow) {
+    return hvo_seq_extract_grid(s, gray, depth16, nframes, out, bow, nullptr);
 }
+
+int hvo_seq_extract(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out) {
+    return hvo_seq_extract_grid(s, gray, depth16, nframes, out, nullptr, nullptr);
+}
+
+int hvo_seq_image_bounds(const hvo_seq* s, float* min_x, float* max_x, float* min_y, float* max_y) {
+    HVO_CHECK_ARG(s, "null handle");
+    return hvo_frame_image_bounds(s->handles[0], min_x, max_x, min_y, max_y);
+}
+
+int hvo_seq_line_grid_capacity(const hvo_seq* s) { return s ? hvo_frame_line_grid_capacity(s->handles[0]) : 0; }
 
 float hvo_seq_last_ms(const hvo_seq* s) { return s ? s->last_ms : 0.f; }
 

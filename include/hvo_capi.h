@@ -638,6 +638,23 @@ typedef struct hvo_frame_bow_outputs {
     int32_t* word_of;     /* [n][orb_capacity]      word id, or -1 where the word is stopped          optional on the host            */
 } hvo_frame_bow_outputs;
 
+/* The frame grids of a batch of n frames (Frame::AssignFeaturesToGrid / AssignFeaturesToGridForLine, src/Frame.cc:832-872, run by
+ * Frame::Frame right after the extraction): mGrid / mGridForLine [64][48] as per-cell counts plus the cells' indices concatenated in
+ * cell order (cell = ix * 48 + iy), a cell's indices ascending (the reference's push_back order).  The point grid is built on mvKeysUn
+ * (kps_un on an undistorting handle, else kps) with Frame::PosInGrid, the line grid on the keylines the call returns (after cullingLine
+ * when line_cull is set) with the reference's LineIterator walk; both with the handle's image bounds (hvo_frame_image_bounds).
+ * Either pair may be NULL; a pair needs its stage (HVO_STAGE_ORB / HVO_STAGE_LINES), otherwise HVO_ERR_ARG.  uint16 entries: a point
+ * grid needs orb_capacity <= 65535.  Device pointers for hvo_frame_extract_batch_device_grid, which writes no item entry past a frame's
+ * total; host pointers for the host calls, which copy whole rows (entries past the total then hold unspecified values).          */
+typedef struct hvo_frame_grid_outputs {
+    uint16_t* grid_counts;   /* [n][3072]                mGrid[ix][iy].size()                                                          */
+    uint16_t* grid_items;    /* [n][orb_capacity]        keypoint indices, first sum(grid_counts[f]) entries                           */
+    uint16_t* lgrid_counts;  /* [n][3072]                mGridForLine[ix][iy].size()                                                   */
+    uint16_t* lgrid_items;   /* [n][line_grid_capacity]  line indices, first sum(lgrid_counts[f]) entries.  line_grid_capacity =
+                                                         64 * max_lines is exact: LineIterator advances the major axis by one cell per
+                                                         step, so a line visits at most 64 in-grid cells and none twice             */
+} hvo_frame_grid_outputs;
+
 /* Host-side expanders of the compact outputs (plain C loops, no CUDA). */
 /* labels4 [H*W/2] -> labels [H*W] int32 (-1 = none) */
 int hvo_membership4_expand(const uint8_t* labels4, int npixels, int32_t* labels);
@@ -678,6 +695,19 @@ int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const u
                                       const hvo_frame_bow_outputs* bow);
 int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
                                        const hvo_frame_bow_outputs* d_bow);
+/* hvo_frame_extract_batch_bow / _async_bow / _device_bow with grid outputs as well; bow and grid may each be NULL, and grid == NULL is exactly
+ * the call without _grid (it launches nothing more).  On an undistorting handle the device call needs d_out->kps_un for point grids. */
+int hvo_frame_extract_batch_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                 const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid);
+int hvo_frame_extract_batch_async_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                       const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid);
+int hvo_frame_extract_batch_device_grid(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                        const hvo_frame_bow_outputs* d_bow, const hvo_frame_grid_outputs* d_grid);
+/* mnMinX, mnMaxX, mnMinY, mnMaxY the grids are built with (hvo_image_bounds of the handle's camera, computed at create; (0, W, 0, H) when
+ * the handle does not undistort).  Frame sets mfGridElementWidthInv = 64.f / (max_x - min_x), mfGridElementHeightInv = 48.f / (max_y - min_y). */
+int hvo_frame_image_bounds(const hvo_frame* h, float* min_x, float* max_x, float* min_y, float* max_y);
+/* rows per frame of lgrid_items: 64 * max_lines (0 without the line stage) */
+int hvo_frame_line_grid_capacity(const hvo_frame* h);
 int hvo_frame_last_launches(const hvo_frame* h);
 int hvo_frame_sync(hvo_frame* h);
 int hvo_frame_timer_start(hvo_frame* h);
@@ -706,6 +736,12 @@ int hvo_seq_set_vocabulary(hvo_seq* s, int n_nodes, const int32_t* child_start, 
 /* hvo_seq_extract with the BoW outputs of hvo_frame_extract_batch_bow (host arrays of n frames); bow == NULL: hvo_seq_extract. */
 int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
                         const hvo_frame_bow_outputs* bow);
+/* hvo_seq_extract_bow with the grid outputs of hvo_frame_extract_batch_grid (host arrays of n frames); bow / grid may each be NULL. */
+int hvo_seq_extract_grid(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                         const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid);
+/* hvo_frame_image_bounds / hvo_frame_line_grid_capacity of the sequence's handles (the same on every device) */
+int hvo_seq_image_bounds(const hvo_seq* s, float* min_x, float* max_x, float* min_y, float* max_y);
+int hvo_seq_line_grid_capacity(const hvo_seq* s);
 /* device time of the last hvo_seq_extract: CUDA events around each device's share (uploads, kernels, downloads), max over devices */
 float hvo_seq_last_ms(const hvo_seq* s);
 
