@@ -94,6 +94,8 @@ ABI = {
     'hvo_seq_extract_grid': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp]),
     'hvo_seq_image_bounds': (C.c_int, [_vp] + [C.POINTER(C.c_float)] * 4),
     'hvo_seq_line_grid_capacity': (C.c_int, [_vp]),
+    'hvo_seq_extract_lpvo': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp]),
+    'hvo_seq_lpvo_capacity': (C.c_int, [_vp]),
     'hvo_seq_last_ms': (C.c_float, [_vp]),
     'hvo_normals3_expand': (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp]),
     'hvo_orb_level_size': (C.c_int, [_vp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
@@ -223,6 +225,10 @@ ABI = {
     'hvo_frame_extract_batch_device_grid': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp]),
     'hvo_frame_image_bounds': (C.c_int, [_vp] + [C.POINTER(C.c_float)] * 4),
     'hvo_frame_line_grid_capacity': (C.c_int, [_vp]),
+    'hvo_frame_extract_batch_lpvo': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp]),
+    'hvo_frame_extract_batch_async_lpvo': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp]),
+    'hvo_frame_extract_batch_device_lpvo': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp]),
+    'hvo_frame_lpvo_capacity': (C.c_int, [_vp]),
     'hvo_frame_last_launches': (C.c_int, [_vp]),
     'hvo_frame_sync': (C.c_int, [_vp]),
     'hvo_frame_timer_start': (C.c_int, [_vp]),
@@ -1950,18 +1956,30 @@ class _FrameGridOutputs(C.Structure):
     _fields_ = [(n, _vp) for n in ('grid_counts', 'grid_items', 'lgrid_counts', 'lgrid_items')]
 
 
+class _FrameLpvoOutputs(C.Structure):
+    _fields_ = [(n, _vp) for n in ('normals3', 'depth', 'pix2', 'counts')]
+
+
+def _check_lpvo_stage(lpvo, stages):
+    if lpvo and not stages & STAGE_NORMALS:
+        raise HvoError(HVO_ERR_ARG, 'lpvo=True needs the normals stage (STAGE_NORMALS)')
+
+
 class FrameFrontEnd:
     """The extraction part of ORB_SLAM2::Frame::Frame(imGray, imDepth, ...) (reference src/Frame.cc:188-233): ORB + RGB-D
-    depth lookup, LSD/LBD lines, PEAC planes and surface normals of a batch of frames, three concurrent CUDA streams."""
+    depth lookup, LSD/LBD lines, PEAC planes and surface normals (and, on request, the LPVO normals) of a batch of frames, on
+    concurrent CUDA streams."""
     FIELDS = [f[0] for f in _FrameOutputs._fields_]
     BOW_FIELDS = [f[0] for f in _FrameBowOutputs._fields_]
     GRID_FIELDS = [f[0] for f in _FrameGridOutputs._fields_]
+    LPVO_FIELDS = ['lpvo_' + f[0] for f in _FrameLpvoOutputs._fields_]   # output keys; the struct's fields without the prefix
     vocabulary = None
     grids = False
+    with_lpvo = False
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, bf=40.0, nfeatures=1000, scale_factor=1.2, nlevels=8, ini_th=20,
                  min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=16, max_batch=1, device=0, line_cull=False, lanes=0, membership='i32',
-                 distorted=False, normals='n8', dist=None, vocabulary=None, levelsup=4, grids=False):
+                 distorted=False, normals='n8', dist=None, vocabulary=None, levelsup=4, grids=False, lpvo=False):
         """membership: 'i32' (int32 labels, -1 = none), 'u8' (one byte per pixel, 255 = none: what a host caller needs to
         rebuild plane_vertices_), 'both', or 'u4' (host calls only: two pixels per byte, 15 = none, max_planes <= 15; expand with
         membership4_expand).  The int32 image is always the device-side working image.
@@ -1972,8 +1990,11 @@ class FrameFrontEnd:
         vocabulary: the dict ORBVocabulary takes.  Every frame then also gets what Frame::ComputeBoW computes, transform(mDescriptors,
         mBowVec, mFeatVec, levelsup), on the device right after its descriptors: the outputs gain the BoW arrays (see bow()).
         grids: every frame also gets Frame::AssignFeaturesToGrid / AssignFeaturesToGridForLine (mGrid, mGridForLine) with the handle's
-        image_bounds(): the outputs gain grid_counts / grid_items (ORB stage) and lgrid_counts / lgrid_items (line stage), see grid()."""
+        image_bounds(): the outputs gain grid_counts / grid_items (ORB stage) and lgrid_counts / lgrid_items (line stage), see grid().
+        lpvo: every frame also gets Manhattan::computeNormalsLPVO (what Frame::Frame runs while !bManhInit) after its surface normals:
+        the outputs gain lpvo_normals3 / lpvo_depth / lpvo_pix2 / lpvo_counts, see lpvo().  Needs the normals stage."""
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
+        _check_lpvo_stage(lpvo, stages)
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
         prm = self._params(fx, fy, cx, cy, depth_factor, bf, nfeatures, scale_factor, nlevels, ini_th, min_th, n_lines, stages, max_planes,
@@ -1988,6 +2009,7 @@ class FrameFrontEnd:
         _check(lib().hvo_frame_lanes(out, C.byref(a), C.byref(b)))
         self.lanes, self.chunk = a.value, b.value
         self.grids, self.line_grid_capacity = bool(grids), lib().hvo_frame_line_grid_capacity(out)
+        self.with_lpvo, self.lpvo_capacity = bool(lpvo), lib().hvo_frame_lpvo_capacity(out)
         if vocabulary is not None:
             self.set_vocabulary(vocabulary, levelsup)
 
@@ -2062,6 +2084,10 @@ class FrameFrontEnd:
                 sh.update(normals8=((n, self.normals_count, 8), np.float32))
             else:
                 sh.update(normals3=((n, self.normals_count, 3), np.float32))
+            if self.with_lpvo:
+                c = self.lpvo_capacity
+                sh.update(lpvo_normals3=((n, c, 3), np.float64), lpvo_depth=((n, c), np.float32), lpvo_pix2=((n, c, 2), np.int32),
+                          lpvo_counts=((n,), np.int32))
         return sh
 
     @staticmethod
@@ -2110,6 +2136,22 @@ class FrameFrontEnd:
             setattr(o, k, ptrs.get(k))
         return C.byref(o)
 
+    def _lpvo_outputs(self, ptrs):
+        """hvo_frame_lpvo_outputs by reference, or None for a handle created without lpvo."""
+        if not self.with_lpvo:
+            return None
+        o = _FrameLpvoOutputs()
+        for k in self.LPVO_FIELDS:
+            setattr(o, k[5:], ptrs.get(k))
+        return C.byref(o)
+
+    @staticmethod
+    def lpvo(out, f):
+        """Frame f's LPVO normals: (pt_normals [m,3] float64, depth_normals [m] float32, pixels (u, v) [m,2] int32), the form of
+        Manhattan.computeNormalsLPVO."""
+        m = int(out['lpvo_counts'][f])
+        return out['lpvo_normals3'][f, :m].copy(), out['lpvo_depth'][f, :m].copy(), out['lpvo_pix2'][f, :m].copy()
+
     @staticmethod
     def _cells(counts, items, f):
         c = np.asarray(counts[f], np.int32)
@@ -2149,8 +2191,8 @@ class FrameFrontEnd:
             self._check_out(out, self.output_shapes(n, device=False))
         ptrs = {k: v.ctypes.data for k, v in out.items()}
         o = self._outputs(ptrs)
-        f = lib().hvo_frame_extract_batch_grid if wait else lib().hvo_frame_extract_batch_async_grid
-        _check(f(self._h, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs), self._grid_outputs(ptrs)))
+        f = lib().hvo_frame_extract_batch_lpvo if wait else lib().hvo_frame_extract_batch_async_lpvo
+        _check(f(self._h, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs), self._grid_outputs(ptrs), self._lpvo_outputs(ptrs)))
         return out
 
     @staticmethod
@@ -2163,8 +2205,8 @@ class FrameFrontEnd:
     def extract_batch_device(self, d_gray, d_depth16, n, d_ptrs):
         """d_ptrs: name -> device pointer (int) for every output of output_shapes(n).  Asynchronous."""
         o = self._outputs(d_ptrs)
-        _check(lib().hvo_frame_extract_batch_device_grid(self._h, _vp(d_gray), _vp(d_depth16), n, C.byref(o), self._bow_outputs(d_ptrs),
-                                                         self._grid_outputs(d_ptrs)))
+        _check(lib().hvo_frame_extract_batch_device_lpvo(self._h, _vp(d_gray), _vp(d_depth16), n, C.byref(o), self._bow_outputs(d_ptrs),
+                                                         self._grid_outputs(d_ptrs), self._lpvo_outputs(d_ptrs)))
 
     def last_launches(self):
         return lib().hvo_frame_last_launches(self._h)
@@ -2188,8 +2230,9 @@ class FrameSequence(FrameFrontEnd):
 
     def __init__(self, width, height, fx, fy, cx, cy, depth_factor, devices, frames_per_call=2368, bf=40.0, nfeatures=1000, scale_factor=1.2,
                  nlevels=8, ini_th=20, min_th=7, n_lines=200, stages=STAGE_ALL, max_planes=15, line_cull=True, lanes=0, membership='u4',
-                 normals='n3', distorted=False, dist=None, vocabulary=None, levelsup=4, grids=False):
+                 normals='n3', distorted=False, dist=None, vocabulary=None, levelsup=4, grids=False, lpvo=False):
         assert membership in ('i32', 'u8', 'both', 'u4') and normals in ('n8', 'n3')
+        _check_lpvo_stage(lpvo, stages)
         self.membership_mode, self.normals_mode = membership, normals
         self.cam = (float(fx), float(fy), float(cx), float(cy), float(np.float32(depth_factor)))
         prm = self._params(fx, fy, cx, cy, depth_factor, bf, nfeatures, scale_factor, nlevels, ini_th, min_th, n_lines, stages, max_planes,
@@ -2205,6 +2248,7 @@ class FrameSequence(FrameFrontEnd):
         _check(lib().hvo_seq_capacities(out, C.byref(a), C.byref(b), C.byref(c)))
         self.orb_capacity, self.max_lines, self.normals_count = a.value, b.value, c.value
         self.grids, self.line_grid_capacity = bool(grids), lib().hvo_seq_line_grid_capacity(out)
+        self.with_lpvo, self.lpvo_capacity = bool(lpvo), lib().hvo_seq_lpvo_capacity(out)
         if vocabulary is not None:
             self.set_vocabulary(vocabulary, levelsup)
 
@@ -2228,13 +2272,13 @@ class FrameSequence(FrameFrontEnd):
             raise HvoError(HVO_ERR_ARG, f'gray / depth16 must be [n, {self.h}, {self.w}]')
         if out is None:
             out = self.alloc_host(n)
-        else:   # kps_un, the BoW and the grid arrays at least: the other arrays' check is a separate change
+        else:   # kps_un, the BoW, grid and LPVO arrays at least: the other arrays' check is a separate change
             self._check_out(out, {k: v for k, v in self.output_shapes(n, device=False).items()
-                                  if k == 'kps_un' or k in self.BOW_FIELDS or k in self.GRID_FIELDS})
+                                  if k == 'kps_un' or k in self.BOW_FIELDS or k in self.GRID_FIELDS or k in self.LPVO_FIELDS})
         ptrs = {k: v.ctypes.data for k, v in out.items()}
         o = self._outputs(ptrs)
-        _check(lib().hvo_seq_extract_grid(self._seq, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs),
-                                          self._grid_outputs(ptrs)))
+        _check(lib().hvo_seq_extract_lpvo(self._seq, _np_ptr(gray), _np_ptr(depth16), n, C.byref(o), self._bow_outputs(ptrs),
+                                          self._grid_outputs(ptrs), self._lpvo_outputs(ptrs)))
         return out
 
     def last_ms(self):

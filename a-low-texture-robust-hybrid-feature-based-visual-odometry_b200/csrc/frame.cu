@@ -1,13 +1,15 @@
 // Frame-level front-end for sm_100a: the extraction part of Frame::Frame(imGray, imDepth, ...) of the reference
-// (src/Frame.cc:188-233), where three std::threads run ExtractORBNDepth (ORB + ComputeStereoFromRGBD, :874-884),
+// (src/Frame.cc:188-233), where std::threads run ExtractORBNDepth (ORB + ComputeStereoFromRGBD, :874-884),
 // ExtractLSD (LINEextractor::operator(), :895-903) and ComputePlanes (PlaneDetection + surface normals, :2104-2212)
-// on the same frame.  Here the frame (gray + raw 16-bit depth) is uploaded once and the three pipelines run on three
+// on the same frame, plus ExtractMainImgPtNormals (Manhattan::computeNormalsLPVO, :218-228, :1324-1328) while the
+// Manhattan axes are not initialised.  Here the frame (gray + raw 16-bit depth) is uploaded once and the pipelines run on
 // CUDA streams chained by events to a master stream, so a batch of frames is one call and one device-timed region.
 #include <algorithm>
 #include <cstdlib>
 #include <new>
 
 #include "hvo_common.cuh"
+#include "lpvo.cuh"
 
 struct hvo_orb;
 struct hvo_line;
@@ -35,6 +37,10 @@ using namespace hvo;
 enum { ST_ORB = 1, ST_LINE = 2, ST_PLANE = 4, ST_NORMALS = 8 };
 static const int kMaxLanes = 8;
 static const int kGridCells = 64 * 48;   // FRAME_GRID_COLS x FRAME_GRID_ROWS
+// frames per pass of the LPVO chain (rows -> cols -> normals): its scratch is 2.6 MB / frame at 640x480 and 7.8 MB at 1280x720, so a
+// chunk-sized copy would take 10.5 GB at 4096 frames.  Measured on B200 (DESIGN section 4): 16 passes of 256 frames take 34.9 ms per
+// 4096 frames, one pass of 4096 (hvo_lpvo) 29.0 ms; 0.66 GB of scratch is worth the 6 ms on a stage only the first frames ask for.
+static const int kLpvoFrames = 256;
 
 // Device-side capacity faults of the pipelines (ORB quadtree arena, LSD segment buffer, plane refinement queue) are folded,
 // on the pipeline's own stream right after its kernels, into one sticky record per frame handle: fault[0] = lowest frame index
@@ -95,6 +101,7 @@ struct FrameLane {
     hvo_frame_outputs d_out;  // device staging of every output (host API)
     hvo_frame_bow_outputs d_bow{};  // device staging of the BoW outputs (host API; allocated while a vocabulary is attached)
     hvo_frame_grid_outputs d_grid{};  // device staging of the grid outputs (host API; allocated by the first call that asks for grids)
+    hvo_frame_lpvo_outputs d_lpvo{};  // device staging of the LPVO outputs (host API; allocated by the first call that asks for them)
 };
 
 struct hvo_frame {
@@ -115,6 +122,8 @@ struct hvo_frame {
     double* d_bow_weight = nullptr;   // per-row leaf weights of one chunk: shared by the lanes, whose ORB kernels run in order on one stream
     float min_x = 0.f, max_x = 0.f, min_y = 0.f, max_y = 0.f;   // mnMinX .. mnMaxY (Frame::ComputeImageBounds), the grids' bounds
     uint32_t* d_lgrid_bits = nullptr;   // line grid bit rows of one chunk: shared by the lanes, whose line kernels run in order on one stream
+    LpvoGeom lpvo_g{};                  // Manhattan::computeNormalsLPVO's lattice for the handle's camera and image size
+    LpvoScratch lpvo_scratch;           // min(kLpvoFrames, chunk) frames: shared by the lanes, whose normals kernels run in order on one stream
 };
 
 static const int kNoFault = 0x7fffffff;
@@ -154,6 +163,15 @@ static hvo_frame_bow_outputs outputs_at(const hvo_frame* h, const hvo_frame_bow_
     if (o.word_of) r.word_of = o.word_of + off * c;
     return r;
 }
+static hvo_frame_lpvo_outputs outputs_at(const hvo_frame* h, const hvo_frame_lpvo_outputs& o, size_t off) {
+    const size_t c = (size_t)lpvo_capacity(h->lpvo_g);
+    hvo_frame_lpvo_outputs r = o;
+    if (o.normals3) r.normals3 = o.normals3 + off * c * 3;
+    if (o.depth) r.depth = o.depth + off * c;
+    if (o.pix2) r.pix2 = o.pix2 + off * c * 2;
+    if (o.counts) r.counts = o.counts + off;
+    return r;
+}
 static hvo_frame_grid_outputs outputs_at(const hvo_frame* h, const hvo_frame_grid_outputs& o, size_t off) {
     hvo_frame_grid_outputs r = o;
     if (o.grid_counts) r.grid_counts = o.grid_counts + off * kGridCells;
@@ -177,13 +195,15 @@ static hvo_frame_grid_outputs outputs_at(const hvo_frame* h, const hvo_frame_gri
 // bo (device, NULL = no BoW) / host_bo (host, NULL = nothing to download): the BoW kernels follow the ORB kernels on the ORB stream; their
 // downloads are the first of phase 2.  go / host_go likewise for the grids (a NULL pair = no such grid): the point grid follows the
 // undistortion on the ORB stream, the line grid the line kernels on the line stream; each is downloaded with its pipeline's results.
+// lo / host_lo likewise for the LPVO normals: their chain follows the surface normals on the normals stream (so it sits beside the ordered
+// pipelines side by side, and runs last in the serial schedule) and is downloaded with them.
 // HVO_FRAME_SERIAL=0 / 1 forces one schedule (tuning aid).  Also measured for 1024-frame chunks and rejected: planes || lines first and
 // ORB || normals afterwards (87 instead of 65-79 ms), a third priority level that puts planes above lines (no change).
 static const int kSerialFrames = 2048;
 static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_t start_depth, const uint8_t* d_gray, const uint16_t* d_depth, int n,
                        int base, const hvo_frame_outputs& o, const hvo_frame_outputs* host, const hvo_frame_bow_outputs* bo,
-                       const hvo_frame_bow_outputs* host_bo, const hvo_frame_grid_outputs* go, const hvo_frame_grid_outputs* host_go, int* launches,
-                       FrameLane* after = nullptr) {
+                       const hvo_frame_bow_outputs* host_bo, const hvo_frame_grid_outputs* go, const hvo_frame_grid_outputs* host_go,
+                       const hvo_frame_lpvo_outputs* lo, const hvo_frame_lpvo_outputs* host_lo, int* launches, FrameLane* after = nullptr) {
     const size_t N = (size_t)n, px = (size_t)h->width * h->height;
     static const int serial_env = [] { const char* e = getenv("HVO_FRAME_SERIAL"); return e ? atoi(e) : -1; }();
     const bool serial = serial_env >= 0 ? serial_env == 1 : n >= kSerialFrames;
@@ -274,6 +294,10 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
             k_pack_normals3<<<(int)std::min<long long>((rows + 255) / 256, 148 * 16), 256, 0, s>>>(o.normals8, o.normals3, rows);
             ++*launches;
         }
+        if (lo) {
+            st = lpvo_launch(s, h->lpvo_g, h->lpvo_scratch, d_depth, n, lo->normals3, lo->depth, lo->pix2, lo->counts, launches);
+            if (st != HVO_OK) return st;
+        }
         HVO_CUDA(cudaEventRecord(L.cdone[3], s));
         prev_done = L.cdone[3];
     }
@@ -352,6 +376,13 @@ static int lane_launch(hvo_frame* h, FrameLane& L, cudaEvent_t start, cudaEvent_
         if (int ds = down_stream(3, normals_stream(L.normals), &s)) return ds;
         if (host && host->normals8) HVO_CUDA(cudaMemcpyAsync(host->normals8, o.normals8, N * (size_t)h->normals_count * 32, cudaMemcpyDeviceToHost, s));
         if (host && host->normals3) HVO_CUDA(cudaMemcpyAsync(host->normals3, o.normals3, N * (size_t)h->normals_count * 12, cudaMemcpyDeviceToHost, s));
+        if (host && host_lo) {
+            const size_t c = (size_t)lpvo_capacity(h->lpvo_g);
+            HVO_CUDA(cudaMemcpyAsync(host_lo->counts, lo->counts, N * 4, cudaMemcpyDeviceToHost, s));
+            HVO_CUDA(cudaMemcpyAsync(host_lo->normals3, lo->normals3, N * c * 24, cudaMemcpyDeviceToHost, s));
+            HVO_CUDA(cudaMemcpyAsync(host_lo->depth, lo->depth, N * c * 4, cudaMemcpyDeviceToHost, s));
+            if (host_lo->pix2) HVO_CUDA(cudaMemcpyAsync(host_lo->pix2, lo->pix2, N * c * 8, cudaMemcpyDeviceToHost, s));
+        }
         timeline_mark(s, "end_normals");
         HVO_CUDA(cudaEventRecord(L.join[3], s));
     }
@@ -470,6 +501,7 @@ int hvo_frame_create(const hvo_frame_params* p, int width, int height, int max_b
     h->orb_cap = L0.orb ? hvo_orb_capacity(L0.orb) : 0;
     h->max_lines = L0.line ? hvo_line_max_lines(L0.line) : 0;
     h->normals_count = L0.normals ? hvo_normals_count(L0.normals) : 0;
+    h->lpvo_g = lpvo_geom(hvo_plane_params{p->fx, p->fy, p->cx, p->cy, p->depth_factor}, width, height);
     // Frame::ComputeImageBounds; a handle that does not undistort has the reference's k1 == 0 bounds
     h->max_x = (float)width; h->max_y = (float)height;
     if (h->undistort) st = hvo_image_bounds(&h->cam, width, height, &h->min_x, &h->max_x, &h->min_y, &h->max_y);
@@ -566,7 +598,8 @@ void hvo_frame_destroy(hvo_frame* h) {
         void* bufs[] = {L.d_gray, L.d_depth, o.kps, o.desc, o.kp_counts, o.kp_depth, o.kp_uright, o.keylines, o.line_desc, o.linevec3,
                         o.line_counts, o.n_planes, o.planes7, o.membership, o.membership8, o.normals8, o.membership4, o.normals3, o.kps_un};
         for (void* b : bufs) if (b) cudaFree(b);
-        void* gbufs[] = {L.d_grid.grid_counts, L.d_grid.grid_items, L.d_grid.lgrid_counts, L.d_grid.lgrid_items};
+        void* gbufs[] = {L.d_grid.grid_counts, L.d_grid.grid_items, L.d_grid.lgrid_counts, L.d_grid.lgrid_items,
+                         L.d_lpvo.normals3, L.d_lpvo.depth, L.d_lpvo.pix2, L.d_lpvo.counts};
         for (void* b : gbufs) if (b) cudaFree(b);
         if (L.fork) cudaEventDestroy(L.fork);
         for (auto& e : L.join) if (e) cudaEventDestroy(e);
@@ -575,6 +608,7 @@ void hvo_frame_destroy(hvo_frame* h) {
     }
     if (h->d_fault) cudaFree(h->d_fault);
     if (h->d_lgrid_bits) cudaFree(h->d_lgrid_bits);
+    lpvo_scratch_free(&h->lpvo_scratch);
     if (h->h_fault) cudaFreeHost(h->h_fault);
     if (h->fork) cudaEventDestroy(h->fork);
     for (auto& e : h->tev) if (e) cudaEventDestroy(e);
@@ -636,6 +670,32 @@ static int frame_check_grid_outputs(const hvo_frame* h, const hvo_frame_grid_out
     return HVO_OK;
 }
 
+static int frame_check_lpvo_outputs(const hvo_frame* h, const hvo_frame_lpvo_outputs* l, bool device) {
+    if (!l) return HVO_OK;
+    HVO_CHECK_ARG(h->p.stages & ST_NORMALS, "LPVO outputs need the normals stage");
+    HVO_CHECK_ARG(l->normals3 && l->depth && l->counts, "LPVO normals3 / depth / counts missing");
+    if (device) HVO_CHECK_ARG(l->pix2, "device LPVO outputs: every array is required");
+    return HVO_OK;
+}
+
+// Allocated by the first call that asks for LPVO outputs, kept until destroy: the chain's scratch (kLpvoFrames frames, shared by the
+// lanes) and, for the host calls, every lane's device staging of the four arrays.
+static int frame_reserve_lpvo(hvo_frame* h, bool host) {
+    if (!h->lpvo_scratch.frames) {
+        const int st = lpvo_scratch_alloc(h->lpvo_g, std::min(kLpvoFrames, h->lane[0].cap), &h->lpvo_scratch);
+        if (st != HVO_OK) { lpvo_scratch_free(&h->lpvo_scratch); return st; }
+    }
+    const size_t B = (size_t)h->lane[0].cap, c = (size_t)lpvo_capacity(h->lpvo_g);
+    for (int li = 0; host && li < h->nlanes; ++li) {
+        hvo_frame_lpvo_outputs& o = h->lane[li].d_lpvo;
+        if (!o.normals3) HVO_CUDA(cudaMalloc(&o.normals3, B * c * 24));
+        if (!o.depth) HVO_CUDA(cudaMalloc(&o.depth, B * c * 4));
+        if (!o.pix2) HVO_CUDA(cudaMalloc(&o.pix2, B * c * 8));
+        if (!o.counts) HVO_CUDA(cudaMalloc(&o.counts, B * 4));
+    }
+    return HVO_OK;
+}
+
 // Allocated by the first call that asks for a grid, kept until destroy: the line grid's bit rows (one chunk, shared by the lanes) and, for
 // the host calls, every lane's device staging of the requested grids.
 static int frame_reserve_grids(hvo_frame* h, const hvo_frame_grid_outputs* g, bool host) {
@@ -690,18 +750,20 @@ int hvo_frame_set_vocabulary(hvo_frame* h, int n_nodes, const int32_t* child_sta
     return HVO_OK;
 }
 
-int hvo_frame_extract_batch_device_grid(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
-                                        const hvo_frame_bow_outputs* d_bow, const hvo_frame_grid_outputs* d_grid) {
+int hvo_frame_extract_batch_device_lpvo(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                        const hvo_frame_bow_outputs* d_bow, const hvo_frame_grid_outputs* d_grid, const hvo_frame_lpvo_outputs* d_lpvo) {
     HVO_CHECK_ARG(h && d_gray && d_depth16, "null argument");
     HVO_CHECK_ARG(nframes >= 1 && nframes <= h->max_batch, "nframes out of range for this handle");
     int st = frame_check_outputs(h, d_out, true);
     if (st == HVO_OK) st = frame_check_bow_outputs(h, d_bow, true);
     if (st == HVO_OK) st = frame_check_grid_outputs(h, d_grid, d_out, true);
+    if (st == HVO_OK) st = frame_check_lpvo_outputs(h, d_lpvo, true);
     if (st != HVO_OK) return st;
     if (h->p.stages & ST_ORB) HVO_CHECK_ARG(d_out->kp_depth && d_out->kp_uright, "kp_depth / kp_uright missing");
     if (h->p.stages & ST_LINE) HVO_CHECK_ARG(d_out->linevec3, "linevec3 missing");
     HVO_CUDA(cudaSetDevice(h->device));
     if (d_grid && (st = frame_reserve_grids(h, d_grid, false)) != HVO_OK) return st;
+    if (d_lpvo && (st = frame_reserve_lpvo(h, false)) != HVO_OK) return st;
     const size_t px = (size_t)h->width * h->height;
     HVO_CUDA(cudaEventRecord(h->fork, h->stream));
     int launches = 0, used = 0;
@@ -716,8 +778,10 @@ int hvo_frame_extract_batch_device_grid(hvo_frame* h, const uint8_t* d_gray, con
         const int n = std::min(per, nframes - off);
         const hvo_frame_bow_outputs bo = d_bow ? outputs_at(h, *d_bow, (size_t)off) : hvo_frame_bow_outputs{};
         const hvo_frame_grid_outputs go = d_grid ? outputs_at(h, *d_grid, (size_t)off) : hvo_frame_grid_outputs{};
+        const hvo_frame_lpvo_outputs lo = d_lpvo ? outputs_at(h, *d_lpvo, (size_t)off) : hvo_frame_lpvo_outputs{};
         st = lane_launch(h, L, h->fork, nullptr, d_gray + (size_t)off * px, d_depth16 + (size_t)off * px, n, off, outputs_at(h, *d_out, (size_t)off), nullptr,
-                         d_bow ? &bo : nullptr, nullptr, d_grid ? &go : nullptr, nullptr, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
+                         d_bow ? &bo : nullptr, nullptr, d_grid ? &go : nullptr, nullptr, d_lpvo ? &lo : nullptr, nullptr, &launches,
+                         h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
         if (st != HVO_OK) return st;
         h->last_lane = used;
     }
@@ -729,6 +793,11 @@ int hvo_frame_extract_batch_device_grid(hvo_frame* h, const uint8_t* d_gray, con
     return HVO_OK;
 }
 
+int hvo_frame_extract_batch_device_grid(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                        const hvo_frame_bow_outputs* d_bow, const hvo_frame_grid_outputs* d_grid) {
+    return hvo_frame_extract_batch_device_lpvo(h, d_gray, d_depth16, nframes, d_out, d_bow, d_grid, nullptr);
+}
+
 int hvo_frame_extract_batch_device_bow(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
                                        const hvo_frame_bow_outputs* d_bow) {
     return hvo_frame_extract_batch_device_grid(h, d_gray, d_depth16, nframes, d_out, d_bow, nullptr);
@@ -738,16 +807,18 @@ int hvo_frame_extract_batch_device(hvo_frame* h, const uint8_t* d_gray, const ui
     return hvo_frame_extract_batch_device_grid(h, d_gray, d_depth16, nframes, d_out, nullptr, nullptr);
 }
 
-int hvo_frame_extract_batch_async_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
-                                       const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
+int hvo_frame_extract_batch_async_lpvo(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                       const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid, const hvo_frame_lpvo_outputs* lpvo) {
     HVO_CHECK_ARG(h && gray && depth16, "null argument");
     HVO_CHECK_ARG(nframes >= 1, "nframes < 1");
     int st = frame_check_outputs(h, out, false);
     if (st == HVO_OK) st = frame_check_bow_outputs(h, bow, false);
     if (st == HVO_OK) st = frame_check_grid_outputs(h, grid, out, false);
+    if (st == HVO_OK) st = frame_check_lpvo_outputs(h, lpvo, false);
     if (st != HVO_OK) return st;
     HVO_CUDA(cudaSetDevice(h->device));
     if (grid && (st = frame_reserve_grids(h, grid, true)) != HVO_OK) return st;
+    if (lpvo && (st = frame_reserve_lpvo(h, true)) != HVO_OK) return st;
     const size_t px = (size_t)h->width * h->height;
     // chunks: as few as the lane capacity allows, of equal size.  Chunks go round-robin through the lanes ACROSS calls
     // (next_lane), so that the upload of a one-chunk call overlaps the kernels of the previous call on the other lane.
@@ -780,8 +851,10 @@ int hvo_frame_extract_batch_async_grid(hvo_frame* h, const uint8_t* gray, const 
         const hvo_frame_outputs hostk = outputs_at(h, *out, (size_t)off);
         const hvo_frame_bow_outputs hostb = bow ? outputs_at(h, *bow, (size_t)off) : hvo_frame_bow_outputs{};
         const hvo_frame_grid_outputs hostg = grid ? outputs_at(h, *grid, (size_t)off) : hvo_frame_grid_outputs{};
+        const hvo_frame_lpvo_outputs hostl = lpvo ? outputs_at(h, *lpvo, (size_t)off) : hvo_frame_lpvo_outputs{};
         st = lane_launch(h, L, L.fork, L.fork_depth, L.d_gray, L.d_depth, n, off, d, &hostk, bow ? &L.d_bow : nullptr, bow ? &hostb : nullptr,
-                         grid ? &dg : nullptr, grid ? &hostg : nullptr, &launches, h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
+                         grid ? &dg : nullptr, grid ? &hostg : nullptr, lpvo ? &L.d_lpvo : nullptr, lpvo ? &hostl : nullptr, &launches,
+                         h->last_lane >= 0 ? &h->lane[h->last_lane] : nullptr);
         if (st != HVO_OK) return st;
         h->last_lane = li;
     }
@@ -794,6 +867,11 @@ int hvo_frame_extract_batch_async_grid(hvo_frame* h, const uint8_t* gray, const 
     return HVO_OK;
 }
 
+int hvo_frame_extract_batch_async_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                       const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
+    return hvo_frame_extract_batch_async_lpvo(h, gray, depth16, nframes, out, bow, grid, nullptr);
+}
+
 int hvo_frame_extract_batch_async_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
                                       const hvo_frame_bow_outputs* bow) {
     return hvo_frame_extract_batch_async_grid(h, gray, depth16, nframes, out, bow, nullptr);
@@ -803,12 +881,17 @@ int hvo_frame_extract_batch_async(hvo_frame* h, const uint8_t* gray, const uint1
     return hvo_frame_extract_batch_async_grid(h, gray, depth16, nframes, out, nullptr, nullptr);
 }
 
-int hvo_frame_extract_batch_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
-                                 const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
-    const int st = hvo_frame_extract_batch_async_grid(h, gray, depth16, nframes, out, bow, grid);
+int hvo_frame_extract_batch_lpvo(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                 const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid, const hvo_frame_lpvo_outputs* lpvo) {
+    const int st = hvo_frame_extract_batch_async_lpvo(h, gray, depth16, nframes, out, bow, grid, lpvo);
     if (st != HVO_OK) return st;
     HVO_CUDA(cudaStreamSynchronize(h->stream));
     return frame_check_fault(h);
+}
+
+int hvo_frame_extract_batch_grid(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                 const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
+    return hvo_frame_extract_batch_lpvo(h, gray, depth16, nframes, out, bow, grid, nullptr);
 }
 
 int hvo_frame_extract_batch_bow(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
@@ -827,6 +910,8 @@ int hvo_frame_image_bounds(const hvo_frame* h, float* min_x, float* max_x, float
 }
 
 int hvo_frame_line_grid_capacity(const hvo_frame* h) { return h ? 64 * h->max_lines : 0; }
+
+int hvo_frame_lpvo_capacity(const hvo_frame* h) { return h && (h->p.stages & ST_NORMALS) ? lpvo_capacity(h->lpvo_g) : 0; }
 
 int hvo_frame_last_launches(const hvo_frame* h) { return h ? h->last_launches : 0; }
 int hvo_frame_sync(hvo_frame* h) {

@@ -3,25 +3,21 @@
 //
 // The reference builds a vertex map, six tangent maps and a mask, takes seven full cv::integral images (CV_32F -> CV_64F)
 // and then reads them at a 15-px lattice only.  Here nothing is materialised per pixel: a thread walks one image row with
-// seven running double sums (cv::integral's own row order) and keeps them at the 84 lattice columns; a second kernel adds
-// the rows up per column (cv::integral's column order) and keeps the 64 lattice rows; a third takes the box means, the
+// seven running double sums (cv::integral's own row order) and keeps them at the lattice columns (84 at 640 px); a second
+// kernel adds the rows up per column (cv::integral's column order) and keeps the lattice rows; a third takes the box means, the
 // cross product and cv::normalize, and compacts the valid samples in the reference's push_back order.  The additions
 // happen in cv::integral's order, so the sums are the same doubles.
 //
 // Reference bug, not reproduced: the live caller passes the raw CV_16U depth Mat and the function reads it as float
 // (SURVEY section 8, row D6).  This implements the intended float-depth behaviour: z = (float)raw * depth_factor.
+#include <algorithm>
 #include <new>
 
-#include "hvo_common.cuh"
+#include "lpvo.cuh"
 
 namespace hvo {
 
 static const int kCell = 10, kDensity = 15;
-
-struct LpvoGeom {
-    int W, H, nsu, nsv;  // lattice: u = 10 + 15 j (j < nsu), v = 10 + 15 i (i < nsv)
-    float cx, cy, inv_fx, inv_fy, factor;
-};
 
 __device__ __forceinline__ bool lpvo_bad(float z) { return z < 0.2f || z > 7.0f; }
 __device__ __forceinline__ float3 lpvo_vertex(const LpvoGeom& g, int u, int v, float z) {
@@ -69,9 +65,11 @@ __global__ void __launch_bounds__(64) k_lpvo_rows(const uint16_t* __restrict__ d
     }
 }
 
-// integ[f][k][r][c]: integral image at lattice row r (r even: v = 15 i, r odd: v = 15 i + 10) and lattice column c
-__global__ void __launch_bounds__(96) k_lpvo_cols(LpvoGeom g, const double* __restrict__ rowsum, double* __restrict__ integ) {
-    const int k = blockIdx.x, f = blockIdx.y, c = threadIdx.x;
+// integ[f][k][r][c]: integral image at lattice row r (r even: v = 15 i, r odd: v = 15 i + 10) and lattice column c.
+// One thread per lattice column, as many CTAs across as the width needs (170 columns at 1280 px).
+static const int kColsBlock = 96;
+__global__ void __launch_bounds__(kColsBlock) k_lpvo_cols(LpvoGeom g, const double* __restrict__ rowsum, double* __restrict__ integ) {
+    const int c = blockIdx.x * kColsBlock + threadIdx.x, k = blockIdx.y, f = blockIdx.z;
     const int ncs = 2 * g.nsu, nrs = 2 * g.nsv, H = g.H;
     if (c >= ncs) return;
     const double* in = rowsum + ((size_t)f * 7 + k) * H * ncs + c;
@@ -152,6 +150,46 @@ __global__ void __launch_bounds__(256) k_lpvo_normals(const uint16_t* __restrict
     if (tid == 0) counts[f] = s_base;
 }
 
+LpvoGeom lpvo_geom(const hvo_plane_params& cam, int width, int height) {
+    LpvoGeom g;
+    g.W = width; g.H = height;
+    g.nsu = (width - 1 - kCell + kDensity - 1) / kDensity;   // u = 10; u < W - 1; u += 15
+    g.nsv = (height - 1 - kCell + kDensity - 1) / kDensity;
+    g.cx = cam.cx; g.cy = cam.cy; g.inv_fx = 1.0f / cam.fx; g.inv_fy = 1.0f / cam.fy; g.factor = cam.depth_factor;
+    return g;
+}
+
+static size_t lpvo_rowsum_bytes(const LpvoGeom& g, int frames) { return (size_t)frames * 7 * g.H * 2 * g.nsu * sizeof(double); }
+static size_t lpvo_integ_bytes(const LpvoGeom& g, int frames) { return (size_t)frames * 7 * 2 * g.nsv * 2 * g.nsu * sizeof(double); }
+
+int lpvo_scratch_alloc(const LpvoGeom& g, int frames, LpvoScratch* s) {
+    HVO_CUDA(cudaMalloc(&s->rowsum, lpvo_rowsum_bytes(g, frames)));
+    HVO_CUDA(cudaMalloc(&s->integ, lpvo_integ_bytes(g, frames)));
+    s->frames = frames;
+    return HVO_OK;
+}
+
+void lpvo_scratch_free(LpvoScratch* s) {
+    if (s->rowsum) cudaFree(s->rowsum);
+    if (s->integ) cudaFree(s->integ);
+    *s = LpvoScratch{};
+}
+
+int lpvo_launch(cudaStream_t s, const LpvoGeom& g, const LpvoScratch& sc, const uint16_t* d_depth, int n, double* d_normals3, float* d_z,
+                int32_t* d_pix2, int32_t* d_counts, int* launches) {
+    const size_t px = (size_t)g.W * g.H, cap = (size_t)lpvo_capacity(g);
+    for (int off = 0; off < n; off += sc.frames) {   // sub-batches: the scratch holds sc.frames frames
+        const int m = std::min(sc.frames, n - off);
+        const uint16_t* D = d_depth + off * px;
+        k_lpvo_rows<<<dim3(div_up(g.H, 64), m), 64, 0, s>>>(D, g, sc.rowsum);
+        k_lpvo_cols<<<dim3(div_up(2 * g.nsu, kColsBlock), 7, m), kColsBlock, 0, s>>>(g, sc.rowsum, sc.integ);
+        k_lpvo_normals<<<m, 256, 0, s>>>(D, g, sc.integ, d_normals3 + off * cap * 3, d_z + off * cap, d_pix2 + off * cap * 2, d_counts + off);
+        HVO_CUDA(cudaGetLastError());
+        *launches += 3;
+    }
+    return HVO_OK;
+}
+
 }  // namespace hvo
 
 using namespace hvo;
@@ -159,21 +197,18 @@ using namespace hvo;
 struct hvo_lpvo {
     int device = 0, max_batch = 0, cap = 0;
     LpvoGeom g;
+    LpvoScratch scratch;   // max_batch frames: one pass of the chain per call
     cudaStream_t stream = nullptr;
     cudaEvent_t tev[2] = {nullptr, nullptr};
     uint16_t* d_depth = nullptr;
-    double *d_rowsum = nullptr, *d_integ = nullptr, *d_normals = nullptr;
+    double* d_normals = nullptr;
     float* d_z = nullptr;
     int32_t *d_pix = nullptr, *d_counts = nullptr;
 };
 
-static int lpvo_launch(hvo_lpvo* h, const uint16_t* d_depth, int n, double* d_normals3, float* d_z, int32_t* d_pix2, int32_t* d_counts) {
-    const LpvoGeom& g = h->g;
-    k_lpvo_rows<<<dim3(div_up(g.H, 64), n), 64, 0, h->stream>>>(d_depth, g, h->d_rowsum);
-    k_lpvo_cols<<<dim3(7, n), 96, 0, h->stream>>>(g, h->d_rowsum, h->d_integ);
-    k_lpvo_normals<<<n, 256, 0, h->stream>>>(d_depth, g, h->d_integ, d_normals3, d_z, d_pix2, d_counts);
-    HVO_CUDA(cudaGetLastError());
-    return HVO_OK;
+static int lpvo_run(hvo_lpvo* h, const uint16_t* d_depth, int n, double* d_normals3, float* d_z, int32_t* d_pix2, int32_t* d_counts) {
+    int launches = 0;
+    return lpvo_launch(h->stream, h->g, h->scratch, d_depth, n, d_normals3, d_z, d_pix2, d_counts, &launches);
 }
 
 extern "C" {
@@ -191,13 +226,8 @@ int hvo_lpvo_create(const hvo_plane_params* cam, int width, int height, int max_
     hvo_lpvo* h = new (std::nothrow) hvo_lpvo();
     if (!h) { set_error("out of host memory"); return HVO_ERR_ARG; }
     h->device = device; h->max_batch = max_batch;
-    LpvoGeom& g = h->g;
-    g.W = width; g.H = height;
-    g.nsu = (width - 1 - kCell + kDensity - 1) / kDensity;   // u = 10; u < W - 1; u += 15
-    g.nsv = (height - 1 - kCell + kDensity - 1) / kDensity;
-    g.cx = cam->cx; g.cy = cam->cy; g.inv_fx = 1.0f / cam->fx; g.inv_fy = 1.0f / cam->fy; g.factor = cam->depth_factor;
-    h->cap = g.nsu * g.nsv;
-    HVO_CHECK_ARG(2 * g.nsu <= 96, "image too wide for the column kernel (max 730 px)");
+    h->g = lpvo_geom(*cam, width, height);
+    h->cap = lpvo_capacity(h->g);
     int st = HVO_OK;
     do {
 #define HVO_TRY(call) if ((call) != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(cudaGetLastError())); st = HVO_ERR_CUDA; break; }
@@ -207,8 +237,7 @@ int hvo_lpvo_create(const hvo_plane_params* cam, int width, int height, int max_
         HVO_TRY(cudaEventCreate(&h->tev[1]));
         const size_t B = (size_t)max_batch, px = (size_t)width * height;
         HVO_TRY(cudaMalloc(&h->d_depth, B * px * 2));
-        HVO_TRY(cudaMalloc(&h->d_rowsum, B * 7 * height * 2 * g.nsu * sizeof(double)));
-        HVO_TRY(cudaMalloc(&h->d_integ, B * 7 * 2 * g.nsv * 2 * g.nsu * sizeof(double)));
+        if ((st = lpvo_scratch_alloc(h->g, max_batch, &h->scratch)) != HVO_OK) break;
         HVO_TRY(cudaMalloc(&h->d_normals, B * h->cap * 3 * sizeof(double)));
         HVO_TRY(cudaMalloc(&h->d_z, B * h->cap * sizeof(float)));
         HVO_TRY(cudaMalloc(&h->d_pix, B * h->cap * 2 * sizeof(int32_t)));
@@ -224,8 +253,9 @@ void hvo_lpvo_destroy(hvo_lpvo* h) {
     if (!h) return;
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    void* bufs[] = {h->d_depth, h->d_rowsum, h->d_integ, h->d_normals, h->d_z, h->d_pix, h->d_counts};
+    void* bufs[] = {h->d_depth, h->d_normals, h->d_z, h->d_pix, h->d_counts};
     for (void* b : bufs) if (b) cudaFree(b);
+    lpvo_scratch_free(&h->scratch);
     for (auto& e : h->tev) if (e) cudaEventDestroy(e);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -238,7 +268,7 @@ int hvo_lpvo_compute_batch_device(hvo_lpvo* h, const uint16_t* d_depth16, int nf
     HVO_CHECK_ARG(h && d_depth16 && d_normals3 && d_depth && d_pix2 && d_counts, "null argument");
     HVO_CHECK_ARG(nframes >= 1 && nframes <= h->max_batch, "nframes out of range for this handle");
     HVO_CUDA(cudaSetDevice(h->device));
-    return lpvo_launch(h, d_depth16, nframes, d_normals3, d_depth, d_pix2, d_counts);
+    return lpvo_run(h, d_depth16, nframes, d_normals3, d_depth, d_pix2, d_counts);
 }
 
 int hvo_lpvo_compute_batch(hvo_lpvo* h, const uint16_t* depth16, int nframes, double* normals3, float* depth, int32_t* pix2, int32_t* counts) {
@@ -247,7 +277,7 @@ int hvo_lpvo_compute_batch(hvo_lpvo* h, const uint16_t* depth16, int nframes, do
     HVO_CUDA(cudaSetDevice(h->device));
     const size_t n = (size_t)nframes, px = (size_t)h->g.W * h->g.H, c = (size_t)h->cap;
     HVO_CUDA(cudaMemcpyAsync(h->d_depth, depth16, n * px * 2, cudaMemcpyHostToDevice, h->stream));
-    int st = lpvo_launch(h, h->d_depth, nframes, h->d_normals, h->d_z, h->d_pix, h->d_counts);
+    int st = lpvo_run(h, h->d_depth, nframes, h->d_normals, h->d_z, h->d_pix, h->d_counts);
     if (st != HVO_OK) return st;
     HVO_CUDA(cudaMemcpyAsync(normals3, h->d_normals, n * c * 24, cudaMemcpyDeviceToHost, h->stream));
     HVO_CUDA(cudaMemcpyAsync(depth, h->d_z, n * c * 4, cudaMemcpyDeviceToHost, h->stream));

@@ -17,7 +17,7 @@ struct hvo_seq {
     std::vector<hvo_frame*> handles;
     int width = 0, height = 0, call_frames = 0;
     hvo_frame_params p;
-    int orb_cap = 0, max_lines = 0, normals_count = 0;
+    int orb_cap = 0, max_lines = 0, normals_count = 0, lpvo_cap = 0;
     float last_ms = 0.f;                 // slowest device of the last call (CUDA events on its master stream)
     std::vector<float> dev_ms;
 };
@@ -66,6 +66,16 @@ static hvo_frame_grid_outputs seq_outputs_at(const hvo_seq* s, const hvo_frame_g
     return r;
 }
 
+static hvo_frame_lpvo_outputs seq_outputs_at(const hvo_seq* s, const hvo_frame_lpvo_outputs& o, size_t off) {
+    const size_t c = (size_t)s->lpvo_cap;
+    hvo_frame_lpvo_outputs r = o;
+    if (o.normals3) r.normals3 = o.normals3 + off * c * 3;
+    if (o.depth) r.depth = o.depth + off * c;
+    if (o.pix2) r.pix2 = o.pix2 + off * c * 2;
+    if (o.counts) r.counts = o.counts + off;
+    return r;
+}
+
 extern "C" {
 
 int hvo_seq_create(const hvo_frame_params* p, int width, int height, const int* devices, int ndevices, int frames_per_call, hvo_seq** out) {
@@ -83,6 +93,7 @@ int hvo_seq_create(const hvo_frame_params* p, int width, int height, const int* 
         if (st != HVO_OK) { hvo_seq_destroy(s); return st; }
     }
     hvo_frame_capacities(s->handles[0], &s->orb_cap, &s->max_lines, &s->normals_count);
+    s->lpvo_cap = hvo_frame_lpvo_capacity(s->handles[0]);
     *out = s;
     return HVO_OK;
 }
@@ -120,8 +131,8 @@ int hvo_seq_set_vocabulary(hvo_seq* s, int n_nodes, const int32_t* child_start, 
     return HVO_OK;
 }
 
-int hvo_seq_extract_grid(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
-                         const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
+int hvo_seq_extract_lpvo(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                         const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid, const hvo_frame_lpvo_outputs* lpvo) {
     HVO_CHECK_ARG(s && gray && depth16 && out && nframes >= 1, "bad argument");
     const int nd = (int)s->devices.size();
     const size_t px = (size_t)s->width * s->height;
@@ -141,8 +152,9 @@ int hvo_seq_extract_grid(hvo_seq* s, const uint8_t* gray, const uint16_t* depth1
                 const hvo_frame_outputs o = seq_outputs_at(s, *out, (size_t)(first + off));
                 const hvo_frame_bow_outputs b = bow ? seq_outputs_at(s, *bow, (size_t)(first + off)) : hvo_frame_bow_outputs{};
                 const hvo_frame_grid_outputs g = grid ? seq_outputs_at(s, *grid, (size_t)(first + off)) : hvo_frame_grid_outputs{};
-                st = hvo_frame_extract_batch_async_grid(h, gray + (size_t)(first + off) * px, depth16 + (size_t)(first + off) * px, n, &o, bow ? &b : nullptr,
-                                                        grid ? &g : nullptr);
+                const hvo_frame_lpvo_outputs l = lpvo ? seq_outputs_at(s, *lpvo, (size_t)(first + off)) : hvo_frame_lpvo_outputs{};
+                st = hvo_frame_extract_batch_async_lpvo(h, gray + (size_t)(first + off) * px, depth16 + (size_t)(first + off) * px, n, &o, bow ? &b : nullptr,
+                                                        grid ? &g : nullptr, lpvo ? &l : nullptr);
             }
             float ms = 0.f;
             const int st2 = hvo_frame_timer_stop(h, &ms);   // waits for every download of this device; reports device-side faults
@@ -156,6 +168,11 @@ int hvo_seq_extract_grid(hvo_seq* s, const uint8_t* gray, const uint16_t* depth1
     for (int d = 0; d < nd; ++d)
         if (status[d] != HVO_OK) { set_error("device %d: %s", s->devices[d], errors[d].c_str()); return status[d]; }
     return HVO_OK;
+}
+
+int hvo_seq_extract_grid(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                         const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid) {
+    return hvo_seq_extract_lpvo(s, gray, depth16, nframes, out, bow, grid, nullptr);
 }
 
 int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
@@ -173,6 +190,8 @@ int hvo_seq_image_bounds(const hvo_seq* s, float* min_x, float* max_x, float* mi
 }
 
 int hvo_seq_line_grid_capacity(const hvo_seq* s) { return s ? hvo_frame_line_grid_capacity(s->handles[0]) : 0; }
+
+int hvo_seq_lpvo_capacity(const hvo_seq* s) { return s ? s->lpvo_cap : 0; }
 
 float hvo_seq_last_ms(const hvo_seq* s) { return s ? s->last_ms : 0.f; }
 

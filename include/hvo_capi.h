@@ -550,7 +550,8 @@ int hvo_lproj_last_launches(const hvo_lproj* h);
  * differences where 0.2 <= z <= 7, seven cv::integral images, 10x10 box means every 15 px from (10, 10), normal = v x u,
  * cv::normalize.  Outputs per frame, in the reference's push_back order: pt_normals (3 doubles each), depth_normals
  * (float) and the pixel (u, v) of each sample.  Input is the raw 16-bit depth; z = (float)raw * depth_factor (the
- * reference's live caller passes the 16-bit Mat where a float Mat is read: that bug is not reproduced). */
+ * reference's live caller passes the 16-bit Mat where a float Mat is read: that bug is not reproduced).  Any image size in
+ * 32..8192 px.  A frame handle returns the same rows from its own call (hvo_frame_lpvo_outputs). */
 typedef struct hvo_lpvo hvo_lpvo;
 int hvo_lpvo_create(const hvo_plane_params* cam, int width, int height, int max_batch, int device, hvo_lpvo** out);
 void hvo_lpvo_destroy(hvo_lpvo* h);
@@ -567,8 +568,10 @@ int hvo_lpvo_timer_stop(hvo_lpvo* h, float* ms_out);
 /* ---------------------------------------------------------------------------------------------- FRAME
  * The extraction part of Frame::Frame(imGray, imDepth, timeStamp, extractors, ...) (src/Frame.cc:188-233): the reference
  * runs three std::threads on one frame — ExtractORBNDepth (:874-884), ExtractLSD (:895-903), ComputePlanes
- * (:2104-2212).  hvo_frame uploads the frame (gray + raw 16-bit depth) once and runs the same three pipelines on three
- * CUDA streams, for a batch of frames per call.                                                               */
+ * (:2104-2212) — and, while the Manhattan axes are not initialised (!bManhInit, :218-228), a fourth, ExtractMainImgPtNormals
+ * (Manhattan::computeNormalsLPVO, :1324-1328).  hvo_frame uploads the frame (gray + raw 16-bit depth) once and runs the same
+ * pipelines on CUDA streams, for a batch of frames per call; the LPVO normals run, after the surface normals on the normals
+ * stream, in the calls given hvo_frame_lpvo_outputs (*_lpvo).                                                 */
 
 #define HVO_STAGE_ORB 1
 #define HVO_STAGE_LINES 2
@@ -655,6 +658,18 @@ typedef struct hvo_frame_grid_outputs {
                                                          step, so a line visits at most 64 in-grid cells and none twice             */
 } hvo_frame_grid_outputs;
 
+/* Manhattan::computeNormalsLPVO of a batch of n frames (src/Frame.cc:218-228, run by Frame::Frame while !bManhInit), on the frame's raw
+ * depth: the rows hvo_lpvo_compute_batch returns for the same depth, bit for bit.  Rows per frame: hvo_frame_lpvo_capacity() (=
+ * hvo_lpvo_capacity for the same camera and image size); frame f's first counts[f] rows are valid, in the reference's push_back order.
+ * Needs HVO_STAGE_NORMALS, otherwise HVO_ERR_ARG.  Host pointers for the host calls, which copy whole rows; device pointers for
+ * hvo_frame_extract_batch_device_lpvo, which needs every array and writes no row at or past a frame's count.                  */
+typedef struct hvo_frame_lpvo_outputs {
+    double* normals3;  /* [n][lpvo_capacity][3]   pt_normals (unit normal v x u)                                                   */
+    float* depth;      /* [n][lpvo_capacity]      depth_normals                                                                    */
+    int32_t* pix2;     /* [n][lpvo_capacity][2]   the sample's pixel (u, v)                                 optional on the host    */
+    int32_t* counts;   /* [n]                     samples of the frame                                                             */
+} hvo_frame_lpvo_outputs;
+
 /* Host-side expanders of the compact outputs (plain C loops, no CUDA). */
 /* labels4 [H*W/2] -> labels [H*W] int32 (-1 = none) */
 int hvo_membership4_expand(const uint8_t* labels4, int npixels, int32_t* labels);
@@ -703,6 +718,18 @@ int hvo_frame_extract_batch_async_grid(hvo_frame* h, const uint8_t* gray, const 
                                        const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid);
 int hvo_frame_extract_batch_device_grid(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
                                         const hvo_frame_bow_outputs* d_bow, const hvo_frame_grid_outputs* d_grid);
+/* hvo_frame_extract_batch_grid / _async_grid / _device_grid with LPVO outputs as well; bow, grid and lpvo may each be NULL, and lpvo == NULL
+ * is exactly the call without _lpvo (it launches nothing more).  Every frame of a call given lpvo gets its LPVO rows: a tracker asks for
+ * them in the calls of the frames it constructs while !bManhInit.  The chain runs over passes of at most 256 frames on scratch that the
+ * first such call allocates (2.6 MB per frame of a pass at 640x480, 7.8 MB at 1280x720). */
+int hvo_frame_extract_batch_lpvo(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                 const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid, const hvo_frame_lpvo_outputs* lpvo);
+int hvo_frame_extract_batch_async_lpvo(hvo_frame* h, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                                       const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid, const hvo_frame_lpvo_outputs* lpvo);
+int hvo_frame_extract_batch_device_lpvo(hvo_frame* h, const uint8_t* d_gray, const uint16_t* d_depth16, int nframes, const hvo_frame_outputs* d_out,
+                                        const hvo_frame_bow_outputs* d_bow, const hvo_frame_grid_outputs* d_grid, const hvo_frame_lpvo_outputs* d_lpvo);
+/* rows per frame of hvo_frame_lpvo_outputs: the LPVO lattice size, ceil((W - 11) / 15) * ceil((H - 11) / 15) (0 without the normals stage) */
+int hvo_frame_lpvo_capacity(const hvo_frame* h);
 /* mnMinX, mnMaxX, mnMinY, mnMaxY the grids are built with (hvo_image_bounds of the handle's camera, computed at create; (0, W, 0, H) when
  * the handle does not undistort).  Frame sets mfGridElementWidthInv = 64.f / (max_x - min_x), mfGridElementHeightInv = 48.f / (max_y - min_y). */
 int hvo_frame_image_bounds(const hvo_frame* h, float* min_x, float* max_x, float* min_y, float* max_y);
@@ -739,9 +766,13 @@ int hvo_seq_extract_bow(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16
 /* hvo_seq_extract_bow with the grid outputs of hvo_frame_extract_batch_grid (host arrays of n frames); bow / grid may each be NULL. */
 int hvo_seq_extract_grid(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
                          const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid);
-/* hvo_frame_image_bounds / hvo_frame_line_grid_capacity of the sequence's handles (the same on every device) */
+/* hvo_seq_extract_grid with the LPVO outputs of hvo_frame_extract_batch_lpvo (host arrays of n frames); bow / grid / lpvo may each be NULL. */
+int hvo_seq_extract_lpvo(hvo_seq* s, const uint8_t* gray, const uint16_t* depth16, int nframes, const hvo_frame_outputs* out,
+                         const hvo_frame_bow_outputs* bow, const hvo_frame_grid_outputs* grid, const hvo_frame_lpvo_outputs* lpvo);
+/* hvo_frame_image_bounds / hvo_frame_line_grid_capacity / hvo_frame_lpvo_capacity of the sequence's handles (the same on every device) */
 int hvo_seq_image_bounds(const hvo_seq* s, float* min_x, float* max_x, float* min_y, float* max_y);
 int hvo_seq_line_grid_capacity(const hvo_seq* s);
+int hvo_seq_lpvo_capacity(const hvo_seq* s);
 /* device time of the last hvo_seq_extract: CUDA events around each device's share (uploads, kernels, downloads), max over devices */
 float hvo_seq_last_ms(const hvo_seq* s);
 
