@@ -45,9 +45,13 @@ __global__ void k_sn_cloud(const uint16_t* __restrict__ depth, SnGeom g, float* 
 }
 
 // SAT layout: [f][ch+1][cw+1][6] doubles (dx.xyz, dy.xyz)
+// The table adds the terms (float differences widened to double) in another order than PCL's recurrence (up + left - up-left
+// + term).  A double sum of floats is exact only while the bits of all its terms fit in 53 places; terms of very different
+// exponents (a difference of 1e-9 next to one of 10) round, and then the order can change the last bit of a window sum.  Depth
+// images keep the terms within that range: tests/test_normals_reference.py requires the oracle's bits on every scene, shape
+// and parameter set it runs.
 // One warp per SAT row: 32 cloud columns at a time, lane <-> column.  Every lane forms its six central differences, the
-// warp adds them up with a shuffle scan (the terms are float differences widened to double, whose partial sums are exact in
-// double, so the association does not matter) and each lane stores its six doubles next to its neighbours' (48 B per lane,
+// warp adds them up with a shuffle scan and each lane stores its six doubles next to its neighbours' (48 B per lane,
 // 1.5 KB contiguous per warp).  Round 1 had one thread per row writing 48-byte records 10 KB apart (2.4 ms per 1184 frames).
 __global__ void __launch_bounds__(128) k_sn_rowscan(const float* __restrict__ pts, SnGeom g, double* __restrict__ sat) {
     const int r = blockIdx.x * 4 + (threadIdx.x >> 5), f = blockIdx.y, lane = threadIdx.x & 31;
@@ -283,11 +287,22 @@ int hvo_normals_create(const hvo_normals_params* p, int width, int height, int m
     HVO_CHECK_ARG(p && out, "null argument");
     *out = nullptr;
     HVO_CHECK_ARG(width >= 64 && height >= 64 && max_batch >= 1, "size out of range");
+    HVO_CHECK_ARG(max_batch <= 65535, "max_batch > 65535 (the frame index is a grid y / z coordinate)");
     HVO_CHECK_ARG(p->fx != 0.f && p->fy != 0.f, "focal length is zero");
     int ndev = 0;
     HVO_CUDA(cudaGetDeviceCount(&ndev));
     if (ndev < 1) { set_error("no CUDA device: libhvofront has no CPU fallback"); return HVO_ERR_CUDA; }
     HVO_CHECK_ARG(device >= 0 && device < ndev, "device index out of range");
+    // k_sn_chamfer keeps 3 cloud rows of each of its kChamferFrames frames in shared memory: 96 * ceil(width / 3) bytes
+    const int cw = (int)std::ceil(width / 3.0);
+    const size_t chamfer_smem = (size_t)kChamferFrames * 3 * cw * sizeof(float);
+    int smem_optin = 0;
+    HVO_CUDA(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+    if (chamfer_smem > (size_t)smem_optin) {
+        set_error("bad argument: width %d needs %zu B of shared memory per chamfer block, the device allows %d B (width <= %d)", width,
+                  chamfer_smem, smem_optin, 3 * (smem_optin / (int)(kChamferFrames * 3 * sizeof(float))));
+        return HVO_ERR_ARG;
+    }
     hvo_normals* h = new (std::nothrow) hvo_normals();
     if (!h) { set_error("out of host memory"); return HVO_ERR_ARG; }
     h->device = device; h->max_batch = max_batch;
@@ -299,6 +314,9 @@ int hvo_normals_create(const hvo_normals_params* p, int width, int height, int m
     const size_t B = (size_t)max_batch, np = (size_t)g.cw * g.ch;
     cudaError_t e = cudaSetDevice(device);
     pin_carveout(k_sn_cloud); pin_carveout(k_sn_rowscan); pin_carveout(k_sn_colscan); pin_carveout(k_sn_chamfer); pin_carveout(k_sn_normals);
+    // widths over 1536 need more than the default 48 KB; the limit is the device's (one value for every handle, so handles of
+    // different widths cannot lower it for each other), each launch asks for what its width needs
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_sn_chamfer, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
     if (e == cudaSuccess) e = create_stream(&h->stream);
     if (e == cudaSuccess) e = cudaEventCreate(&h->tev[0]);
     if (e == cudaSuccess) e = cudaEventCreate(&h->tev[1]);
