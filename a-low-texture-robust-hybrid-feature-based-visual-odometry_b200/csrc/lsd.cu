@@ -549,9 +549,12 @@ __device__ __forceinline__ float lsd_length(const float e[4]) {
     return (float)sqrt(a * a + b * b);
 }
 
+// Idx = uint16_t: the sorted index list and the ranks live in shared memory (seg_cap <= 65535, 4 bytes per possible segment).
+// Idx = uint32_t: they live in `scratch` ([B][2 seg_cap] in global memory), for images whose segment bound exceeds either limit.
+template <class Idx>
 __global__ void __launch_bounds__(256) k_line_keylines(const float* __restrict__ seg, int seg_cap, const int* __restrict__ nseg, int W, int H,
                                                        int nfeat, int max_lines, float* __restrict__ resp, KeyLineOut* __restrict__ kls,
-                                                       double* __restrict__ linevec, int32_t* __restrict__ counts) {
+                                                       double* __restrict__ linevec, int32_t* __restrict__ counts, uint32_t* __restrict__ scratch) {
     const int f = blockIdx.x, tid = threadIdx.x;
     const int n = min(nseg[f], seg_cap);
     const float* S = seg + (long long)f * seg_cap * 4;
@@ -571,21 +574,23 @@ __global__ void __launch_bounds__(256) k_line_keylines(const float* __restrict__
     // sort_lines_by_response (LineExtractor.cpp:351-360) is an unstable std::sort.  Without equal responses the result is the
     // plain descending rank (computed in parallel); with ties the order is libstdc++'s, replayed by one thread (std_sort.cuh).
     extern __shared__ uint16_t kl_sm[];   // [seg_cap] sorted index list, then [seg_cap] rank of every input line
-    uint16_t* sidx = kl_sm;
-    uint16_t* srank = kl_sm + seg_cap;
+    Idx* sidx;
+    if constexpr (sizeof(Idx) == 2) sidx = kl_sm;
+    else sidx = scratch + (long long)f * seg_cap * 2;
+    Idx* srank = sidx + seg_cap;
     if (select) {
         int tie = 0;
         for (int i = tid; i < n; i += 256) {
             const float r = R[i];
             int rank = 0;
             for (int j = 0; j < n; ++j) { const float q = R[j]; rank += (q > r || (q == r && j < i)) ? 1 : 0; tie |= (q == r && j != i) ? 1 : 0; }
-            srank[i] = (uint16_t)rank;
-            sidx[i] = (uint16_t)i;
+            srank[i] = (Idx)rank;
+            sidx[i] = (Idx)i;
         }
         if (__syncthreads_or(tie)) {
-            if (tid == 0) stdsort::sort(sidx, n, [R](uint16_t a, uint16_t b) { return R[a] > R[b]; });
+            if (tid == 0) stdsort::sort(sidx, n, [R](Idx a, Idx b) { return R[a] > R[b]; });
             __syncthreads();
-            for (int k = tid; k < n; k += 256) srank[sidx[k]] = (uint16_t)k;
+            for (int k = tid; k < n; k += 256) srank[sidx[k]] = (Idx)k;
             __syncthreads();
         }
     }
@@ -902,6 +907,7 @@ struct hvo_line {
     bool cull = false;               // run Frame::cullingLine after the extractor (hvo_line_set_culling)
     CullLine* d_cull = nullptr;      // [B][nfeat]
     float* d_newline = nullptr;      // [B][nfeat][5]
+    uint32_t* d_klscratch = nullptr; // [B][2 seg_cap]: k_line_keylines<uint32_t>'s index and rank lists (null: the uint16_t kernel)
     int last_launches = 0;
 };
 
@@ -972,9 +978,15 @@ static int line_extract_device(hvo_line* h, const uint8_t* d_gray, int nframes, 
                                int32_t* d_counts) {
     int st = line_detect_device(h, d_gray, nframes);
     if (st != HVO_OK) return st;
-    timeline_mark(h->stream, "k_line_keylines");
-    k_line_keylines<<<nframes, 256, (size_t)h->seg_cap * 4, h->stream>>>(h->d_seg, h->seg_cap, h->d_nseg, h->width, h->height, h->nfeat, h->nfeat, h->d_resp,
-                                                    d_kl, d_linevec, d_counts);
+    if (h->d_klscratch) {
+        timeline_mark(h->stream, "k_line_keylines<uint32_t>");
+        k_line_keylines<uint32_t><<<nframes, 256, 0, h->stream>>>(h->d_seg, h->seg_cap, h->d_nseg, h->width, h->height, h->nfeat, h->nfeat, h->d_resp,
+                                                                d_kl, d_linevec, d_counts, h->d_klscratch);
+    } else {
+        timeline_mark(h->stream, "k_line_keylines");
+        k_line_keylines<uint16_t><<<nframes, 256, (size_t)h->seg_cap * 4, h->stream>>>(h->d_seg, h->seg_cap, h->d_nseg, h->width, h->height, h->nfeat, h->nfeat,
+                                                                                h->d_resp, d_kl, d_linevec, d_counts, nullptr);
+    }
     HVO_CUDA(cudaGetLastError());
     if (h->cull) {
         // the reference computes LBD twice (LineExtractor.cpp:361-363, Frame.cc:1094-1096) and discards the first result;
@@ -1047,7 +1059,8 @@ int hvo_line_create(const hvo_line_params* p, int width, int height, int max_bat
     do {
 #define HVO_TRY(call) if ((call) != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(cudaGetLastError())); st = HVO_ERR_CUDA; break; }
         HVO_TRY(cudaSetDevice(device));
-        pin_carveout(k_lsd_prep); pin_carveout(k_lsd_order); pin_carveout(k_lsd_grow); pin_carveout(k_line_keylines); pin_carveout(k_line_cull);
+        pin_carveout(k_lsd_prep); pin_carveout(k_lsd_order); pin_carveout(k_lsd_grow); pin_carveout(k_line_keylines<uint16_t>); pin_carveout(k_line_keylines<uint32_t>);
+        pin_carveout(k_line_cull);
         HVO_TRY(create_stream(&h->stream));
         for (auto& e : h->tev) HVO_TRY(cudaEventCreate(&e));
         if (st != HVO_OK) break;
@@ -1078,12 +1091,14 @@ int hvo_line_create(const hvo_line_params* p, int width, int height, int max_bat
         HVO_TRY(cudaMemcpy(h->d_cy, cy.data(), cy.size() * sizeof(LinCoef), cudaMemcpyHostToDevice));
         HVO_TRY(cudaMemcpy(h->d_cstab, tab.data(), tab.size() * sizeof(float2), cudaMemcpyHostToDevice));
         HVO_TRY(cudaFuncSetAttribute(k_lsd_order, cudaFuncAttributeMaxDynamicSharedMemorySize, kOrdWarps * kBins * (int)sizeof(uint32_t)));
-        {   // k_line_keylines keeps two u16 per possible segment; the attribute is per function: only ever raise it
+        {   // k_line_keylines<uint16_t> keeps two u16 per possible segment in shared memory; the attribute is per function: only ever
+            // raise it.  Beyond 65535 segments or 200 KB, k_line_keylines<uint32_t> keeps two u32 per possible segment in global memory.
             static size_t s_kl_smem_max[64] = {0};
             const size_t want = std::max<size_t>((size_t)h->seg_cap * 4, 48 * 1024);
-            if (want > 200 * 1024 || h->seg_cap > 65535) { set_error("image too large for the KeyLine kernel"); st = HVO_ERR_ARG; break; }
-            if (device < 64 && want > s_kl_smem_max[device]) {
-                HVO_TRY(cudaFuncSetAttribute(k_line_keylines, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)want));
+            if (want > 200 * 1024 || h->seg_cap > 65535) {
+                HVO_TRY(cudaMalloc(&h->d_klscratch, B * (size_t)h->seg_cap * 2 * sizeof(uint32_t)));
+            } else if (device < 64 && want > s_kl_smem_max[device]) {
+                HVO_TRY(cudaFuncSetAttribute(k_line_keylines<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)want));
                 s_kl_smem_max[device] = want;
             }
         }
@@ -1101,7 +1116,7 @@ void hvo_line_destroy(hvo_line* h) {
     if (h->stream) cudaStreamSynchronize(h->stream);
     if (h->lbd) hvo_lbd_destroy(h->lbd);
     void* bufs[] = {h->d_gray, h->d_cx, h->d_cy, h->d_cstab, h->d_pix, h->d_scaled, h->d_maxsq, h->d_order, h->d_reg, h->d_used, h->d_norder,
-                    h->d_nseg, h->d_seg, h->d_resp, h->d_kl, h->d_linevec, h->d_counts, h->d_desc, h->d_cull, h->d_newline};
+                    h->d_nseg, h->d_seg, h->d_resp, h->d_kl, h->d_linevec, h->d_counts, h->d_desc, h->d_cull, h->d_newline, h->d_klscratch};
     for (void* b : bufs) if (b) cudaFree(b);
     for (auto& e : h->tev) if (e) cudaEventDestroy(e);
     for (auto& e : h->sev) if (e) cudaEventDestroy(e);

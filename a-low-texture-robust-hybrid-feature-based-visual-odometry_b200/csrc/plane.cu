@@ -174,6 +174,9 @@ struct __align__(16) NodeG { double s[9]; double center[3]; double normal[3]; in
 #endif
 static const int kMinSupport = 3000, kAhcThreads = 128;
 static const int kRowW = 9;  // neighbour-matrix row words per lane: up to 9 * 32 * 32 = 9216 blocks (1280x720)
+// beyond that: up to 24 * 32 * 32 = 24576 blocks (1920x1200).  Node ids, keys (< 2 Nb + max_ext), union-log halves and the
+// disjoint set stay below 2^16 there, and a heap entry keeps 15 id bits + 17 key bits.
+static const int kRowWL = 24;
 #define AHC_TH_MERGE 0.50000000000000011   /* cos(pi/180*60) as computed by std::cos */
 #define AHC_TH_REFINE 0.86602540378443871  /* cos(pi/180*30) */
 
@@ -523,7 +526,7 @@ __device__ void ahc_cluster(const AhcArgs& A, AhcS& S, NodeG* nodes, uint32_t* a
         }
         __syncwarp();
         // the next node to be popped is known now (heap top): pull its neighbour row and its record towards L1 while
-        // lane 0 runs the next pop's sift loop
+        // lane 0 runs the next pop's sift loop (one 128-byte line per lane covers rows of up to 1024 words, kRowWL uses 768)
         if (S.ctl[0] > 0) {
             const int q = (int)(S.heap[0] & S.idmask);
             const char* rq = (const char*)(adj + (size_t)q * nw);
@@ -749,6 +752,9 @@ __global__ void __launch_bounds__(32, HVO_AHC_MINBLOCKS) k_plane_cluster(AhcArgs
 #ifndef HVO_FLOOD_THREADS
 #define HVO_FLOOD_THREADS 256
 #endif
+// a refinement queue entry is pixel | plane << kQPixBits: 22 pixel bits (1920x1200 = 2.3 M pixels), 10 plane bits (max_ext <= 821)
+static const int kQPixBits = 22;
+static const uint32_t kQPixMask = (1u << kQPixBits) - 1u;
 // visits per step = 4 * threads; a visit's rank inside the step takes kFloodPosBits bits of the tournament word, 4 buckets per visit
 static const int kFloodThreads = HVO_FLOOD_THREADS;
 static const int kFloodPosBits = kFloodThreads == 128 ? 9 : (kFloodThreads == 256 ? 10 : (kFloodThreads == 512 ? 11 : 12));
@@ -832,10 +838,10 @@ __global__ void __launch_bounds__(kFloodThreads, HVO_FLOOD_MINBLOCKS) k_plane_fl
             int pos = tail + pre - c;
             if (c && pos + c <= A.qcap) {
                 if (me < 0) {
-                    if (c0) { const uint32_t u = (uint32_t)blkmap[b - Nw] << 20; const int sp = (i * 10 - 1) * W + j * 10; for (int k = 1; k < 10; ++k) queue[pos++] = (uint32_t)(sp + k) | u; }
-                    if (c1) { const uint32_t l = (uint32_t)blkmap[b - 1] << 20; const int sp = (i * 10) * W + j * 10 - 1; for (int k = 0; k < 9; ++k) queue[pos++] = (uint32_t)(sp + k * W) | l; }
+                    if (c0) { const uint32_t u = (uint32_t)blkmap[b - Nw] << kQPixBits; const int sp = (i * 10 - 1) * W + j * 10; for (int k = 1; k < 10; ++k) queue[pos++] = (uint32_t)(sp + k) | u; }
+                    if (c1) { const uint32_t l = (uint32_t)blkmap[b - 1] << kQPixBits; const int sp = (i * 10) * W + j * 10 - 1; for (int k = 0; k < 9; ++k) queue[pos++] = (uint32_t)(sp + k * W) | l; }
                 } else {
-                    const uint32_t u = (uint32_t)me << 20;
+                    const uint32_t u = (uint32_t)me << kQPixBits;
                     const int sp = (i * 10) * W + j * 10;
                     if (c0) for (int k = 0; k < 9; ++k) queue[pos++] = (uint32_t)(sp + k) | u;
                     if (c1) for (int k = 1; k < 10; ++k) queue[pos++] = (uint32_t)(sp + k * W) | u;
@@ -865,14 +871,14 @@ __global__ void __launch_bounds__(kFloodThreads, HVO_FLOOD_MINBLOCKS) k_plane_fl
         const uint32_t q = have ? (have_next ? q_next : queue[head + tid]) : 0u;
         have_next = head + nbat + tid < tail;
         if (have_next) q_next = queue[head + nbat + tid];
-        const int plid = (int)(q >> 20);
+        const int plid = (int)(q >> kQPixBits);
         int cI[4], trail0[4];
         int cxs[4] = {0, 0, 0, 0}, cys[4] = {0, 0, 0, 0};
         uint16_t z16[4] = {0, 0, 0, 0};
         float cdist[4];
         unsigned okm = 0, pend = 0, pushm = 0;  // bit d: visit d passes the plane test / is pending / pushes a new seed
         if (have) {
-            const int sIdx = (int)(q & 0xfffffu);
+            const int sIdx = (int)(q & kQPixMask);
             const int sy = sIdx / W, sx = sIdx - sy * W;
             // valid4 order: left, right, up, down
             cI[0] = sx > 0 ? sIdx - 1 : -1;
@@ -978,7 +984,7 @@ __global__ void __launch_bounds__(kFloodThreads, HVO_FLOOD_MINBLOCKS) k_plane_fl
             int pos = tail + base + pre - mine;
 #pragma unroll
             for (int d = 0; d < 4; ++d)
-                if (pushm & (1u << d)) { if (pos < A.qcap) queue[pos] = (uint32_t)cI[d] | ((uint32_t)plid << 20); ++pos; }
+                if (pushm & (1u << d)) { if (pos < A.qcap) queue[pos] = (uint32_t)cI[d] | ((uint32_t)plid << kQPixBits); ++pos; }
         }
         __syncthreads();
         if (tid == 0) {
@@ -1132,7 +1138,7 @@ int hvo_plane_create(const hvo_plane_params* p, int width, int height, int max_b
     *out = nullptr;
     HVO_CHECK_ARG(p, "null params");
     HVO_CHECK_ARG(width >= 20 && height >= 20 && width <= 8192 && height <= 8192, "image size out of range");
-    HVO_CHECK_ARG((long long)width * height < (1 << 20), "image too large for the 20-bit pixel index of the refinement queue");
+    HVO_CHECK_ARG((long long)width * height <= (1 << kQPixBits), "image too large for the 22-bit pixel index of the refinement queue");
     HVO_CHECK_ARG(max_batch >= 1, "max_batch < 1");
     HVO_CHECK_ARG(p->fx != 0 && p->fy != 0, "fx / fy must be non-zero");
     int ndev = 0;
@@ -1144,12 +1150,12 @@ int hvo_plane_create(const hvo_plane_params* p, int width, int height, int max_b
     h->device = device; h->width = width; h->height = height; h->max_batch = max_batch;
     h->Nw = width / 10; h->Nh = height / 10;
     const int Nb = h->Nw * h->Nh;
-    HVO_CHECK_ARG(Nb <= kRowW * 1024, "too many 10x10 blocks (max 9216, i.e. 1280x720)");
+    if (Nb > kRowWL * 1024) { delete h; set_error("bad argument: too many 10x10 blocks (max 24576, e.g. 1920x1200)"); return HVO_ERR_ARG; }
     h->nw = (Nb + 31) / 32;
     h->qcap = 2 * width * height;
     // test aid: a smaller refinement queue, to provoke HVO_ERR_OVERFLOW
     if (const char* e = getenv("HVO_DEBUG_PLANE_QCAP")) h->qcap = std::max(64, std::min(h->qcap, atoi(e)));
-    h->max_ext = Nb * 100 / kMinSupport + 2;
+    h->max_ext = Nb * 100 / kMinSupport + 2;   // <= 821 < 2^(32 - kQPixBits)
     h->cam.factor = (double)p->depth_factor; h->cam.fx = (double)p->fx; h->cam.fy = (double)p->fy;
     h->cam.rfx = 1.0 / h->cam.fx; h->cam.rfy = 1.0 / h->cam.fy;
     h->cam.cx = (double)p->cx; h->cam.cy = (double)p->cy;
@@ -1160,14 +1166,25 @@ int hvo_plane_create(const hvo_plane_params* p, int width, int height, int max_b
 #define HVO_TRY(call) if ((call) != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(cudaGetLastError())); st = HVO_ERR_CUDA; break; }
         HVO_TRY(cudaSetDevice(device));
         if (h->ahc_smem > 220 * 1024) { set_error("image too large: the plane graph does not fit shared memory"); st = HVO_ERR_ARG; break; }
-        HVO_TRY(cudaFuncSetAttribute(k_plane_cluster<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->ahc_smem));
-        HVO_TRY(cudaFuncSetAttribute(k_plane_cluster<kRowW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->ahc_smem));
-        HVO_TRY(cudaFuncSetAttribute(k_plane_merge<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->merge_smem));
-        HVO_TRY(cudaFuncSetAttribute(k_plane_merge<kRowW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->merge_smem));
         h->flood_smem = (size_t)h->max_ext * 64 + (size_t)Nb * 2 + (size_t)h->max_ext * 2 + 16;
-        HVO_TRY(cudaFuncSetAttribute(k_plane_flood, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->flood_smem));
+        // the attribute is per function (shared by all handles on the device, whatever their image size): only ever raise it, or a
+        // smaller handle created later would make the larger one's launches fail
+        static size_t s_smem_max[64][3] = {};
+        size_t sm[3] = {h->ahc_smem, h->merge_smem, h->flood_smem};
+        if (device < 64)
+            for (int k = 0; k < 3; ++k) sm[k] = std::max(s_smem_max[device][k], sm[k]);
+        HVO_TRY(cudaFuncSetAttribute(k_plane_cluster<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm[0]));
+        HVO_TRY(cudaFuncSetAttribute(k_plane_cluster<kRowW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm[0]));
+        HVO_TRY(cudaFuncSetAttribute(k_plane_cluster<kRowWL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm[0]));
+        HVO_TRY(cudaFuncSetAttribute(k_plane_merge<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm[1]));
+        HVO_TRY(cudaFuncSetAttribute(k_plane_merge<kRowW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm[1]));
+        HVO_TRY(cudaFuncSetAttribute(k_plane_merge<kRowWL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm[1]));
+        HVO_TRY(cudaFuncSetAttribute(k_plane_flood, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm[2]));
+        if (device < 64)   // recorded once every attribute holds it
+            for (int k = 0; k < 3; ++k) s_smem_max[device][k] = sm[k];
         pin_carveout(k_plane_blocks); pin_carveout(k_plane_cluster<3>); pin_carveout(k_plane_cluster<kRowW>);
         pin_carveout(k_plane_flood); pin_carveout(k_plane_merge<3>); pin_carveout(k_plane_merge<kRowW>);
+        pin_carveout(k_plane_cluster<kRowWL>); pin_carveout(k_plane_merge<kRowWL>);
         HVO_TRY(create_stream(&h->stream));
         HVO_TRY(cudaEventCreate(&h->tev[0]));
         HVO_TRY(cudaEventCreate(&h->tev[1]));
@@ -1243,15 +1260,18 @@ static int plane_detect_launch(hvo_plane* h, const uint16_t* d_depth, int nframe
     A.th_refine = std::cos(M_PI / 180.0 * 30.0);  // ParamSet::similarityTh_refine
     A.g_mse = h->d_gmse; A.g_ds = h->d_gds; A.g_nouse = h->d_gnouse; A.g_blkmap = h->d_gblkmap; A.g_ext = h->d_gext;
     A.g_isvalid = h->d_gisvalid; A.g_pl = h->d_gpl; A.g_ctl = h->d_gctl;
-    const bool small = h->nw <= 3 * 32;  // row words per lane: 3 up to 3072 blocks (640x480), kRowW beyond
-    timeline_mark(h->stream, "k_plane_cluster");
-    if (small) k_plane_cluster<3><<<nframes, 32, h->ahc_smem, h->stream>>>(A);
-    else k_plane_cluster<kRowW><<<nframes, 32, h->ahc_smem, h->stream>>>(A);
+    // row words per lane: 3 up to 3072 blocks (640x480), kRowW up to 9216 (1280x720), kRowWL beyond
+    const int rw = h->nw <= 3 * 32 ? 3 : (h->nw <= kRowW * 32 ? kRowW : kRowWL);
+    timeline_mark(h->stream, rw == kRowWL ? "k_plane_cluster<24>" : "k_plane_cluster");
+    if (rw == 3) k_plane_cluster<3><<<nframes, 32, h->ahc_smem, h->stream>>>(A);
+    else if (rw == kRowW) k_plane_cluster<kRowW><<<nframes, 32, h->ahc_smem, h->stream>>>(A);
+    else k_plane_cluster<kRowWL><<<nframes, 32, h->ahc_smem, h->stream>>>(A);
     timeline_mark(h->stream, "k_plane_flood");
     k_plane_flood<<<nframes, kFloodThreads, h->flood_smem, h->stream>>>(A);
-    timeline_mark(h->stream, "k_plane_merge");
-    if (small) k_plane_merge<3><<<nframes, kAhcThreads, h->merge_smem, h->stream>>>(A);
-    else k_plane_merge<kRowW><<<nframes, kAhcThreads, h->merge_smem, h->stream>>>(A);
+    timeline_mark(h->stream, rw == kRowWL ? "k_plane_merge<24>" : "k_plane_merge");
+    if (rw == 3) k_plane_merge<3><<<nframes, kAhcThreads, h->merge_smem, h->stream>>>(A);
+    else if (rw == kRowW) k_plane_merge<kRowW><<<nframes, kAhcThreads, h->merge_smem, h->stream>>>(A);
+    else k_plane_merge<kRowWL><<<nframes, kAhcThreads, h->merge_smem, h->stream>>>(A);
     timeline_mark(h->stream, "k_plane_relabel");
     k_plane_relabel<<<dim3(div_up(div_up(h->width * h->height, 4), 256), nframes), 256, 0, h->stream>>>(A);
     HVO_CUDA(cudaGetLastError());

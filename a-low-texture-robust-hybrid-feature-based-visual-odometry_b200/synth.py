@@ -3,6 +3,8 @@
 S1  TUM-fr3-shaped, textured 640x480 (TUM3.yaml intrinsics, depth factor 5000)
 S2  ICL-NUIM-shaped, low texture 640x480 (ICL.yaml intrinsics, fy < 0)
 S3  RealSense-shaped 1280x720, 2000 ORB
+S6  1080p-colour-shaped 1920x1080 (depth aligned to a 1080p colour stream), 3000 ORB
+S7  wide-FOV-depth-shaped 1024x1024 (Azure-Kinect-class WFOV depth mode), 2000 ORB
 S4  matching stress descriptors (2000 x 50 000 ORB, 200 x 5 000 LBD)
 
 Every frame is a ray-cast box room (floor, ceiling, two side walls, back wall) seen from a camera on a
@@ -15,6 +17,8 @@ CONFIGS = {
     'S1': dict(w=640, h=480, fx=535.4, fy=539.2, cx=320.1, cy=247.6, factor=5000.0, bf=40.0, textured=True, nfeatures=1000),
     'S2': dict(w=640, h=480, fx=481.2, fy=-480.0, cx=319.5, cy=239.5, factor=5000.0, bf=40.0, textured=False, nfeatures=1000),
     'S3': dict(w=1280, h=720, fx=910.0, fy=910.0, cx=640.0, cy=360.0, factor=1000.0, bf=45.0, textured=True, nfeatures=2000),
+    'S6': dict(w=1920, h=1080, fx=1380.0, fy=1380.0, cx=959.5, cy=539.5, factor=1000.0, bf=69.0, textured=True, nfeatures=3000),
+    'S7': dict(w=1024, h=1024, fx=504.0, fy=504.0, cx=511.5, cy=511.5, factor=1000.0, bf=25.2, textured=True, nfeatures=2000),
 }
 
 _ROOM = dict(x=(-2.6, 2.6), y=(-1.4, 1.4), z=4.5)  # metres; camera near the origin looking down +z

@@ -425,6 +425,7 @@ typedef struct hvo_plane_params {
 } hvo_plane_params;
 
 typedef struct hvo_plane hvo_plane;
+/* images of up to 24576 10x10 blocks (1920x1200); larger ones are refused with HVO_ERR_ARG */
 int hvo_plane_create(const hvo_plane_params* p, int width, int height, int max_batch, int device, hvo_plane** out);
 void hvo_plane_destroy(hvo_plane* h);
 /* depth16: host [H][W] uint16.  planes7: [max_planes][7] doubles = normal(3), center(3), N.  membership: [H*W]
