@@ -99,24 +99,35 @@ public:
             return;
         }
         if (n > maxp) n = maxp;
+        assignPlanes(n, planes.data(), membership_.data(), depth_.data(), w_, hgt_, p_);
+    }
+
+    // Fills plane_num_, plane_vertices_, cloud and plane_filter from one frame's plane outputs of the C ABI: planes7 [n][7], the
+    // labels [w*h] (plane id; any value outside [0, n), such as -1 or 255, is no plane), the raw depth and the camera the planes were
+    // detected with.  runPlaneDetection and hvo_shim::FrameExtractorGPU (the frame call's int32 or one-byte labels) both fill through it.
+    template <class LabelT>
+    void assignPlanes(int n, const double* planes7, const LabelT* labels, const uint16_t* depth, int w, int h, const hvo_plane_params& cam) {
+        const int npx = w * h;
         plane_num_ = n;
         plane_vertices_.assign(n, std::vector<int>());
-        cloud.vertices.resize(depth_.size());
-        const double f = (double)p_.depth_factor, fx = (double)p_.fx, fy = (double)p_.fy, cx = (double)p_.cx, cy = (double)p_.cy;
-        for (int i = 0; i < (int)membership_.size(); ++i) {
-            const int m = membership_[i];
+        plane_filter.extractedPlanes.clear();
+        cloud.w = w; cloud.h = h;
+        cloud.vertices.resize(npx);
+        const double f = (double)cam.depth_factor, fx = (double)cam.fx, fy = (double)cam.fy, cx = (double)cam.cx, cy = (double)cam.cy;
+        for (int i = 0; i < npx; ++i) {
+            const int m = labels[i];
             if (m < 0 || m >= n) continue;
             plane_vertices_[m].push_back(i);
-            const int row = i / w_, col = i - row * w_;
-            const double z = (double)depth_[i] * f;  // PlaneExtractor.cpp:44-53
+            const int row = i / w, col = i - row * w;
+            const double z = (double)depth[i] * f;  // PlaneExtractor.cpp:44-53
             cloud.vertices[i][0] = ((double)col - cx) * z / fx;
             cloud.vertices[i][1] = ((double)row - cy) * z / fy;
             cloud.vertices[i][2] = z;
         }
         for (int i = 0; i < n; ++i) {
             auto s = std::make_shared<hvo_shim::PlaneSegLite>();
-            for (int k = 0; k < 3; ++k) { s->normal[k] = planes[7 * i + k]; s->center[k] = planes[7 * i + 3 + k]; }
-            s->N = (int)planes[7 * i + 6];
+            for (int k = 0; k < 3; ++k) { s->normal[k] = planes7[7 * i + k]; s->center[k] = planes7[7 * i + 3 + k]; }
+            s->N = (int)planes7[7 * i + 6];
             plane_filter.extractedPlanes.push_back(s);
         }
     }
